@@ -15,6 +15,9 @@ site table inside the timing): the batch cut into --e2e-shards window shards, th
 per shard on --e2e-lanes engine handles of the GPU (own stream and buffers, one CUDA context; pipeline.count_shards_pipelined), so that transfers and
 kernels of different shards overlap; the one-call figure is reported next to it (e2e.single_call_*).
 One JSON line on stdout (rank 0).
+
+  python bench.py ... --dump-outputs DIR   also writes the site table of the last timed step as DIR/<name>.npy
+                                           (see dump_outputs), so that two builds can be compared output for output
 """
 import argparse
 import json
@@ -201,6 +204,24 @@ def algorithmic_bytes(batch, n_tiles, tile, n_sites):
     return 1.5 * qbases + 4.0 * batch.cigar.shape[0] + 19.0 * batch.n_reads + 1.0 * n_tiles * tile + 104.0 * n_sites
 
 
+DUMP_SITES = 200_000  # sampled rows of the site table: 30 float64 values each, ~48 MB in all
+
+
+def dump_outputs(out_dir, sites, rank, world):
+    """Writes what a caller of the timed step receives, the compacted site table (tid, pos, ref, counts[26]), as
+    float64 .npy files.  The full table has ~1.7e7 rows at scale 1, so only a fixed, seeded sample of rows is written
+    (site_index.npy holds their row numbers), together with the column sums of counts over every row.  With
+    several GPUs each rank writes its own shard's table under a rank<r>_ prefix and samples a 1/world share."""
+    os.makedirs(out_dir, exist_ok=True)
+    n, k = sites.n_sites, DUMP_SITES // world
+    idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False)) if n > k else np.arange(n)
+    prefix = "rank%d_" % rank if world > 1 else ""
+    arrays = {"site_index": idx, "tid": sites.tid[idx], "pos": sites.pos[idx], "ref": sites.ref[idx],
+              "counts": sites.counts[idx], "counts_column_sums": sites.counts.sum(axis=0, dtype=np.uint64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a.astype(np.float64))
+
+
 def cpu_oracle_rate(sample, threads, steps=1):
     """Oracle port (plain C, OpenMP over windows) on a bounded sample; aligned bases / s."""
     import oracle
@@ -337,6 +358,8 @@ def run_ours(args, rank, world, local_rank):
         launches += 1
     barrier()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng.fetch(n_sites), rank, world)
     # a short timed region can end between two nvidia-smi rows: keep the same load running (untimed) until the sampler
     # has at least three rows taken under it
     extra = 0
@@ -647,7 +670,11 @@ def main():
     ap.add_argument("--cli-scale", type=float, default=0.2,
                     help="size of the BAM of the disk-to-disk CLI leg as a fraction of the workload (0 = skip; 1.0 = the "
                          "whole 5 M-read BAM, which takes ~100 s to write)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the site table of the last timed step (a seeded sample) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     quiet_stdout()
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     # torchrun pins OMP_NUM_THREADS=1; the (untimed) synthetic generator and the CPU oracle are OpenMP code

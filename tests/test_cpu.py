@@ -206,3 +206,29 @@ def test_early_cuda_warm_is_light_and_harmless(built):
             "print('ok')\n") % ROOT
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0 and r.stdout.strip() == "ok", r.stderr[-2000:]
+
+
+def test_bench_dump_outputs_is_a_seeded_float64_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the same table gives the same files, the sampled rows are the rows site_index names,
+    and counts_column_sums covers every row, not only the sample."""
+    import bench
+    from longsom_b200.batch import SiteCounts
+    rng = np.random.default_rng(3)
+    n = 1000
+    s = SiteCounts(rng.integers(0, 3, n).astype(np.int32), np.sort(rng.integers(0, 1 << 30, n)).astype(np.int32),
+                   rng.integers(0, 4, n).astype(np.uint8), rng.integers(0, 1 << 31, (n, 26)).astype(np.uint32))
+    monkeypatch.setattr(bench, "DUMP_SITES", 100)
+    bench.dump_outputs(str(tmp_path / "a"), s, 0, 1)
+    bench.dump_outputs(str(tmp_path / "b"), s, 0, 1)
+    names = ("site_index", "tid", "pos", "ref", "counts", "counts_column_sums")
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(x + ".npy" for x in names)
+    got = {x: np.load(tmp_path / "a" / (x + ".npy")) for x in names}
+    for x in names:
+        assert got[x].dtype == np.float64
+        assert np.array_equal(got[x], np.load(tmp_path / "b" / (x + ".npy")))
+    idx = got["site_index"].astype(np.int64)
+    assert idx.shape == (100,) and np.all(np.diff(idx) > 0)
+    assert np.array_equal(got["pos"], s.pos[idx]) and np.array_equal(got["counts"], s.counts[idx])
+    assert np.array_equal(got["counts_column_sums"], s.counts.sum(axis=0, dtype=np.uint64).astype(np.float64))
+    bench.dump_outputs(str(tmp_path / "r"), s, 1, 2)
+    assert np.load(tmp_path / "r" / "rank1_counts.npy").shape == (50, 26)
