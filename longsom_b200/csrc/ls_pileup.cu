@@ -176,6 +176,9 @@ extern "C" int ls_pileup_run(ls_ctx *ctx, const ls_count_params *params, int64_t
   // at once; the sizes are verified against the device counters with the final read-back, and the run is repeated
   // with read-backs if they ever differ.
   const bool replay = ctx->cache_valid && memcmp(&ctx->cache_params, params, sizeof *params) == 0 && !getenv("LS_NO_REPLAY");
+  // A run that is not a replay overwrites the sizes the next run starts from (n_segments, n_pieces), so the cache only
+  // survives it if the run refreshes it below.
+  if (!replay) ctx->cache_valid = false;
 
   const int64_t n = ctx->n_reads;
   ctx->cell_bits = ls_bits_for((uint64_t)(ctx->max_cell + 1));
@@ -213,9 +216,12 @@ extern "C" int ls_pileup_run(ls_ctx *ctx, const ls_count_params *params, int64_t
       LS_CK(cudaMemsetAsync(ctx->wcount.p, 0, (size_t)ctx->n_windows * 4, st));
     }
     // Output sizes are only known after the walk: start from the previous run's sizes (or an estimate) and
-    // relaunch with exact sizes if the reservation counters ran past the buffers.
-    uint64_t seg_need = ctx->n_segments > 0 ? (uint64_t)ctx->n_segments : (uint64_t)n * 5 + 1024;
-    uint64_t piece_need = ctx->n_pieces > 0 ? (uint64_t)ctx->n_pieces : (uint64_t)ctx->n_cigar + seg_need;
+    // relaunch with exact sizes if the reservation counters ran past the buffers.  A replay has no relaunch: it sizes
+    // the builder with the sizes it will sort and count.
+    uint64_t seg_need = replay ? ctx->cache_seg[0]
+                               : (ctx->n_segments > 0 ? (uint64_t)ctx->n_segments : (uint64_t)n * 5 + 1024);
+    uint64_t piece_need = replay ? ctx->cache_seg[1]
+                                 : (ctx->n_pieces > 0 ? (uint64_t)ctx->n_pieces : (uint64_t)ctx->n_cigar + seg_need);
     std::vector<uint32_t> wc;
     bool want_wcount = cap_possible;
     for (int attempt = 0;; ++attempt) {
