@@ -154,7 +154,7 @@ extern "C" int ls_pileup_upload(ls_ctx *ctx, const ls_read_batch *b, const ls_wi
   if (!b) LS_FAIL(LS_E_ARG, "ls_pileup_upload: batch is null");
   ctx->have_batch = false;
   ctx->have_run = false;
-  ctx->cache_valid = false;
+  ctx->replay.valid = false;
   const int64_t n = b->n_reads;
   if (n < 0 || b->n_cigar < 0 || b->n_bases < 0) LS_FAIL(LS_E_ARG, "ls_pileup_upload: negative size");
   if (n >= (int64_t)0xffffffffll) LS_FAIL(LS_E_ARG, "ls_pileup_upload: more than 2^32-1 reads per batch");
@@ -250,21 +250,29 @@ extern "C" int ls_pileup_upload(ls_ctx *ctx, const ls_read_batch *b, const ls_wi
 // (= per window): the first kept record at a start position P is always accepted; a later
 // record at P is dropped iff 1 + #{accepted records of this call with end >= P} > maxcnt.
 // Only windows that fetch more than max_depth records can ever drop, so the common case
-// costs one device-side count (done inside seg_build_kernel) and nothing here.
-int ls_depth_cap_host(ls_ctx *ctx, int min_mq, int max_depth, const std::vector<uint32_t> &wcount) {
-  const int64_t n = ctx->n_reads, nw = ctx->n_windows;
+// costs one device-side count of the fetches per window and nothing here.
+// The windows (pileup() calls) are host arrays; d_wcount, if not null, holds their fetch counts
+// on the device, and windows at or below the cap are skipped.  ctx->rend (reference end of every
+// read) must be filled on ctx->stream.  Sets ctx->drop_keys / ctx->n_drop: (window << 32 | read).
+int ls_depth_cap_host(ls_ctx *ctx, const std::vector<int32_t> &wtid, const std::vector<int32_t> &wstart,
+                      const std::vector<int32_t> &wend, const uint32_t *d_wcount, int min_mq, int max_depth) {
+  const int64_t n = ctx->n_reads, nw = (int64_t)wtid.size();
+  cudaStream_t st = ctx->stream;
   std::vector<int32_t> tid(n), pos(n), rend(n);
   std::vector<uint16_t> flag(n);
   std::vector<uint8_t> mapq(n);
-  LS_CK(cudaMemcpy(tid.data(), ctx->tid.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
-  LS_CK(cudaMemcpy(pos.data(), ctx->pos.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
-  LS_CK(cudaMemcpy(rend.data(), ctx->rend.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
-  LS_CK(cudaMemcpy(flag.data(), ctx->flag.p, (size_t)n * 2, cudaMemcpyDeviceToHost));
-  LS_CK(cudaMemcpy(mapq.data(), ctx->mapq.p, (size_t)n, cudaMemcpyDeviceToHost));
+  std::vector<uint32_t> wcount(d_wcount ? nw : 0);
+  LS_CK(cudaMemcpyAsync(tid.data(), ctx->tid.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaMemcpyAsync(pos.data(), ctx->pos.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaMemcpyAsync(rend.data(), ctx->rend.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaMemcpyAsync(flag.data(), ctx->flag.p, (size_t)n * 2, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaMemcpyAsync(mapq.data(), ctx->mapq.p, (size_t)n, cudaMemcpyDeviceToHost, st));
+  if (d_wcount) LS_CK(cudaMemcpyAsync(wcount.data(), d_wcount, (size_t)nw * 4, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaStreamSynchronize(st));
   std::vector<uint64_t> drops;
   for (int64_t w = 0; w < nw; ++w) {
-    if ((int64_t)wcount[w] <= (int64_t)max_depth) continue;
-    const int32_t wt = ctx->h_wtid[w], ws = ctx->h_wstart[w], we = ctx->h_wend[w];
+    if (d_wcount && (int64_t)wcount[w] <= (int64_t)max_depth) continue;
+    const int32_t wt = wtid[w], ws = wstart[w], we = wend[w];
     // first read of this contig
     int64_t r0 = std::lower_bound(tid.begin(), tid.end(), wt) - tid.begin();
     std::priority_queue<int32_t, std::vector<int32_t>, std::greater<int32_t>> live;
@@ -294,7 +302,9 @@ int ls_depth_cap_host(ls_ctx *ctx, int min_mq, int max_depth, const std::vector<
   std::sort(drops.begin(), drops.end());
   ctx->n_drop = (int64_t)drops.size();
   LS_CK(ctx->drop_keys.ensure(drops.size() * 8 + 16));
-  if (!drops.empty())
-    LS_CK(cudaMemcpy(ctx->drop_keys.p, drops.data(), drops.size() * 8, cudaMemcpyHostToDevice));
+  if (!drops.empty()) {
+    LS_CK(cudaMemcpyAsync(ctx->drop_keys.p, drops.data(), drops.size() * 8, cudaMemcpyHostToDevice, st));
+    LS_CK(cudaStreamSynchronize(st));  // the copy reads `drops`
+  }
   return LS_OK;
 }

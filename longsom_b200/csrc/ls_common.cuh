@@ -83,6 +83,33 @@ __host__ __device__ __forceinline__ uint32_t piece_units(uint32_t meta) {
 // loads the aligned 40-byte / 24-byte blocks around its bases, which may reach a few bytes past either end.
 #define LS_QPAD 64
 
+// Device counters of one pileup run (ctx->counters, zeroed at the start of ls_pileup_run).  Kernels get pointers to
+// single fields; the 32-bit flags and counters sit in 8-byte slots.
+struct RunCounters {
+  unsigned long long n_aligned;  // aligned bases (seg_build_kernel)
+  unsigned long long n_events;   // pileup entries (pileup_count_kernel)
+  uint64_t n_sites;              // passing sites: total of the scan of the per-slot pass counts
+  uint64_t n_slots;              // non-empty tiles
+  alignas(8) uint32_t n_parts;   // parts of deep tiles (part_build_kernel)
+  alignas(8) uint32_t long_run;  // some same-cell run is too long for the packed counters (classify_kernel)
+  alignas(8) uint32_t n_light;   // parts of shallow tiles
+  alignas(8) uint32_t cap_flag;  // some window fetches more than max_depth records
+  // reservation totals of seg_build_kernel, which takes them as one array
+  unsigned long long n_segments, n_pieces, n_units;
+  uint64_t tot_s, tot_m, tot_u;  // sizes of the S / M / U unit streams
+  uint64_t n_groups;             // (cell, window) groups in M
+  uint64_t n_members;            // run-member segments
+};
+static_assert(sizeof(RunCounters) == 128, "RunCounters layout");
+
+// What a replay of ls_pileup_run takes from the last run on the batch that it can stand for
+struct ReplaySnapshot {
+  bool valid = false;
+  ls_count_params params = {};
+  RunCounters mid = {};  // the device counters at the run's middle read-back
+  int64_t n_sites = 0;
+};
+
 struct ls_ctx {
   int device = 0;
   int num_sms = LS_NUM_SMS_DEFAULT;
@@ -107,11 +134,7 @@ struct ls_ctx {
 
   // ---- run state ----
   bool have_run = false, compacted = false;
-  // sizes of the last completed run on this batch, for the replay mode of ls_pileup_run
-  bool cache_valid = false;
-  ls_count_params cache_params = {};
-  uint64_t cache_seg[3] = {0, 0, 0}, cache_tot[16] = {0};
-  int64_t cache_n_sites = 0;
+  ReplaySnapshot replay;  // sizes of the last completed run on this batch, for the replay mode of ls_pileup_run
   ls_count_params params = {};
   DBuf segs, pieces, keys_a, keys_b, vals_a, vals_b, rs_hist, scan_tmp, counters;
   DBuf tile_flag, tile_rank, slot_tile, slot_lo, slot_out, slot_mask, slot_npass, slot_off;
@@ -224,7 +247,8 @@ __device__ __forceinline__ uint8_t class_letter(int cls) {
 
 __device__ __forceinline__ uint8_t upper_ascii(uint8_t c) { return (c >= 'a' && c <= 'z') ? (uint8_t)(c - 32) : c; }
 
-int ls_depth_cap_host(ls_ctx *ctx, int min_mq, int max_depth, const std::vector<uint32_t> &wcount);
+int ls_depth_cap_host(ls_ctx *ctx, const std::vector<int32_t> &wtid, const std::vector<int32_t> &wstart,
+                      const std::vector<int32_t> &wend, const uint32_t *d_wcount, int min_mq, int max_depth);
 int ls_tile_size(void);
 
 // ---- utilities implemented in ls_util.cu --------------------------------------------------

@@ -37,7 +37,7 @@
 // shared-memory state, no atomics and no warp-level serialisation per run.
 #pragma once
 
-constexpr int K1_WARPS = 8;              // default CTA shape (the kernel is templated on it: LS_K1_SHAPE)
+constexpr int K1_WARPS = 8;              // warps of a count CTA (3 CTAs / SM with packed counters, 1 without)
 constexpr int K1_THREADS = K1_WARPS * 32;
 constexpr int K1_PART_SEGS = 2048;       // nominal segments per part
 constexpr int K1_MAX_RUN_PACKED = 2039;  // packed counters (12-bit) need: part segs + run extension <= 4095
@@ -611,10 +611,8 @@ __global__ void __launch_bounds__(256) expand_runs_kernel(ExpandArgs a) {
   });
 }
 
-template <bool PACKED, int MIN_CTAS, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, MIN_CTAS) pileup_count_kernel(CountArgs a) {
-  constexpr int K1_THREADS = WARPS * 32;  // shadows the default shape inside the kernel
-  constexpr int K1_WARPS = WARPS;
+template <bool PACKED>
+__global__ void __launch_bounds__(K1_THREADS, PACKED ? 3 : 1) pileup_count_kernel(CountArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   TileSmemT<PACKED> &sm = *reinterpret_cast<TileSmemT<PACKED> *>(smem_raw);
   PartDesc pd;

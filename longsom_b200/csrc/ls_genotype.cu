@@ -11,9 +11,6 @@
 // sites inside each reference-consuming op and scatters with global atomics into the dense
 // [site][cell] tensors (one int32 add per hit; hits are ~depth x sites, tiny next to HBM).
 // Bases that cover no candidate site are never loaded.
-#include <algorithm>
-#include <queue>
-
 #include "ls_common.cuh"
 
 struct GenoArgs {
@@ -278,7 +275,7 @@ __global__ void __launch_bounds__(256) bin_fetch_count_kernel(int64_t n, const i
 }
 
 // Depth cap per pileup() call of the genotype scripts: one call per 50 kb bin of candidate sites
-// over [min-1, max+1) (SingleCellGenotype.py:110-124).  Same rule as ls_depth_cap_host.
+// over [min-1, max+1) (SingleCellGenotype.py:110-124); the rule is K1's (ls_depth_cap_host).
 static int geno_depth_cap(ls_ctx *ctx, const std::vector<int32_t> &btid, const std::vector<int32_t> &bstart,
                           const std::vector<int32_t> &bend, int min_mq, int max_depth, CandArgs ca = CandArgs{}) {
   const int64_t n = ctx->n_reads;
@@ -310,48 +307,9 @@ static int geno_depth_cap(ls_ctx *ctx, const std::vector<int32_t> &btid, const s
   LS_CK(ctx->rend.ensure((size_t)n * 4));
   read_end_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, ctx->pos.as<int32_t>(), ctx->cigar_off.as<uint32_t>(),
                                                                ctx->cigar.as<uint32_t>(), ctx->rend.as<int32_t>());
-  std::vector<int32_t> tid(n), pos(n), rend(n);
-  std::vector<uint16_t> flag(n);
-  std::vector<uint8_t> mapq(n);
-  LS_CK(cudaMemcpyAsync(rend.data(), ctx->rend.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaMemcpyAsync(tid.data(), ctx->tid.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaMemcpyAsync(pos.data(), ctx->pos.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaMemcpyAsync(flag.data(), ctx->flag.p, (size_t)n * 2, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaMemcpyAsync(mapq.data(), ctx->mapq.p, (size_t)n, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaStreamSynchronize(st));
-  std::vector<uint64_t> drops;
-  for (size_t w = 0; w < btid.size(); ++w) {
-    const int32_t wt = btid[w], ws = bstart[w], we = bend[w];
-    int64_t r0 = std::lower_bound(tid.begin(), tid.end(), wt) - tid.begin();
-    std::priority_queue<int32_t, std::vector<int32_t>, std::greater<int32_t>> live;
-    int32_t last_p = -1;
-    bool any_at_p = false;
-    for (int64_t r = r0; r < n && tid[r] == wt && pos[r] < we; ++r) {
-      uint32_t f = flag[r];
-      if (f & LS_FLAG_FILTER) continue;
-      if ((int)mapq[r] < min_mq) continue;
-      if ((f & LS_FLAG_PAIRED) && !(f & LS_FLAG_PROPER)) continue;
-      int32_t e = rend[r] > pos[r] ? rend[r] : pos[r] + 1;
-      if (e <= ws) continue;
-      const int32_t P = pos[r];
-      if (P != last_p) {
-        last_p = P;
-        any_at_p = false;
-      }
-      while (!live.empty() && live.top() < P) live.pop();
-      if (any_at_p && (int64_t)1 + (int64_t)live.size() > (int64_t)max_depth) {
-        drops.push_back(((uint64_t)w << 32) | (uint64_t)r);
-        continue;
-      }
-      any_at_p = true;
-      live.push(rend[r]);
-    }
-  }
-  std::sort(drops.begin(), drops.end());
-  ctx->n_drop = (int64_t)drops.size();
-  LS_CK(ctx->drop_keys.ensure(drops.size() * 8 + 16));
-  if (!drops.empty()) LS_CK(cudaMemcpy(ctx->drop_keys.p, drops.data(), drops.size() * 8, cudaMemcpyHostToDevice));
-  return LS_OK;
+  LS_CK(cudaGetLastError());
+  // every bin is walked: one that fetches at most max_depth records drops nothing
+  return ls_depth_cap_host(ctx, btid, bstart, bend, nullptr, min_mq, max_depth);
 }
 
 // Site table of a genotype call: sorted keys, the pileup() call (bin) of every site, and the bins.
@@ -608,27 +566,12 @@ extern "C" int ls_genotype_count(ls_ctx *ctx, const int32_t *site_tid, const int
   }
   if (!site_tid || !site_pos || !alt_class || !dp || !alt) LS_FAIL(LS_E_ARG, "ls_genotype_count: null array");
   const int32_t bin = params->bin_size > 0 ? params->bin_size : 50000;
-  std::vector<uint64_t> keys((size_t)n_sites);
-  std::vector<uint32_t> sbin((size_t)n_sites);
-  std::vector<int32_t> btid, bstart, bend;
-  for (int64_t i = 0; i < n_sites; ++i) {
-    if (site_tid[i] < 0 || site_pos[i] < 0) LS_FAIL(LS_E_ARG, "ls_genotype_count: negative site coordinate");
-    keys[i] = ((uint64_t)(uint32_t)site_tid[i] << 32) | (uint32_t)site_pos[i];
-    if (i > 0 && keys[i] <= keys[i - 1]) LS_FAIL(LS_E_ARG, "ls_genotype_count: sites must be sorted and unique");
-    // build_dict_variants: CHROM_floor(POS / bin) with the 1-based POS of the TSV (:253-274)
-    const int64_t code = ((int64_t)site_pos[i] + 1) / bin;
-    if (i == 0 || site_tid[i] != site_tid[i - 1] || code != ((int64_t)site_pos[i - 1] + 1) / bin) {
-      btid.push_back(site_tid[i]);
-      bstart.push_back(site_pos[i] - 1 < 0 ? 0 : site_pos[i] - 1);
-      bend.push_back(site_pos[i] + 1);
-    } else {
-      bend.back() = site_pos[i] + 1;
-    }
-    sbin[i] = (uint32_t)(btid.size() - 1);
-  }
+  GenoSites g;
+  int rc = geno_prepare_sites(ctx, site_tid, site_pos, n_sites, bin, g);
+  if (rc != LS_OK) return rc;
   LS_CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  int rc = geno_depth_cap(ctx, btid, bstart, bend, params->min_mq, params->max_depth);
+  rc = geno_depth_cap(ctx, g.btid, g.bstart, g.bend, params->min_mq, params->max_depth);
   if (rc != LS_OK) return rc;
   const size_t cells = (size_t)n_sites * (size_t)n_cells;
   LS_CK(ctx->g_a.ensure((size_t)n_sites * 8));
@@ -637,45 +580,18 @@ extern "C" int ls_genotype_count(ls_ctx *ctx, const int32_t *site_tid, const int
   LS_CK(ctx->g_d.ensure(cells * 4));
   LS_CK(ctx->g_e.ensure((size_t)n_sites * 4));
   LS_CK(ctx->counters.ensure(64));
-  LS_CK(cudaMemcpyAsync(ctx->g_a.p, keys.data(), (size_t)n_sites * 8, cudaMemcpyHostToDevice, st));
+  LS_CK(cudaMemcpyAsync(ctx->g_a.p, g.keys.data(), (size_t)n_sites * 8, cudaMemcpyHostToDevice, st));
   LS_CK(cudaMemcpyAsync(ctx->g_b.p, alt_class, (size_t)n_sites, cudaMemcpyHostToDevice, st));
-  LS_CK(cudaMemcpyAsync(ctx->g_e.p, sbin.data(), (size_t)n_sites * 4, cudaMemcpyHostToDevice, st));
+  LS_CK(cudaMemcpyAsync(ctx->g_e.p, g.sbin.data(), (size_t)n_sites * 4, cudaMemcpyHostToDevice, st));
   LS_CK(cudaEventRecord(ctx->ev[0], st));
   LS_CK(cudaMemsetAsync(ctx->g_c.p, 0, cells * 4, st));
   LS_CK(cudaMemsetAsync(ctx->g_d.p, 0, cells * 4, st));
   LS_CK(cudaMemsetAsync(ctx->counters.p, 0, 64, st));
   GenoArgs a;
-  a.n_reads = ctx->n_reads;
-  a.tid = ctx->tid.as<int32_t>();
-  a.pos = ctx->pos.as<int32_t>();
-  a.cell = ctx->cell.as<int32_t>();
-  a.lq = ctx->lq.as<int32_t>();
-  a.flag = ctx->flag.as<uint16_t>();
-  a.mapq = ctx->mapq.as<uint8_t>();
-  a.cigar_off = ctx->cigar_off.as<uint32_t>();
-  a.cigar = ctx->cigar.as<uint32_t>();
-  a.base_off = ctx->base_off.as<uint64_t>();
-  a.seq4 = ctx->seq4_d();
-  a.qual = ctx->qual_d();
-  a.site_key = ctx->g_a.as<uint64_t>();
-  a.alt_class = ctx->g_b.as<uint8_t>();
-  a.site_bin = ctx->g_e.as<uint32_t>();
-  a.n_sites = n_sites;
-  a.n_cells = n_cells;
-  a.min_bq = params->min_bq;
-  a.min_mq = params->min_mq;
-  a.alt_only = params->alt_only;
-  a.drop_keys = ctx->drop_keys.as<uint64_t>();
-  a.n_drop = ctx->n_drop;
+  geno_fill_args(ctx, a, n_sites, n_cells, params);
   a.dp = ctx->g_c.as<int32_t>();
   a.alt = ctx->g_d.as<int32_t>();
-  a.n_events = ctx->counters.as<unsigned long long>();
   LS_CK(cudaEventRecord(ctx->ev[1], st));
-  a.hit_cnt = nullptr;
-  a.hit_off = nullptr;
-  a.hits = nullptr;
-  a.hits32 = nullptr;
-  a.sentinel = 0;
   if (ctx->n_reads > 0) genotype_kernel<0><<<(unsigned)((ctx->n_reads + 255) / 256), 256, 0, st>>>(a);
   LS_CK(cudaGetLastError());
   LS_CK(cudaEventRecord(ctx->ev[2], st));

@@ -5,20 +5,13 @@
 //   :152-180 (EasyReadPileup) and the htslib pileup engine behind
 //   pysam.AlignmentFile.pileup (SURVEY.md Appendix A).
 //
-// Design (B200): the reference walks reference columns and, per column, a Python
-// list of reads.  Here the unit of work is a TILE of LS_TILE reference positions
-// owned by exactly one CTA, so all accumulation is shared-memory atomics and the
-// result leaves the SM with plain coalesced stores (no global atomics, no
-// zero-initialised global histograms).
-//   1. seg_build_kernel (ls_segments.cuh): one thread per read walks its CIGAR and emits one Segment per
-//      (read, tile) pair that has at least one pileup entry, plus the segment's Pieces (ops clipped to the tile).
-//   2. radix sort of segments by (tile, cell)  -> same-cell segments of a tile are adjacent.
-//   3. pileup_count_kernel : CTA per part (<= 2048 sorted segments of one tile); a warp owns a run of same-cell
-//      segments, lanes stride consecutive reference positions (coalesced seq4/qual
-//      reads, conflict-free shared atomics); distinct-cell counts NC/CC are
-//      "reads minus same-cell duplicates", the duplicates found with a per-warp
-//      T-byte seen[] mask that is only touched for runs longer than one segment.
-//   4. site epilogue applies the reference's gates and writes [slot][field][T] words.
+// Design (B200): the reference walks reference columns and, per column, a Python list of reads.  Here the unit of
+// work is a TILE of LS_TILE reference positions, and the accumulation of a tile is shared-memory atomics of the CTAs
+// that own it.  One run (DESIGN.md §4, K1):
+//   1. seg_build_kernel (ls_segments.cuh): one Segment per (read, tile) pair with a pileup entry, plus its Pieces.
+//   2. radix sort of the segments by (tile, cell); the sorted segments become the S / M / U unit streams (ls_count.cuh).
+//   3. pileup_count_kernel: a CTA per part of a tile, a lane per unit; the site epilogue applies the reference's gates.
+//   4. compact_sites_kernel: the passing sites in the reference's output order.
 #include <cstddef>
 #include <cstdlib>
 
@@ -158,6 +151,257 @@ static SegArgs make_seg_args(ls_ctx *ctx, const ls_count_params &p, bool emit_un
 int ls_tile_size(void) { return LS_TILE; }
 extern "C" int ls_pileup_tile_size(void) { return LS_TILE; }
 
+static int read_counters(ls_ctx *ctx, const RunCounters *d, RunCounters &h) {
+  LS_CK(cudaMemcpyAsync(&h, d, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+  LS_CK(cudaStreamSynchronize(ctx->stream));
+  return LS_OK;
+}
+
+// Phase 1: one Segment per (read, tile) pair and its Pieces.  Their numbers are only known after the walk: a cold run
+// starts from the previous run's sizes (or an estimate), reads the counters back into h and relaunches with exact
+// sizes if the reservations ran past the buffers, or without the (window, read) pairs the depth cap drops.  A replay
+// sizes the builder from h (the snapshot) and has no relaunch.
+static int build_segments(ls_ctx *ctx, const ls_count_params &p, bool replay, RunCounters *d, RunCounters &h,
+                          int &launches) {
+  const int64_t n = ctx->n_reads;
+  if (n == 0 || ctx->n_windows == 0) return LS_OK;
+  cudaStream_t st = ctx->stream;
+  ctx->n_drop = 0;
+  SegArgs sa = make_seg_args(ctx, p, p.min_ac > 0);
+  // the depth cap can only fire in a window that fetches more than max_depth records (replay: known not to fire)
+  bool want_wcount = !replay && p.max_depth > 0 && n > (int64_t)p.max_depth;
+  if (want_wcount) {
+    LS_CK(ctx->rend.ensure((size_t)n * 4));
+    LS_CK(ctx->wcount.ensure((size_t)ctx->n_windows * 4));
+    LS_CK(cudaMemsetAsync(ctx->wcount.p, 0, (size_t)ctx->n_windows * 4, st));
+  }
+  uint64_t seg_need = replay ? h.n_segments : (ctx->n_segments > 0 ? (uint64_t)ctx->n_segments : (uint64_t)n * 5 + 1024);
+  uint64_t piece_need =
+      replay ? h.n_pieces : (ctx->n_pieces > 0 ? (uint64_t)ctx->n_pieces : (uint64_t)ctx->n_cigar + seg_need);
+  for (int attempt = 0;; ++attempt) {
+    LS_CK(ctx->segs.ensure((size_t)seg_need * sizeof(Segment)));
+    LS_CK(ctx->pieces.ensure((size_t)piece_need * sizeof(Piece)));
+    LS_CK(ctx->keys_a.ensure((size_t)seg_need * 8));
+    LS_CK(ctx->keys_b.ensure((size_t)seg_need * 8));
+    LS_CK(ctx->vals_a.ensure((size_t)seg_need * 4));
+    LS_CK(ctx->vals_b.ensure((size_t)seg_need * 4));
+    seg_build_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(
+        sa, ctx->segs.as<Segment>(), ctx->keys_a.as<uint64_t>(), ctx->pieces.as<Piece>(), seg_need, piece_need,
+        &d->n_segments, &d->n_aligned, want_wcount ? ctx->rend.as<int32_t>() : nullptr,
+        want_wcount ? ctx->wcount.as<uint32_t>() : nullptr, (uint32_t)p.max_depth, &d->cap_flag);
+    ++launches;
+    LS_CK(cudaGetLastError());
+    if (replay) return LS_OK;
+    int rc = read_counters(ctx, d, h);
+    if (rc != LS_OK) return rc;
+    bool again = false;
+    if (want_wcount && h.cap_flag) {  // some window fetches more than max_depth records
+      rc = ls_depth_cap_host(ctx, ctx->h_wtid, ctx->h_wstart, ctx->h_wend, ctx->wcount.as<uint32_t>(), p.min_mq,
+                             p.max_depth);
+      if (rc != LS_OK) return rc;
+      if (ctx->n_drop > 0) {  // redo the walk without the dropped (window, read) pairs
+        sa = make_seg_args(ctx, p, p.min_ac > 0);
+        again = true;
+      }
+    }
+    want_wcount = false;
+    if (!again && (h.n_segments > seg_need || h.n_pieces > piece_need)) {
+      seg_need = h.n_segments > seg_need ? h.n_segments : seg_need;
+      piece_need = h.n_pieces > piece_need ? h.n_pieces : piece_need;
+      again = true;
+    }
+    if (!again) return LS_OK;
+    if (attempt >= 3) LS_FAIL(LS_E_STATE, "ls_pileup_run: segment builder did not converge");
+    LS_CK(cudaMemsetAsync(&d->n_aligned, 0, sizeof d->n_aligned, st));
+    LS_CK(cudaMemsetAsync(&d->n_segments, 0, 3 * sizeof d->n_segments, st));
+  }
+}
+
+// Phase 2: the segments sorted by (tile, cell), the slot ranks of the non-empty tiles, and the place of every segment
+// in the unit streams (S: single segments, M: same-cell runs, U: uncounted reads).  The stream sizes go to the device
+// counters; ea comes back set up for the expansion.
+static int build_streams(ls_ctx *ctx, const ls_count_params &p, int64_t nseg, RunCounters *d, ExpandArgs &ea,
+                         int &launches) {
+  cudaStream_t st = ctx->stream;
+  const int tile_bits = ls_bits_for((uint64_t)(ctx->n_tiles_total > 0 ? ctx->n_tiles_total - 1 : 0));
+  LS_CK(cudaEventRecord(ctx->ev[1], st));
+  LS_CK(ls_radix_sort_pairs(ctx->keys_a.as<uint64_t>(), ctx->keys_b.as<uint64_t>(), ctx->vals_a.as<uint32_t>(),
+                            ctx->vals_b.as<uint32_t>(), nseg, tile_bits + ctx->cell_bits, ctx->rs_hist,
+                            &ctx->sorted_keys, &ctx->sorted_vals, ctx->num_sms, st, &launches));
+  LS_CK(ctx->tile_flag.ensure((size_t)nseg * 4));
+  LS_CK(ctx->tile_rank.ensure((size_t)nseg * 4));
+  const uint64_t cmask = (1ull << ctx->cell_bits) - 1ull;
+  const uint64_t unc = (uint64_t)(uint32_t)(ctx->max_cell + 1);
+  const bool with_u = p.min_ac > 0;
+  LS_CK(ctx->offs_s.ensure((size_t)(nseg + 1) * 4));
+  LS_CK(ctx->offs_m.ensure((size_t)(nseg + 1) * 4));
+  LS_CK(ctx->goffs.ensure((size_t)(nseg + 1) * 4));
+  LS_CK(ctx->mrank.ensure((size_t)(nseg + 1) * 4));
+  LS_CK(ctx->mlist.ensure((size_t)(nseg + 1) * 4));
+  if (with_u) LS_CK(ctx->offs_u.ensure((size_t)(nseg + 1) * 4));
+  uint32_t *os = ctx->offs_s.as<uint32_t>(), *om = ctx->offs_m.as<uint32_t>(), *og = ctx->goffs.as<uint32_t>();
+  uint32_t *ou = with_u ? ctx->offs_u.as<uint32_t>() : nullptr, *mr = ctx->mrank.as<uint32_t>();
+  classify_kernel<<<(unsigned)((nseg + 1 + 255) / 256), 256, 0, st>>>(
+      ctx->sorted_keys, ctx->sorted_vals, ctx->segs.as<Segment>(), nseg, cmask, unc, ctx->cell_bits, os, om, ou, mr,
+      ctx->tile_flag.as<uint32_t>(), &d->long_run);
+  ++launches;
+  // slot ranks, S / M (/ U) stream offsets and run-member ranks: independent scans, one launch
+  LsScanJob jobs[5];
+  int nj = 0;
+  jobs[nj++] = LsScanJob{ctx->tile_flag.as<uint32_t>(), ctx->tile_rank.as<uint32_t>(), nseg, &d->n_slots};
+  jobs[nj++] = LsScanJob{os, os, nseg + 1, &d->tot_s};
+  jobs[nj++] = LsScanJob{om, om, nseg + 1, &d->tot_m};
+  jobs[nj++] = LsScanJob{mr, mr, nseg + 1, &d->n_members};
+  if (with_u) jobs[nj++] = LsScanJob{ou, ou, nseg + 1, &d->tot_u};
+  LS_CK(ls_scan_exclusive_u32_multi(jobs, nj, ctx->scan_tmp, st));
+  ++launches;
+  mlist_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(ctx->sorted_keys, nseg, cmask, unc, mr,
+                                                               ctx->mlist.as<uint32_t>());
+  ++launches;
+  ea.keys = ctx->sorted_keys;
+  ea.vals = ctx->sorted_vals;
+  ea.segs = ctx->segs.as<Segment>();
+  ea.pieces = ctx->pieces.as<Piece>();
+  ea.n = nseg;
+  ea.cmask = cmask;
+  ea.unc = unc;
+  ea.offs_s = os;
+  ea.offs_m = om;
+  ea.offs_u = ou;
+  ea.tot_s = &d->tot_s;
+  ea.tot_m = &d->tot_m;
+  ea.tot_g = &d->n_groups;
+  ea.tot_ms = &d->n_members;
+  ea.mlist = ctx->mlist.as<uint32_t>();
+  ea.goffs = og;
+  ea.gdir = nullptr;
+  ea.units = nullptr;
+  // one warp per 32 run members; the grid covers the worst case (every segment a run member)
+  LS_CK(cudaMemsetAsync(og, 0, (size_t)(nseg + 1) * 4, st));
+  rungroups_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(ea);
+  ++launches;
+  LS_CK(ls_scan_exclusive_u32(og, og, nseg + 1, &d->n_groups, ctx->scan_tmp, st));
+  launches += 1;
+  LS_CK(cudaGetLastError());
+  return LS_OK;
+}
+
+// Phase 3: the units written into their streams, the tiles split into parts, the count kernel, and the scan of the
+// per-slot pass counts that places every tile's passing sites in the output (its total goes to n_sites).  Sized by h,
+// the counters of the middle read-back.
+static int count_tiles(ls_ctx *ctx, const ls_count_params &p, int64_t nseg, const RunCounters &h, RunCounters *d,
+                       ExpandArgs ea, int &launches) {
+  cudaStream_t st = ctx->stream;
+  const int64_t n_slots = (int64_t)h.n_slots;
+  const bool with_u = p.min_ac > 0;
+  LS_CK(ctx->slot_tile.ensure((size_t)n_slots * 8));
+  LS_CK(ctx->slot_lo.ensure((size_t)(n_slots + 1) * 4));
+  slot_fill_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(
+      ctx->sorted_keys, nseg, ctx->cell_bits, ctx->tile_flag.as<uint32_t>(), ctx->tile_rank.as<uint32_t>(), n_slots,
+      ctx->slot_tile.as<int64_t>(), ctx->slot_lo.as<uint32_t>());
+  ++launches;
+  LS_CK(ctx->units.ensure((size_t)(h.n_units + 1) * 8));
+  LS_CK(ctx->gdir.ensure((size_t)(h.n_groups + 1) * 4));
+  ea.gdir = ctx->gdir.as<uint32_t>();
+  ea.units = ctx->units.as<uint2>();
+  expand_single_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(ea);
+  if (h.n_members > 0) expand_runs_kernel<<<(unsigned)((h.n_members + 255) / 256), 256, 0, st>>>(ea);
+  launches += 2;
+  LS_CK(cudaGetLastError());
+  LS_CK(cudaEventRecord(ctx->ev[2], st));
+
+  LS_CK(ctx->slot_out.ensure((size_t)n_slots * LS_SITE_WORDS * LS_TILE * 4));
+  LS_CK(ctx->slot_mask.ensure((size_t)n_slots * (LS_TILE / 32) * 4));
+  LS_CK(ctx->slot_npass.ensure((size_t)n_slots * 4));
+  LS_CK(ctx->slot_off.ensure((size_t)n_slots * 4));
+  const int64_t max_parts = n_slots + nseg / K1_PART_SEGS + 1;
+  LS_CK(ctx->part_slot.ensure((size_t)max_parts * sizeof(PartDesc)));
+  LS_CK(ctx->slot_done.ensure((size_t)n_slots * 4));
+  LS_CK(ctx->slot_desc.ensure((size_t)n_slots * sizeof(SlotDesc)));
+  if (with_u) LS_CK(ctx->acbuf.ensure((size_t)n_slots * LS_TILE * 4));
+  LS_CK(cudaMemsetAsync(ctx->part_slot.p, 0xff, (size_t)max_parts * sizeof(PartDesc), st));
+  PartBuildArgs pb;
+  pb.slot_lo = ctx->slot_lo.as<uint32_t>();
+  pb.slot_tile = ctx->slot_tile.as<int64_t>();
+  pb.n_slots = n_slots;
+  pb.keys = ctx->sorted_keys;
+  pb.offs_s = ctx->offs_s.as<uint32_t>();
+  pb.offs_u = with_u ? ctx->offs_u.as<uint32_t>() : nullptr;
+  pb.goffs = ctx->goffs.as<uint32_t>();
+  pb.n_windows = ctx->n_windows;
+  pb.wstart = ctx->wstart.as<int32_t>();
+  pb.wend = ctx->wend.as<int32_t>();
+  pb.wtile_base = ctx->wtile_base.as<int64_t>();
+  pb.wref_off = ctx->wref_off.as<uint64_t>();
+  pb.parts = ctx->part_slot.as<PartDesc>();
+  pb.slot_desc = ctx->slot_desc.as<SlotDesc>();
+  pb.wtid = ctx->wtid.as<int32_t>();
+  pb.slot_done = ctx->slot_done.as<uint32_t>();
+  pb.n_parts = &d->n_parts;
+  pb.n_light = &d->n_light;
+  pb.max_parts = (uint32_t)max_parts;
+  pb.out = ctx->slot_out.as<uint32_t>();
+  pb.acbuf = with_u ? ctx->acbuf.as<uint32_t>() : nullptr;
+  part_build_kernel<<<(unsigned)n_slots, 128, 0, st>>>(pb);
+  ++launches;
+  CountArgs ca;
+  ca.parts = ctx->part_slot.as<PartDesc>();
+  ca.slot_done = ctx->slot_done.as<uint32_t>();
+  ca.acbuf = with_u ? ctx->acbuf.as<uint32_t>() : nullptr;
+  ca.units = ctx->units.as<uint2>();
+  ca.with_u = with_u ? 1 : 0;
+  ca.tot_s = &d->tot_s;
+  ca.tot_m = &d->tot_m;
+  ca.gdir = ctx->gdir.as<uint32_t>();
+  ca.seq4 = ctx->seq4_d();
+  ca.qual = ctx->qual_d();
+  ca.ref = ctx->ref.as<uint8_t>();
+  ca.out = ctx->slot_out.as<uint32_t>();
+  ca.mask = ctx->slot_mask.as<uint32_t>();
+  ca.npass = ctx->slot_npass.as<uint32_t>();
+  ca.n_events = &d->n_events;
+  ca.cell_bits = ctx->cell_bits;
+  ca.uncounted_key = (uint32_t)(ctx->max_cell + 1);
+  ca.min_bq = p.min_bq;
+  ca.min_dp = p.min_dp;
+  ca.min_cc = p.min_cc;
+  ca.min_ac = p.min_ac;
+  // shared memory per CTA: the acx row sits last and is only allocated with --min_ac > 0
+  const size_t sm_p = with_u ? sizeof(TileSmemT<true>) : offsetof(TileSmemT<true>, acx);
+  const size_t sm_u = with_u ? sizeof(TileSmemT<false>) : offsetof(TileSmemT<false>, acx);
+  if (!ctx->k1_attr_set) {
+    LS_CK(cudaFuncSetAttribute(pileup_count_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)sizeof(TileSmemT<true>)));
+    LS_CK(cudaFuncSetAttribute(pileup_count_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)sizeof(TileSmemT<false>)));
+    ctx->k1_attr_set = true;
+  }
+  // 12-bit packed counters unless some cell has > K1_MAX_RUN_PACKED reads in one tile
+  const bool packed = h.long_run == 0;
+  ca.cnt1 = packed ? (1u << K1_CNT_SHIFT) : 0u;
+  if (packed)
+    pileup_count_kernel<true><<<(unsigned)max_parts, K1_THREADS, sm_p, st>>>(ca);
+  else
+    pileup_count_kernel<false><<<(unsigned)max_parts, K1_THREADS, sm_u, st>>>(ca);
+  ++launches;
+  LS_CK(cudaGetLastError());
+  LS_CK(cudaEventRecord(ctx->ev[3], st));
+  LS_CK(ls_scan_exclusive_u32(ctx->slot_npass.as<uint32_t>(), ctx->slot_off.as<uint32_t>(), n_slots, &d->n_sites,
+                              ctx->scan_tmp, st));
+  launches += 1;
+  LS_CK(cudaEventRecord(ctx->ev[4], st));
+  return LS_OK;
+}
+
+// What the device produced in a replayed run against the snapshot its enqueued sizes came from
+static bool replay_matches(const ReplaySnapshot &s, const RunCounters &h, bool pre_compacted) {
+  const RunCounters &m = s.mid;
+  return h.n_aligned == m.n_aligned && h.n_slots == m.n_slots && h.long_run == m.long_run &&
+         h.n_segments == m.n_segments && h.n_pieces == m.n_pieces && h.n_units == m.n_units && h.tot_s == m.tot_s &&
+         h.tot_m == m.tot_m && h.tot_u == m.tot_u && h.n_groups == m.n_groups && h.n_members == m.n_members &&
+         (!pre_compacted || (int64_t)h.n_sites == s.n_sites);
+}
+
 extern "C" int ls_pileup_run(ls_ctx *ctx, const ls_count_params *params, int64_t *n_sites, ls_run_stats *stats) {
   if (!ctx) return LS_E_ARG;
   if (!params) LS_FAIL(LS_E_ARG, "ls_pileup_run: params is null");
@@ -175,342 +419,69 @@ extern "C" int ls_pileup_run(ls_ctx *ctx, const ls_count_params *params, int64_t
   // (the pipeline is deterministic), so the two size read-backs in the middle are skipped and everything is enqueued
   // at once; the sizes are verified against the device counters with the final read-back, and the run is repeated
   // with read-backs if they ever differ.
-  const bool replay = ctx->cache_valid && memcmp(&ctx->cache_params, params, sizeof *params) == 0 && !getenv("LS_NO_REPLAY");
-  // A run that is not a replay overwrites the sizes the next run starts from (n_segments, n_pieces), so the cache only
-  // survives it if the run refreshes it below.
-  if (!replay) ctx->cache_valid = false;
-
-  const int64_t n = ctx->n_reads;
+  const bool replay =
+      ctx->replay.valid && memcmp(&ctx->replay.params, params, sizeof *params) == 0 && !getenv("LS_NO_REPLAY");
+  // A run that is not a replay overwrites the sizes the next run starts from (n_segments, n_pieces), so the snapshot
+  // only survives it if the run refreshes it below.
+  if (!replay) ctx->replay.valid = false;
   ctx->cell_bits = ls_bits_for((uint64_t)(ctx->max_cell + 1));
-  const int tile_bits = ls_bits_for((uint64_t)(ctx->n_tiles_total > 0 ? ctx->n_tiles_total - 1 : 0));
-  SegArgs sa = make_seg_args(ctx, *params, params->min_ac > 0);
 
-  LS_CK(ctx->counters.ensure(128));
-  LS_CK(cudaMemsetAsync(ctx->counters.p, 0, 128, st));
-  unsigned long long *d_aligned = ctx->counters.as<unsigned long long>();
-  unsigned long long *d_events = d_aligned + 1;
-  uint64_t *d_nseg_total = reinterpret_cast<uint64_t *>(d_aligned + 2);
-  uint64_t *d_nslot_total = reinterpret_cast<uint64_t *>(d_aligned + 3);
-  uint32_t *d_nparts = reinterpret_cast<uint32_t *>(d_aligned + 4);
-  uint32_t *d_longrun = reinterpret_cast<uint32_t *>(d_aligned + 5);
-  uint32_t *d_nlight = reinterpret_cast<uint32_t *>(d_aligned + 6);
-  uint32_t *d_capflag = reinterpret_cast<uint32_t *>(d_aligned + 7);
-
+  LS_CK(ctx->counters.ensure(sizeof(RunCounters)));
+  RunCounters *d = ctx->counters.as<RunCounters>();
+  LS_CK(cudaMemsetAsync(d, 0, sizeof *d, st));
   LS_CK(cudaEventRecord(ctx->ev[0], st));
-  uint64_t h_tot[16] = {0};
-  uint64_t h_seg[3] = {0, 0, 0};
-  uint64_t *d_seg_totals = reinterpret_cast<uint64_t *>(d_aligned + 8);  // [0] segments, [1] pieces, [2] units
-  uint64_t *d_tot_s = reinterpret_cast<uint64_t *>(d_aligned + 11);      // sizes of the S / M / U unit streams
-  uint64_t *d_tot_m = reinterpret_cast<uint64_t *>(d_aligned + 12);
-  uint64_t *d_tot_u = reinterpret_cast<uint64_t *>(d_aligned + 13);
-  uint64_t *d_tot_g = reinterpret_cast<uint64_t *>(d_aligned + 14);      // number of (cell, window) groups in M
-  uint64_t *d_tot_ms = reinterpret_cast<uint64_t *>(d_aligned + 15);     // number of run-member segments
-  if (n > 0 && ctx->n_windows > 0) {
-    ctx->n_drop = 0;
-    sa.n_drop = 0;
-    // the depth cap can only fire in a window that fetches more than max_depth records
-    const bool cap_possible = !replay && params->max_depth > 0 && n > (int64_t)params->max_depth;  // replay: known not to fire
-    if (cap_possible) {
-      LS_CK(ctx->rend.ensure((size_t)n * 4));
-      LS_CK(ctx->wcount.ensure((size_t)ctx->n_windows * 4));
-      LS_CK(cudaMemsetAsync(ctx->wcount.p, 0, (size_t)ctx->n_windows * 4, st));
-    }
-    // Output sizes are only known after the walk: start from the previous run's sizes (or an estimate) and
-    // relaunch with exact sizes if the reservation counters ran past the buffers.  A replay has no relaunch: it sizes
-    // the builder with the sizes it will sort and count.
-    uint64_t seg_need = replay ? ctx->cache_seg[0]
-                               : (ctx->n_segments > 0 ? (uint64_t)ctx->n_segments : (uint64_t)n * 5 + 1024);
-    uint64_t piece_need = replay ? ctx->cache_seg[1]
-                                 : (ctx->n_pieces > 0 ? (uint64_t)ctx->n_pieces : (uint64_t)ctx->n_cigar + seg_need);
-    std::vector<uint32_t> wc;
-    bool want_wcount = cap_possible;
-    for (int attempt = 0;; ++attempt) {
-      LS_CK(ctx->segs.ensure((size_t)seg_need * sizeof(Segment)));
-      LS_CK(ctx->pieces.ensure((size_t)piece_need * sizeof(Piece)));
-      LS_CK(ctx->keys_a.ensure((size_t)seg_need * 8));
-      LS_CK(ctx->keys_b.ensure((size_t)seg_need * 8));
-      LS_CK(ctx->vals_a.ensure((size_t)seg_need * 4));
-      LS_CK(ctx->vals_b.ensure((size_t)seg_need * 4));
-      seg_build_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(
-          sa, ctx->segs.as<Segment>(), ctx->keys_a.as<uint64_t>(), ctx->pieces.as<Piece>(), seg_need, piece_need,
-          reinterpret_cast<unsigned long long *>(d_seg_totals), d_aligned, want_wcount ? ctx->rend.as<int32_t>() : nullptr,
-          want_wcount ? ctx->wcount.as<uint32_t>() : nullptr, (uint32_t)params->max_depth, d_capflag);
-      ++launches;
-      LS_CK(cudaGetLastError());
-      if (replay) {
-        memcpy(h_seg, ctx->cache_seg, sizeof h_seg);
-        h_tot[0] = ctx->cache_tot[0];
-        break;
-      }
-      LS_CK(cudaMemcpyAsync(h_tot, ctx->counters.p, 64, cudaMemcpyDeviceToHost, st));
-      LS_CK(cudaMemcpyAsync(h_seg, d_seg_totals, 24, cudaMemcpyDeviceToHost, st));
-      LS_CK(cudaStreamSynchronize(st));
-      bool again = false;
-      if (want_wcount) {
-        want_wcount = false;
-        const bool any = (h_tot[7] & 0xffffffffull) != 0;  // some window fetches more than max_depth records
-        if (any) {
-          wc.resize((size_t)ctx->n_windows);
-          LS_CK(cudaMemcpy(wc.data(), ctx->wcount.p, wc.size() * 4, cudaMemcpyDeviceToHost));
-          int rc = ls_depth_cap_host(ctx, params->min_mq, params->max_depth, wc);
-          if (rc != LS_OK) return rc;
-          if (ctx->n_drop > 0) {  // redo the walk without the dropped (window, read) pairs
-            sa = make_seg_args(ctx, *params, params->min_ac > 0);
-            again = true;
-          }
-        }
-      }
-      if (!again && (h_seg[0] > seg_need || h_seg[1] > piece_need)) {
-        seg_need = h_seg[0] > seg_need ? h_seg[0] : seg_need;
-        piece_need = h_seg[1] > piece_need ? h_seg[1] : piece_need;
-        again = true;
-      }
-      if (!again) break;
-      if (attempt >= 3) LS_FAIL(LS_E_STATE, "ls_pileup_run: segment builder did not converge");
-      LS_CK(cudaMemsetAsync(d_aligned, 0, 8, st));
-      LS_CK(cudaMemsetAsync(d_seg_totals, 0, 24, st));
-    }
-  }
-  const int64_t nseg = (int64_t)h_seg[0];
-  if (nseg >= (int64_t)0xffffffffll || h_seg[1] >= 0xffffffffull || h_seg[2] >= 0xffffffffull)
+  // host copy of the counters: a cold run reads them back after the builder, in the middle and at the end; a replay
+  // takes the middle read-back of the snapshot and reads back only at the end
+  RunCounters h = replay ? ctx->replay.mid : RunCounters{};
+  int rc = build_segments(ctx, *params, replay, d, h, launches);
+  if (rc != LS_OK) return rc;
+  const int64_t nseg = (int64_t)h.n_segments;
+  if (nseg >= (int64_t)0xffffffffll || h.n_pieces >= 0xffffffffull || h.n_units >= 0xffffffffull)
     LS_FAIL(LS_E_ARG, "ls_pileup_run: more than 2^32 segments, pieces or units in one batch");
-  S.n_aligned = (int64_t)h_tot[0];
+  S.n_aligned = (int64_t)h.n_aligned;
   S.n_segments = nseg;
   ctx->n_segments = nseg;
-  ctx->n_pieces = (int64_t)h_seg[1];
+  ctx->n_pieces = (int64_t)h.n_pieces;
   int64_t n_slots = 0;
   if (nseg > 0) {
-    LS_CK(cudaEventRecord(ctx->ev[1], st));
-    LS_CK(ls_radix_sort_pairs(ctx->keys_a.as<uint64_t>(), ctx->keys_b.as<uint64_t>(), ctx->vals_a.as<uint32_t>(),
-                              ctx->vals_b.as<uint32_t>(), nseg, tile_bits + ctx->cell_bits, ctx->rs_hist,
-                              &ctx->sorted_keys, &ctx->sorted_vals, ctx->num_sms, st, &launches));
-    // non-empty tiles -> slots
-    LS_CK(ctx->tile_flag.ensure((size_t)nseg * 4));
-    LS_CK(ctx->tile_rank.ensure((size_t)nseg * 4));
-    const uint64_t cmask = (1ull << ctx->cell_bits) - 1ull;
-    const uint64_t unc = (uint64_t)(uint32_t)(ctx->max_cell + 1);
-    const bool with_u = params->min_ac > 0;
-    uint32_t *os = nullptr, *om = nullptr, *ou = nullptr, *og = nullptr;
     ExpandArgs ea;
-    {
-      // sorted segments -> unit streams (S: single segments, M: same-cell runs, U: uncounted reads): sizes first
-      LS_CK(ctx->offs_s.ensure((size_t)(nseg + 1) * 4));
-      LS_CK(ctx->offs_m.ensure((size_t)(nseg + 1) * 4));
-      LS_CK(ctx->goffs.ensure((size_t)(nseg + 1) * 4));
-      LS_CK(ctx->mrank.ensure((size_t)(nseg + 1) * 4));
-      LS_CK(ctx->mlist.ensure((size_t)(nseg + 1) * 4));
-      if (with_u) LS_CK(ctx->offs_u.ensure((size_t)(nseg + 1) * 4));
-      os = ctx->offs_s.as<uint32_t>();
-      om = ctx->offs_m.as<uint32_t>();
-      og = ctx->goffs.as<uint32_t>();
-      ou = with_u ? ctx->offs_u.as<uint32_t>() : nullptr;
-      uint32_t *mr = ctx->mrank.as<uint32_t>();
-      classify_kernel<<<(unsigned)((nseg + 1 + 255) / 256), 256, 0, st>>>(
-          ctx->sorted_keys, ctx->sorted_vals, ctx->segs.as<Segment>(), nseg, cmask, unc, ctx->cell_bits, os, om, ou, mr,
-          ctx->tile_flag.as<uint32_t>(), d_longrun);
-      ++launches;
-      {
-        // slot ranks, S / M (/ U) stream offsets and run-member ranks: independent scans, one launch
-        LsScanJob jobs[5];
-        int nj = 0;
-        jobs[nj++] = LsScanJob{ctx->tile_flag.as<uint32_t>(), ctx->tile_rank.as<uint32_t>(), nseg, d_nslot_total};
-        jobs[nj++] = LsScanJob{os, os, nseg + 1, d_tot_s};
-        jobs[nj++] = LsScanJob{om, om, nseg + 1, d_tot_m};
-        jobs[nj++] = LsScanJob{mr, mr, nseg + 1, d_tot_ms};
-        if (with_u) jobs[nj++] = LsScanJob{ou, ou, nseg + 1, d_tot_u};
-        LS_CK(ls_scan_exclusive_u32_multi(jobs, nj, ctx->scan_tmp, st));
-        ++launches;
-      }
-      mlist_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(ctx->sorted_keys, nseg, cmask, unc, mr,
-                                                                   ctx->mlist.as<uint32_t>());
-      ++launches;
-      ea.keys = ctx->sorted_keys;
-      ea.vals = ctx->sorted_vals;
-      ea.segs = ctx->segs.as<Segment>();
-      ea.pieces = ctx->pieces.as<Piece>();
-      ea.n = nseg;
-      ea.cmask = cmask;
-      ea.unc = unc;
-      ea.offs_s = os;
-      ea.offs_m = om;
-      ea.offs_u = ou;
-      ea.tot_s = d_tot_s;
-      ea.tot_m = d_tot_m;
-      ea.tot_g = d_tot_g;
-      ea.tot_ms = d_tot_ms;
-      ea.mlist = ctx->mlist.as<uint32_t>();
-      ea.goffs = og;
-      ea.gdir = nullptr;
-      ea.units = nullptr;
-      // one warp per 32 run members; the grid covers the worst case (every segment a run member)
-      LS_CK(cudaMemsetAsync(og, 0, (size_t)(nseg + 1) * 4, st));
-      rungroups_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(ea);
-      ++launches;
-      LS_CK(ls_scan_exclusive_u32(og, og, nseg + 1, d_tot_g, ctx->scan_tmp, st));
-      launches += 1;
-      LS_CK(cudaGetLastError());
+    rc = build_streams(ctx, *params, nseg, d, ea, launches);
+    if (rc != LS_OK) return rc;
+    if (!replay) {
+      rc = read_counters(ctx, d, h);
+      if (rc != LS_OK) return rc;
     }
-    if (replay) {
-      memcpy(h_tot, ctx->cache_tot, sizeof h_tot);
-    } else {
-      LS_CK(cudaMemcpyAsync(h_tot, ctx->counters.p, 128, cudaMemcpyDeviceToHost, st));
-      LS_CK(cudaStreamSynchronize(st));
-    }
-    uint64_t h_mid[16];
-    memcpy(h_mid, h_tot, sizeof h_mid);
-    n_slots = (int64_t)h_tot[3];
-    const bool packed = (h_tot[5] & 0xffffffffull) == 0;
-    LS_CK(ctx->slot_tile.ensure((size_t)n_slots * 8));
-    LS_CK(ctx->slot_lo.ensure((size_t)(n_slots + 1) * 4));
-    slot_fill_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(
-        ctx->sorted_keys, nseg, ctx->cell_bits, ctx->tile_flag.as<uint32_t>(), ctx->tile_rank.as<uint32_t>(), n_slots,
-        ctx->slot_tile.as<int64_t>(), ctx->slot_lo.as<uint32_t>());
-    ++launches;
-    {
-      LS_CK(ctx->units.ensure((size_t)(h_seg[2] + 1) * 8));
-      LS_CK(ctx->gdir.ensure((size_t)(h_tot[14] + 1) * 4));
-      ea.gdir = ctx->gdir.as<uint32_t>();
-      ea.units = ctx->units.as<uint2>();
-      expand_single_kernel<<<(unsigned)((nseg + 255) / 256), 256, 0, st>>>(ea);
-      const int64_t n_members = (int64_t)h_tot[15];
-      if (n_members > 0) expand_runs_kernel<<<(unsigned)((n_members + 255) / 256), 256, 0, st>>>(ea);
-      launches += 2;
-      LS_CK(cudaGetLastError());
-    }
-    LS_CK(cudaEventRecord(ctx->ev[2], st));
-
-    LS_CK(ctx->slot_out.ensure((size_t)n_slots * LS_SITE_WORDS * LS_TILE * 4));
-    LS_CK(ctx->slot_mask.ensure((size_t)n_slots * (LS_TILE / 32) * 4));
-    LS_CK(ctx->slot_npass.ensure((size_t)n_slots * 4));
-    LS_CK(ctx->slot_off.ensure((size_t)n_slots * 4));
-    const int64_t max_parts = n_slots + nseg / K1_PART_SEGS + 1;
-    LS_CK(ctx->part_slot.ensure((size_t)max_parts * sizeof(PartDesc)));
-    LS_CK(ctx->slot_done.ensure((size_t)n_slots * 4));
-    LS_CK(ctx->slot_desc.ensure((size_t)n_slots * sizeof(SlotDesc)));
-    if (params->min_ac > 0) LS_CK(ctx->acbuf.ensure((size_t)n_slots * LS_TILE * 4));
-    LS_CK(cudaMemsetAsync(ctx->part_slot.p, 0xff, (size_t)max_parts * sizeof(PartDesc), st));
-    {
-      PartBuildArgs pb;
-      pb.slot_lo = ctx->slot_lo.as<uint32_t>();
-      pb.slot_tile = ctx->slot_tile.as<int64_t>();
-      pb.n_slots = n_slots;
-      pb.keys = ctx->sorted_keys;
-      pb.offs_s = ctx->offs_s.as<uint32_t>();
-      pb.offs_u = params->min_ac > 0 ? ctx->offs_u.as<uint32_t>() : nullptr;
-      pb.goffs = ctx->goffs.as<uint32_t>();
-      pb.n_windows = ctx->n_windows;
-      pb.wstart = ctx->wstart.as<int32_t>();
-      pb.wend = ctx->wend.as<int32_t>();
-      pb.wtile_base = ctx->wtile_base.as<int64_t>();
-      pb.wref_off = ctx->wref_off.as<uint64_t>();
-      pb.parts = ctx->part_slot.as<PartDesc>();
-      pb.slot_desc = ctx->slot_desc.as<SlotDesc>();
-      pb.wtid = ctx->wtid.as<int32_t>();
-      pb.slot_done = ctx->slot_done.as<uint32_t>();
-      pb.n_parts = d_nparts;
-      pb.n_light = d_nlight;
-      pb.max_parts = (uint32_t)max_parts;
-      pb.out = ctx->slot_out.as<uint32_t>();
-      pb.acbuf = params->min_ac > 0 ? ctx->acbuf.as<uint32_t>() : nullptr;
-      part_build_kernel<<<(unsigned)n_slots, 128, 0, st>>>(pb);
-    }
-    ++launches;
-    CountArgs ca;
-    ca.parts = ctx->part_slot.as<PartDesc>();
-    ca.slot_done = ctx->slot_done.as<uint32_t>();
-    ca.acbuf = params->min_ac > 0 ? ctx->acbuf.as<uint32_t>() : nullptr;
-    ca.units = ctx->units.as<uint2>();
-    ca.with_u = params->min_ac > 0 ? 1 : 0;
-    ca.tot_s = d_tot_s;
-    ca.tot_m = d_tot_m;
-    ca.gdir = ctx->gdir.as<uint32_t>();
-    ca.seq4 = ctx->seq4_d();
-    ca.qual = ctx->qual_d();
-    ca.ref = ctx->ref.as<uint8_t>();
-    ca.out = ctx->slot_out.as<uint32_t>();
-    ca.mask = ctx->slot_mask.as<uint32_t>();
-    ca.npass = ctx->slot_npass.as<uint32_t>();
-    ca.n_events = d_events;
-    ca.cell_bits = ctx->cell_bits;
-    ca.uncounted_key = (uint32_t)(ctx->max_cell + 1);
-    ca.min_bq = params->min_bq;
-    ca.min_dp = params->min_dp;
-    ca.min_cc = params->min_cc;
-    ca.min_ac = params->min_ac;
-    {
-      // shared memory per CTA: the acx row sits last and is only allocated with --min_ac > 0 (without it four CTAs fit)
-      const size_t sm_p = params->min_ac > 0 ? sizeof(TileSmemT<true>) : offsetof(TileSmemT<true>, acx);
-      const size_t sm_u = params->min_ac > 0 ? sizeof(TileSmemT<false>) : offsetof(TileSmemT<false>, acx);
-      // CTA shape of the packed kernel: 8 warps x 3 CTAs / SM (default), 6 warps x 4 CTAs (same warps per SM, more
-      // tiles in flight; needs the acx row absent), 8 warps x 4 CTAs (64 registers: spills, measured slower)
-      static int shape = -1;
-      if (shape < 0) {
-        const char *e = getenv("LS_K1_SHAPE");
-        shape = !e ? 0 : (!strcmp(e, "6x4") ? 1 : (!strcmp(e, "8x4") ? 2 : 0));
-      }
-      if (!ctx->k1_attr_set) {
-        LS_CK(cudaFuncSetAttribute(pileup_count_kernel<true, 3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)sizeof(TileSmemT<true>)));
-        LS_CK(cudaFuncSetAttribute(pileup_count_kernel<true, 4, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)sizeof(TileSmemT<true>)));
-        LS_CK(cudaFuncSetAttribute(pileup_count_kernel<true, 4, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)sizeof(TileSmemT<true>)));
-        LS_CK(cudaFuncSetAttribute(pileup_count_kernel<false, 1, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)sizeof(TileSmemT<false>)));
-        ctx->k1_attr_set = true;
-      }
-      ca.cnt1 = packed ? (1u << K1_CNT_SHIFT) : 0u;
-      // 12-bit packed counters unless some cell has > K1_MAX_RUN_PACKED reads in one tile
-      if (!packed)
-        pileup_count_kernel<false, 1, 8><<<(unsigned)max_parts, 256, sm_u, st>>>(ca);
-      else if (shape == 1)
-        pileup_count_kernel<true, 4, 6><<<(unsigned)max_parts, 192, sm_p, st>>>(ca);
-      else if (shape == 2)
-        pileup_count_kernel<true, 4, 8><<<(unsigned)max_parts, 256, sm_p, st>>>(ca);
-      else
-        pileup_count_kernel<true, 3, 8><<<(unsigned)max_parts, 256, sm_p, st>>>(ca);
-    }
-    ++launches;
-    LS_CK(cudaGetLastError());
-    LS_CK(cudaEventRecord(ctx->ev[3], st));
-    // the number of passing sites goes to counter 2: counter 3 keeps the number of slots for the replay check
-    LS_CK(ls_scan_exclusive_u32(ctx->slot_npass.as<uint32_t>(), ctx->slot_off.as<uint32_t>(), n_slots, d_nseg_total,
-                                ctx->scan_tmp, st));
-    launches += 1;
-    LS_CK(cudaEventRecord(ctx->ev[4], st));
+    const RunCounters mid = h;
+    n_slots = (int64_t)mid.n_slots;
+    rc = count_tiles(ctx, *params, nseg, mid, d, ea, launches);
+    if (rc != LS_OK) return rc;
     // a replayed run knows how many sites will pass: the compaction goes into the same submission, one synchronisation
     // per step instead of two
-    bool pre_compacted = false;
-    if (replay && ctx->cache_n_sites > 0) {
+    const bool pre_compacted = replay && ctx->replay.n_sites > 0;
+    if (pre_compacted) {
       ctx->n_slots = n_slots;
-      const int rc = enqueue_compact(ctx, ctx->cache_n_sites);
+      rc = enqueue_compact(ctx, ctx->replay.n_sites);
       if (rc != LS_OK) return rc;
-      pre_compacted = true;
     }
-    LS_CK(cudaMemcpyAsync(h_tot, ctx->counters.p, 128, cudaMemcpyDeviceToHost, st));
-    LS_CK(cudaStreamSynchronize(st));
+    rc = read_counters(ctx, d, h);
+    if (rc != LS_OK) return rc;
     if (replay) {
-      // what the device actually produced against what the enqueued sizes assumed
-      bool same = h_tot[0] == h_mid[0] && h_tot[3] == h_mid[3] && (h_tot[5] & 0xffffffffull) == (h_mid[5] & 0xffffffffull);
-      if (pre_compacted) same = same && (int64_t)h_tot[2] == ctx->cache_n_sites;
-      for (int k = 8; k < 16; ++k) same = same && h_tot[k] == (k < 11 ? ctx->cache_seg[k - 8] : h_mid[k]);
-      if (!same) {
-        ctx->cache_valid = false;
+      if (!replay_matches(ctx->replay, h, pre_compacted)) {
+        ctx->replay.valid = false;
         return ls_pileup_run(ctx, params, n_sites, stats);
       }
-    } else if (ctx->n_drop == 0 && (h_mid[7] & 0xffffffffull) == 0) {
-      ctx->cache_valid = true;
-      ctx->cache_params = *params;
-      memcpy(ctx->cache_seg, h_seg, sizeof h_seg);
-      memcpy(ctx->cache_tot, h_mid, sizeof h_mid);
-      ctx->cache_n_sites = (int64_t)h_tot[2];
+    } else if (ctx->n_drop == 0 && mid.cap_flag == 0) {  // a replay skips the depth cap: only a run it spared qualifies
+      ctx->replay.valid = true;
+      ctx->replay.params = *params;
+      ctx->replay.mid = mid;
+      ctx->replay.n_sites = (int64_t)h.n_sites;
     }
-    ctx->n_sites = (int64_t)h_tot[2];
+    ctx->n_sites = (int64_t)h.n_sites;
     if (pre_compacted) {
       ctx->compacted = true;
       LS_CK(cudaEventElapsedTime(&S.ms_compact, ctx->ev[5], ctx->ev[6]));  // (the caller counts this launch)
     }
-    S.n_events = (int64_t)h_tot[1];
+    S.n_events = (int64_t)h.n_events;
     LS_CK(cudaEventElapsedTime(&S.ms_segments, ctx->ev[0], ctx->ev[1]));
     LS_CK(cudaEventElapsedTime(&S.ms_sort, ctx->ev[1], ctx->ev[2]));
     LS_CK(cudaEventElapsedTime(&S.ms_count, ctx->ev[2], ctx->ev[3]));
