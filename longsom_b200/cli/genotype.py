@@ -2,11 +2,11 @@
 workflow/scripts/CellClustering/SingleCellGenotype.py and
 workflow/scripts/CellTypeReannotation/HCCVSingleCellGenotype.py).
 
-GPU part: K1' (ls_genotype_count) produces the dense Dp / Alt tensors [site, cell] for every
-candidate site of the run in one pass over the reads, and K2 (ls_betabinom_sf) all
-beta-binomial tails of the (site, cell) pairs with ALT > 0.  The reference does this with one
-pysam pileup per 50 kb bin, a Python dict per (site, barcode) and one scipy call per pair
-(:114-218).  Host part kept byte-compatible: barcode cleaning, bin codes and temp-file order,
+GPU part: K1' (ls_genotype_sparse_run / _fetch) counts Dp / Alt of every touched (site, cell)
+pair of the run in one pass over the reads, and K2 evaluates on the device the beta-binomial
+tails of the pairs with ALT > 0; only the touched pairs come back, and the dense rows are
+expanded from them on the host.  The reference does this with one pysam pileup per 50 kb bin,
+a Python dict per (site, barcode) and one scipy call per pair (:114-218).  Host part kept byte-compatible: barcode cleaning, bin codes and temp-file order,
 Python set iteration order of the sites inside a bin (:112,130), row formatting, and the pandas
 pivots with the natural-sorted index (:342-379)."""
 import argparse

@@ -40,21 +40,10 @@ extern "C" int ls_ctx_destroy(ls_ctx *ctx) {
   if (!ctx) return LS_OK;
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  DBuf *bufs[] = {&ctx->tid,       &ctx->pos,       &ctx->flag,      &ctx->mapq,       &ctx->cell,     &ctx->cigar_off,
-                  &ctx->cigar,     &ctx->base_off,  &ctx->lq,        &ctx->seq4,       &ctx->qual,     &ctx->wtid,
-                  &ctx->wstart,    &ctx->wend,      &ctx->wref_off,  &ctx->ref,        &ctx->wtile_base,
-                  &ctx->segs,      &ctx->pieces,      &ctx->keys_a,    &ctx->keys_b,     &ctx->vals_a,   &ctx->vals_b,
-                  &ctx->rs_hist,   &ctx->scan_tmp,  &ctx->counters,  &ctx->tile_flag,  &ctx->tile_rank, &ctx->slot_tile,
-                  &ctx->slot_lo,   &ctx->slot_out,  &ctx->slot_mask, &ctx->slot_npass, &ctx->slot_off, &ctx->drop_keys,
-                  &ctx->out_tid,   &ctx->out_pos,   &ctx->out_ref,   &ctx->out_counts, &ctx->l2_scratch, &ctx->g_a,
-                  &ctx->g_b,       &ctx->g_c,       &ctx->g_d,       &ctx->g_e,        &ctx->rend,     &ctx->wcount,   &ctx->part_slot, &ctx->slot_done, &ctx->slot_desc, &ctx->acbuf, &ctx->offs_s, &ctx->offs_m, &ctx->offs_u, &ctx->units, &ctx->goffs, &ctx->gdir, &ctx->mrank, &ctx->mlist, &ctx->gs_cnt, &ctx->gs_hits_a, &ctx->gs_hits_b, &ctx->gs_flag,
-                  &ctx->gs_tup, &ctx->gs_p, &ctx->gs_skip};
-  for (DBuf *b : bufs) b->release();
-  for (DBuf &b : ctx->site_tab) b.release();
   for (auto &ev : ctx->ev)
     if (ev) cudaEventDestroy(ev);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  delete ctx;
+  delete ctx;  // frees every device buffer
   return LS_OK;
 }
 

@@ -169,10 +169,7 @@ extern "C" int ls_betabinom_sf(ls_ctx *ctx, const int32_t *k, const int32_t *n, 
     bk[j] = k[big[j]];
     bn[j] = n[big[j]];
   }
-  const int32_t *k_all = k, *n_all = n;
   double *p_all = p;
-  (void)k_all;
-  (void)n_all;
   k = bk.data();
   n = bn.data();
   p = bp.data();

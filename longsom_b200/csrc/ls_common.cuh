@@ -21,14 +21,17 @@ enum { OP_M = 0, OP_I = 1, OP_D = 2, OP_N = 3, OP_S = 4, OP_H = 5, OP_P = 6, OP_
 #define LS_FLAG_REVERSE 0x10u
 #define LS_FLAG_SUPPL 0x800u
 
+// A device buffer that grows on demand and is freed with its owner.
 struct DBuf {
   void *p = nullptr;
   size_t cap = 0;
+  DBuf() = default;
+  DBuf(const DBuf &) = delete;
+  DBuf &operator=(const DBuf &) = delete;
+  ~DBuf() { release(); }
   cudaError_t ensure(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
+    release();
     size_t want = bytes + bytes / 8 + 256;
     cudaError_t e = cudaMalloc(&p, want);
     if (e != cudaSuccess) {
@@ -102,6 +105,29 @@ struct RunCounters {
 };
 static_assert(sizeof(RunCounters) == 128, "RunCounters layout");
 
+// Device counters of one genotype call (the start of ctx->counters, zeroed by ls_genotype_count and
+// ls_genotype_sparse_run)
+struct GenoCounters {
+  unsigned long long n_events;  // real hits (genotype_kernel)
+  uint64_t n_slots;             // hit slots: total of the scan of the per-read candidate counts
+  uint64_t n_tuples;            // touched (site, cell) pairs: total of the scan of the first-hit flags
+  alignas(8) uint32_t n_big;    // pairs K2 leaves to the staged path (p = -1)
+};
+static_assert(sizeof(GenoCounters) == 32, "GenoCounters layout");
+
+// What K1' keeps between its kernels, and between ls_genotype_sparse_run and ls_genotype_sparse_fetch
+struct GenoState {
+  DBuf site_key, alt_class, site_bin, skip;  // site table of the last call: keys, ALT classes, bins, skip_p flags
+  DBuf slots;           // per read: its candidate sites, scanned in place into its first hit slot
+  DBuf hits_a, hits_b;  // hit keys and the radix sort's second buffer
+  DBuf flag;            // first hit of a pair: flag, scanned in place into the pair's tuple index
+  DBuf tup, p;          // tuples: site, cell, Dp, Alt and the K2 query k, each [n_tuples]; p [n_tuples]
+  DBuf dp, alt;         // dense [site][cell] tensors of ls_genotype_count
+  int64_t n_tuples = 0;
+  bool have_tuples = false;
+  double alpha = 0.0, beta = 0.0;
+};
+
 // What a replay of ls_pileup_run takes from the last run on the batch that it can stand for
 struct ReplaySnapshot {
   bool valid = false;
@@ -151,15 +177,12 @@ struct ls_ctx {
   // ---- fetch / misc scratch ----
   DBuf out_tid, out_pos, out_ref, out_counts;
   DBuf l2_scratch;
-  DBuf g_a, g_b, g_c, g_d, g_e;  // genotype / betabinom / mask scratch
+  DBuf g_a, g_b, g_c, g_d, g_e;  // scratch of K2 and K3: nothing lives in them across an entry-point call
   // K3: resident sorted site tables (slot LS_SITE_TABLES is the scratch table of the one-shot ls_site_mask)
   DBuf site_tab[LS_SITE_TABLES + 1];
   int64_t site_tab_n[LS_SITE_TABLES + 1] = {};
   bool site_tab_ok[LS_SITE_TABLES + 1] = {};
-  DBuf gs_cnt, gs_hits_a, gs_hits_b, gs_flag, gs_tup, gs_p, gs_skip;  // sparse genotyping
-  int64_t n_tuples = 0;
-  bool have_tuples = false;
-  double gs_alpha = 0.0, gs_beta = 0.0;
+  GenoState geno;  // K1'
 };
 
 #define LS_CK(call)                                                                        \

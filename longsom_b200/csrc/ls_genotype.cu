@@ -8,9 +8,13 @@
 //
 // Design: candidate sites are sparse (<= 2e5) while reads are dense, so the scan is
 // read-major: one thread walks one read's CIGAR, binary-searches the sorted site table for
-// sites inside each reference-consuming op and scatters with global atomics into the dense
-// [site][cell] tensors (one int32 add per hit; hits are ~depth x sites, tiny next to HBM).
+// sites inside each reference-consuming op and either scatters with global atomics into the
+// dense [site][cell] tensors (ls_genotype_count; one int32 add per hit, and hits are ~depth x
+// sites, tiny next to HBM) or writes one key per hit, which a sort reduces to the touched
+// (site, cell) pairs (ls_genotype_sparse_run).
 // Bases that cover no candidate site are never loaded.
+#include <type_traits>
+
 #include "ls_common.cuh"
 
 struct GenoArgs {
@@ -29,20 +33,19 @@ struct GenoArgs {
   int min_bq, min_mq, alt_only;
   const uint64_t *drop_keys;  // (bin<<32 | read) removed by the depth cap
   int64_t n_drop;
-  int32_t *dp, *alt;            // dense [site][cell] tensors (dense mode), else null
-  uint32_t *hit_cnt;            // sparse pass 1: hits per read
-  const uint32_t *hit_off;      // sparse pass 2: first hit slot of every read (exclusive scan of hit_cnt)
-  uint64_t *hits;               // sparse pass 2: (site * n_cells + cell) << 1 | (class == ALT_expected)
+  int32_t *dp, *alt;            // dense [site][cell] tensors (genotype_kernel<void>), else null
+  const uint32_t *hit_off;      // first hit slot of every read (exclusive scan of its candidate sites)
+  void *hits;                   // hit keys: (site * n_cells + cell) << 1 | (class == ALT_expected)
   uint64_t sentinel;            // key of an unused slot (n_sites * n_cells * 2: behind every real key)
-  uint32_t *hits32;             // the same as 32-bit keys (MODE 3: when n_sites * n_cells * 2 < 2^32 -- half the sort traffic)
   unsigned long long *n_events;
 };
 
-__device__ __forceinline__ int64_t lower_site(const GenoArgs &a, uint64_t key) {
-  int64_t lo = 0, hi = a.n_sites;
+// first index i of the sorted keys[0, n) with keys[i] >= key
+__device__ __forceinline__ int64_t lower_key(const uint64_t *__restrict__ keys, int64_t n, uint64_t key) {
+  int64_t lo = 0, hi = n;
   while (lo < hi) {
-    int64_t m = (lo + hi) >> 1;
-    if (a.site_key[m] < key)
+    const int64_t m = (lo + hi) >> 1;
+    if (keys[m] < key)
       lo = m + 1;
     else
       hi = m;
@@ -52,26 +55,21 @@ __device__ __forceinline__ int64_t lower_site(const GenoArgs &a, uint64_t key) {
 
 __device__ __forceinline__ bool geno_dropped(const GenoArgs &a, uint32_t bin, uint32_t r) {
   if (a.n_drop == 0) return false;
-  uint64_t key = ((uint64_t)bin << 32) | r;
-  int64_t lo = 0, hi = a.n_drop;
-  while (lo < hi) {
-    int64_t m = (lo + hi) >> 1;
-    if (a.drop_keys[m] < key)
-      lo = m + 1;
-    else
-      hi = m;
-  }
-  return lo < a.n_drop && a.drop_keys[lo] == key;
+  const uint64_t key = ((uint64_t)bin << 32) | r;
+  const int64_t i = lower_key(a.drop_keys, a.n_drop, key);
+  return i < a.n_drop && a.drop_keys[i] == key;
 }
 
-// MODE 0: dense atomics, 1: count the read's hits, 2 / 3: write them at the read's slots as 64-bit / 32-bit keys
-template <int MODE>
+// K = void: dense atomics into dp / alt.  K = uint32_t / uint64_t: the read's hits as keys of that width at its slots,
+// and the sentinel in the slots it does not use.
+template <typename K>
 __global__ void __launch_bounds__(256) genotype_kernel(GenoArgs a) {
+  constexpr bool DENSE = std::is_void<K>::value;
   int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long nev = 0;
   if (r < a.n_reads) {
-    uint64_t *hp = MODE == 2 ? a.hits + a.hit_off[r] : nullptr;
-    uint32_t *hp32 = MODE == 3 ? a.hits32 + a.hit_off[r] : nullptr;
+    K *hp = nullptr;
+    if constexpr (!DENSE) hp = static_cast<K *>(a.hits) + a.hit_off[r];
     const uint32_t flag = a.flag[r];
     const int32_t cell = a.cell[r];
     const int32_t tid = a.tid[r];
@@ -82,7 +80,7 @@ __global__ void __launch_bounds__(256) genotype_kernel(GenoArgs a) {
       uint32_t y = 0;
       const uint64_t boff = a.base_off[r];
       const uint32_t lq = (uint32_t)a.lq[r];
-      int64_t s = lower_site(a, ((uint64_t)(uint32_t)tid << 32) | (uint32_t)x);
+      int64_t s = lower_key(a.site_key, a.n_sites, ((uint64_t)(uint32_t)tid << 32) | (uint32_t)x);
       for (uint32_t k = k0; k < kend && s < a.n_sites; ++k) {
         const uint32_t c = a.cigar[k];
         const uint32_t op = c & 15u;
@@ -115,13 +113,11 @@ __global__ void __launch_bounds__(256) genotype_kernel(GenoArgs a) {
               const int ac = a.alt_class[s];
               const bool use = a.alt_only ? (cls == ac && cls != LS_CLASS_NA) : (cls != LS_CLASS_NA && cls != LS_CLASS_O);
               if (use) {
-                if (MODE == 0) {
+                if constexpr (DENSE) {
                   atomicAdd(&a.dp[(size_t)s * a.n_cells + cell], 1);
                   if (cls == ac) atomicAdd(&a.alt[(size_t)s * a.n_cells + cell], 1);
-                } else if (MODE == 2) {
-                  *hp++ = (((uint64_t)s * (uint64_t)a.n_cells + (uint64_t)cell) << 1) | (cls == ac ? 1u : 0u);
-                } else if (MODE == 3) {
-                  *hp32++ = (((uint32_t)s * (uint32_t)a.n_cells + (uint32_t)cell) << 1) | (cls == ac ? 1u : 0u);
+                } else {
+                  *hp++ = (((K)s * (K)a.n_cells + (K)cell) << 1) | (cls == ac ? 1u : 0u);
                 }
                 ++nev;
               }
@@ -139,11 +135,8 @@ __global__ void __launch_bounds__(256) genotype_kernel(GenoArgs a) {
         }
       }
     }
-    if (MODE == 1) a.hit_cnt[r] = (uint32_t)nev;
-    if (MODE == 2)
-      for (uint64_t *e = a.hits + a.hit_off[r + 1]; hp < e; ++hp) *hp = a.sentinel;
-    if (MODE == 3)
-      for (uint32_t *e = a.hits32 + a.hit_off[r + 1]; hp32 < e; ++hp32) *hp32 = (uint32_t)a.sentinel;
+    if constexpr (!DENSE)
+      for (K *e = static_cast<K *>(a.hits) + a.hit_off[r + 1]; hp < e; ++hp) *hp = (K)a.sentinel;
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) nev += __shfl_xor_sync(0xffffffffu, nev, o);
@@ -209,18 +202,6 @@ struct CandArgs {          // sparse path: slots per read = candidate sites insi
   int32_t n_cells;
   uint32_t *cand_cnt;      // null: bin counts only
 };
-
-__device__ __forceinline__ int64_t lower_key(const uint64_t *__restrict__ keys, int64_t n, uint64_t key) {
-  int64_t lo = 0, hi = n;
-  while (lo < hi) {
-    const int64_t m = (lo + hi) >> 1;
-    if (keys[m] < key)
-      lo = m + 1;
-    else
-      hi = m;
-  }
-  return lo;
-}
 
 __global__ void __launch_bounds__(256) bin_fetch_count_kernel(int64_t n, const int32_t *__restrict__ tid,
                                                               const int32_t *__restrict__ pos,
@@ -288,19 +269,19 @@ static int geno_depth_cap(ls_ctx *ctx, const std::vector<int32_t> &btid, const s
     const size_t nb = cap_possible ? btid.size() : 0;
     LS_CK(ctx->wcount.ensure(nb * 4 * 4 + 16));
     int32_t *d_bt = ctx->wcount.as<int32_t>(), *d_bs = d_bt + nb, *d_be = d_bs + nb;
-    uint32_t *d_cnt = reinterpret_cast<uint32_t *>(d_be + nb);  // [nb] counts + 1 flag word
+    uint32_t *d_fetch = reinterpret_cast<uint32_t *>(d_be + nb), *d_over = d_fetch + nb;
     LS_CK(cudaMemcpyAsync(d_bt, btid.data(), nb * 4, cudaMemcpyHostToDevice, st));
     LS_CK(cudaMemcpyAsync(d_bs, bstart.data(), nb * 4, cudaMemcpyHostToDevice, st));
     LS_CK(cudaMemcpyAsync(d_be, bend.data(), nb * 4, cudaMemcpyHostToDevice, st));
-    LS_CK(cudaMemsetAsync(d_cnt, 0, nb * 4 + 4, st));
+    LS_CK(cudaMemsetAsync(d_fetch, 0, nb * 4 + 4, st));
     bin_fetch_count_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(
         n, ctx->tid.as<int32_t>(), ctx->pos.as<int32_t>(), ctx->flag.as<uint16_t>(), ctx->mapq.as<uint8_t>(),
         ctx->cigar_off.as<uint32_t>(), ctx->cigar.as<uint32_t>(), (int64_t)nb, d_bt, d_bs, d_be, min_mq,
-        (uint32_t)max_depth, d_cnt, d_cnt + nb, ca);
+        (uint32_t)max_depth, d_fetch, d_over, ca);
     LS_CK(cudaGetLastError());
     if (!cap_possible) return LS_OK;
     uint32_t over = 0;
-    LS_CK(cudaMemcpyAsync(&over, d_cnt + nb, 4, cudaMemcpyDeviceToHost, st));
+    LS_CK(cudaMemcpyAsync(&over, d_over, 4, cudaMemcpyDeviceToHost, st));
     LS_CK(cudaStreamSynchronize(st));
     if (!over) return LS_OK;
   }
@@ -319,8 +300,20 @@ struct GenoSites {
   std::vector<int32_t> btid, bstart, bend;
 };
 
-static int geno_prepare_sites(ls_ctx *ctx, const int32_t *site_tid, const int32_t *site_pos, int64_t n_sites, int32_t bin,
-                              GenoSites &g) {
+// The checks both entry points begin with; `who` names the entry point in the errors.
+static int geno_check(ls_ctx *ctx, const char *who, const ls_geno_params *params, int64_t n_sites, int32_t n_cells) {
+  const std::string w = who;
+  if (!params) LS_FAIL(LS_E_ARG, w + ": params is null");
+  if (!ctx->have_batch) LS_FAIL(LS_E_STATE, w + ": no batch uploaded");
+  if (n_sites < 0 || n_cells < 0) LS_FAIL(LS_E_ARG, w + ": negative size");
+  return LS_OK;
+}
+
+// Site setup of both entry points: the site table goes to ctx->geno and the counters are zeroed.  g keeps the host
+// side, which the uploads read until the stream is next synchronized, and the bins for the depth cap.
+static int geno_setup(ls_ctx *ctx, const int32_t *site_tid, const int32_t *site_pos, const uint8_t *alt_class,
+                      int64_t n_sites, const ls_geno_params *params, GenoSites &g) {
+  const int32_t bin = params->bin_size > 0 ? params->bin_size : 50000;
   g.keys.resize((size_t)n_sites);
   g.sbin.resize((size_t)n_sites);
   for (int64_t i = 0; i < n_sites; ++i) {
@@ -338,10 +331,23 @@ static int geno_prepare_sites(ls_ctx *ctx, const int32_t *site_tid, const int32_
     }
     g.sbin[i] = (uint32_t)(g.btid.size() - 1);
   }
+  LS_CK(cudaSetDevice(ctx->device));
+  GenoState &gs = ctx->geno;
+  cudaStream_t st = ctx->stream;
+  LS_CK(gs.site_key.ensure((size_t)n_sites * 8));
+  LS_CK(gs.alt_class.ensure((size_t)n_sites));
+  LS_CK(gs.site_bin.ensure((size_t)n_sites * 4));
+  LS_CK(ctx->counters.ensure(sizeof(GenoCounters)));
+  LS_CK(cudaMemcpyAsync(gs.site_key.p, g.keys.data(), (size_t)n_sites * 8, cudaMemcpyHostToDevice, st));
+  LS_CK(cudaMemcpyAsync(gs.alt_class.p, alt_class, (size_t)n_sites, cudaMemcpyHostToDevice, st));
+  LS_CK(cudaMemcpyAsync(gs.site_bin.p, g.sbin.data(), (size_t)n_sites * 4, cudaMemcpyHostToDevice, st));
+  LS_CK(cudaMemsetAsync(ctx->counters.p, 0, sizeof(GenoCounters), st));
   return LS_OK;
 }
 
-static void geno_fill_args(ls_ctx *ctx, GenoArgs &a, int64_t n_sites, int32_t n_cells, const ls_geno_params *params) {
+// The kernel arguments of a call: the batch, the site table in ctx->geno and the depth cap's drops; no output yet
+static GenoArgs geno_args(ls_ctx *ctx, int64_t n_sites, int32_t n_cells, const ls_geno_params *params) {
+  GenoArgs a = {};
   a.n_reads = ctx->n_reads;
   a.tid = ctx->tid.as<int32_t>();
   a.pos = ctx->pos.as<int32_t>();
@@ -354,9 +360,9 @@ static void geno_fill_args(ls_ctx *ctx, GenoArgs &a, int64_t n_sites, int32_t n_
   a.base_off = ctx->base_off.as<uint64_t>();
   a.seq4 = ctx->seq4_d();
   a.qual = ctx->qual_d();
-  a.site_key = ctx->g_a.as<uint64_t>();
-  a.alt_class = ctx->g_b.as<uint8_t>();
-  a.site_bin = ctx->g_e.as<uint32_t>();
+  a.site_key = ctx->geno.site_key.as<uint64_t>();
+  a.alt_class = ctx->geno.alt_class.as<uint8_t>();
+  a.site_bin = ctx->geno.site_bin.as<uint32_t>();
   a.n_sites = n_sites;
   a.n_cells = n_cells;
   a.min_bq = params->min_bq;
@@ -364,151 +370,145 @@ static void geno_fill_args(ls_ctx *ctx, GenoArgs &a, int64_t n_sites, int32_t n_
   a.alt_only = params->alt_only;
   a.drop_keys = ctx->drop_keys.as<uint64_t>();
   a.n_drop = ctx->n_drop;
-  a.dp = a.alt = nullptr;
-  a.hit_cnt = nullptr;
-  a.hit_off = nullptr;
-  a.hits = nullptr;
-  a.hits32 = nullptr;
-  a.sentinel = 0;
-  a.n_events = ctx->counters.as<unsigned long long>();
+  a.n_events = &ctx->counters.as<GenoCounters>()->n_events;
+  return a;
+}
+
+static int read_counters(ls_ctx *ctx, const GenoCounters *d, GenoCounters &h) {
+  LS_CK(cudaMemcpyAsync(&h, d, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+  LS_CK(cudaStreamSynchronize(ctx->stream));
+  return LS_OK;
 }
 
 int ls_betabinom_device(ls_ctx *ctx, const int32_t *d_k, const int32_t *d_n, double a, double b, double *d_p, int64_t m,
                         uint32_t *d_nbig);
 
 // ---- sparse genotyping: only the touched (site, cell) pairs leave the device -------------------------------------
+// Phase 1: per read, how many candidate sites lie inside [pos, reference end) -- an upper bound of its hits, which
+// sizes its slots -- scanned into its first slot.  The same walk over the CIGARs gives the depth cap its per-bin fetch
+// counts, so there is no separate counting pass over the bases.
+static int count_slots(ls_ctx *ctx, const GenoSites &g, int64_t n_sites, int32_t n_cells, const ls_geno_params *params,
+                       const uint8_t *skip_p, GenoCounters *d, GenoCounters &h) {
+  GenoState &gs = ctx->geno;
+  cudaStream_t st = ctx->stream;
+  const int64_t n = ctx->n_reads;
+  LS_CK(gs.skip.ensure((size_t)n_sites));
+  LS_CK(gs.slots.ensure((size_t)(n + 1) * 4));
+  if (skip_p) LS_CK(cudaMemcpyAsync(gs.skip.p, skip_p, (size_t)n_sites, cudaMemcpyHostToDevice, st));
+  LS_CK(cudaMemsetAsync(gs.slots.as<uint32_t>() + n, 0, 4, st));
+  LS_CK(cudaEventRecord(ctx->ev[0], st));
+  const CandArgs ca = {gs.site_key.as<uint64_t>(), n_sites, ctx->cell.as<int32_t>(), n_cells, gs.slots.as<uint32_t>()};
+  int rc = geno_depth_cap(ctx, g.btid, g.bstart, g.bend, params->min_mq, params->max_depth, ca);
+  if (rc != LS_OK) return rc;
+  LS_CK(ls_scan_exclusive_u32(gs.slots.as<uint32_t>(), gs.slots.as<uint32_t>(), n + 1, &d->n_slots, ctx->scan_tmp, st));
+  return read_counters(ctx, d, h);
+}
+
+static cudaError_t sort_hits(ls_ctx *ctx, uint32_t *a, uint32_t *b, int64_t n, int bits, uint32_t **sorted, int *launches) {
+  return ls_radix_sort_keys32(a, b, n, bits, ctx->rs_hist, sorted, ctx->num_sms, ctx->stream, launches);
+}
+static cudaError_t sort_hits(ls_ctx *ctx, uint64_t *a, uint64_t *b, int64_t n, int bits, uint64_t **sorted, int *launches) {
+  return ls_radix_sort_keys(a, b, n, bits, ctx->rs_hist, sorted, ctx->num_sms, ctx->stream, launches);
+}
+
+// Phase 2: the hits of every read as K-wide keys in its nh slots, sorted, and reduced to one (site, cell, Dp, Alt, k)
+// tuple per touched pair.  h gets the counters after the tuple count.
+template <typename K>
+static int hits_to_tuples(ls_ctx *ctx, GenoArgs a, int64_t nh, bool skip, GenoCounters *d, GenoCounters &h,
+                          int &launches) {
+  GenoState &gs = ctx->geno;
+  cudaStream_t st = ctx->stream;
+  const K sentinel = (K)a.sentinel;
+  LS_CK(gs.hits_a.ensure((size_t)nh * sizeof(K)));
+  LS_CK(gs.hits_b.ensure((size_t)nh * sizeof(K)));
+  LS_CK(gs.flag.ensure((size_t)(nh + 1) * 4));
+  a.hit_off = gs.slots.as<uint32_t>();
+  a.hits = gs.hits_a.p;
+  genotype_kernel<K><<<(unsigned)((a.n_reads + 255) / 256), 256, 0, st>>>(a);
+  K *sorted = nullptr;
+  LS_CK(sort_hits(ctx, gs.hits_a.as<K>(), gs.hits_b.as<K>(), nh, ls_bits_for(a.sentinel), &sorted, &launches));
+  uint32_t *flag = gs.flag.as<uint32_t>();
+  hit_flag_kernel<K><<<(unsigned)((nh + 1 + 255) / 256), 256, 0, st>>>(sorted, nh, sentinel, flag);
+  LS_CK(ls_scan_exclusive_u32(flag, flag, nh + 1, &d->n_tuples, ctx->scan_tmp, st));
+  int rc = read_counters(ctx, d, h);
+  if (rc != LS_OK) return rc;
+  const int64_t nt = (int64_t)h.n_tuples;
+  LS_CK(gs.tup.ensure((size_t)nt * 5 * 4 + 16));
+  LS_CK(gs.p.ensure((size_t)nt * 8 + 16));
+  int32_t *t_site = gs.tup.as<int32_t>(), *t_cell = t_site + nt, *t_dp = t_cell + nt, *t_alt = t_dp + nt, *t_k = t_alt + nt;
+  hit_reduce_kernel<K><<<(unsigned)((nh + 255) / 256), 256, 0, st>>>(
+      sorted, nh, sentinel, flag, a.n_cells, skip ? gs.skip.as<uint8_t>() : nullptr, t_site, t_cell, t_dp, t_alt, t_k);
+  launches += 4;
+  LS_CK(cudaGetLastError());
+  return LS_OK;
+}
+
 extern "C" int ls_genotype_sparse_run(ls_ctx *ctx, const int32_t *site_tid, const int32_t *site_pos,
                                       const uint8_t *alt_class, const uint8_t *skip_p, int64_t n_sites, int32_t n_cells,
                                       const ls_geno_params *params, double alpha, double beta, int64_t *n_tuples,
                                       ls_run_stats *stats) {
   if (!ctx) return LS_E_ARG;
-  if (!params) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_run: params is null");
-  if (!ctx->have_batch) LS_FAIL(LS_E_STATE, "ls_genotype_sparse_run: no batch uploaded");
-  if (n_sites < 0 || n_cells < 0) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_run: negative size");
+  int rc = geno_check(ctx, "ls_genotype_sparse_run", params, n_sites, n_cells);
+  if (rc != LS_OK) return rc;
   if (!(alpha > 0.0) || !(beta > 0.0)) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_run: alpha and beta must be > 0");
+  GenoState &gs = ctx->geno;
   ls_run_stats S;
   memset(&S, 0, sizeof S);
-  ctx->n_tuples = 0;
-  ctx->have_tuples = false;
-  ctx->gs_alpha = alpha;
-  ctx->gs_beta = beta;
+  gs.n_tuples = 0;
+  gs.have_tuples = false;
+  gs.alpha = alpha;
+  gs.beta = beta;
   if (n_tuples) *n_tuples = 0;
   if (n_sites == 0 || n_cells == 0 || ctx->n_reads == 0) {
-    ctx->have_tuples = true;
+    gs.have_tuples = true;
     if (stats) *stats = S;
     return LS_OK;
   }
   if (!site_tid || !site_pos || !alt_class) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_run: null array");
   if ((uint64_t)n_sites * (uint64_t)n_cells >= ((uint64_t)1 << 62)) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_run: too many pairs");
-  const int32_t bin = params->bin_size > 0 ? params->bin_size : 50000;
   GenoSites g;
-  int rc = geno_prepare_sites(ctx, site_tid, site_pos, n_sites, bin, g);
+  rc = geno_setup(ctx, site_tid, site_pos, alt_class, n_sites, params, g);
   if (rc != LS_OK) return rc;
-  LS_CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int64_t n = ctx->n_reads;
-  LS_CK(ctx->g_a.ensure((size_t)n_sites * 8));
-  LS_CK(ctx->g_b.ensure((size_t)n_sites));
-  LS_CK(ctx->g_e.ensure((size_t)n_sites * 4));
-  LS_CK(ctx->gs_skip.ensure((size_t)n_sites));
-  LS_CK(ctx->gs_cnt.ensure((size_t)(n + 1) * 4));
-  LS_CK(ctx->counters.ensure(128));
-  LS_CK(cudaMemcpyAsync(ctx->g_a.p, g.keys.data(), (size_t)n_sites * 8, cudaMemcpyHostToDevice, st));
-  LS_CK(cudaMemcpyAsync(ctx->g_b.p, alt_class, (size_t)n_sites, cudaMemcpyHostToDevice, st));
-  LS_CK(cudaMemcpyAsync(ctx->g_e.p, g.sbin.data(), (size_t)n_sites * 4, cudaMemcpyHostToDevice, st));
-  if (skip_p) LS_CK(cudaMemcpyAsync(ctx->gs_skip.p, skip_p, (size_t)n_sites, cudaMemcpyHostToDevice, st));
-  LS_CK(cudaMemsetAsync(ctx->counters.p, 0, 128, st));
-  LS_CK(cudaMemsetAsync((uint32_t *)ctx->gs_cnt.p + n, 0, 4, st));
-  LS_CK(cudaEventRecord(ctx->ev[0], st));
-  // One walk over the CIGARs: per-bin fetch counts for the depth cap and, per read, how many candidate sites lie
-  // inside [pos, reference end) -- an upper bound of its hits, which sizes its slots (the slots a read does not use
-  // are filled with a key that sorts behind every real one).  No separate counting pass over the bases.
-  CandArgs ca;
-  ca.site_key = ctx->g_a.as<uint64_t>();
-  ca.n_sites = n_sites;
-  ca.cell = ctx->cell.as<int32_t>();
-  ca.n_cells = n_cells;
-  ca.cand_cnt = ctx->gs_cnt.as<uint32_t>();
-  rc = geno_depth_cap(ctx, g.btid, g.bstart, g.bend, params->min_mq, params->max_depth, ca);
+  GenoCounters *d = ctx->counters.as<GenoCounters>(), h;
+  rc = count_slots(ctx, g, n_sites, n_cells, params, skip_p, d, h);
   if (rc != LS_OK) return rc;
-  GenoArgs a;
-  geno_fill_args(ctx, a, n_sites, n_cells, params);
-  unsigned long long *d_cnt = ctx->counters.as<unsigned long long>();
-  uint64_t *d_nhits = reinterpret_cast<uint64_t *>(d_cnt + 1), *d_ntup = reinterpret_cast<uint64_t *>(d_cnt + 2);
-  uint32_t *d_nbig = reinterpret_cast<uint32_t *>(d_cnt + 3);
-  const unsigned grid = (unsigned)((n + 255) / 256);
-  LS_CK(ls_scan_exclusive_u32(ctx->gs_cnt.as<uint32_t>(), ctx->gs_cnt.as<uint32_t>(), n + 1, d_nhits, ctx->scan_tmp, st));
-  uint64_t h[4] = {0, 0, 0, 0};
-  LS_CK(cudaMemcpyAsync(h, d_cnt, 32, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaStreamSynchronize(st));
-  const int64_t nh = (int64_t)h[1];  // slots (>= hits)
-  int launches = 2;
-  int64_t nt = 0;
+  const int64_t nh = (int64_t)h.n_slots;  // slots (>= hits)
   if (nh >= (int64_t)0xffffffffll) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_run: more than 2^32 hits; split the site list");
+  // The stats keep the meaning callers and bench.py read: ms_count from the slot count to the end of the reduction,
+  // ms_sort the K2 tails, n_events the real hits, n_segments the tuples.  count_launches counts the slot count and its
+  // scan, then, if there are slots, genotype_kernel, the radix sort, hit_flag_kernel, the scan, hit_reduce_kernel and
+  // K2's 2 or 4 launches; a capped call's read_end_kernel is not counted.
+  int launches = 2;
   if (nh > 0) {
     // keys that fit 32 bits are written, sorted and reduced as 32-bit words (half the traffic of the hit sort)
     const uint64_t key_span = (uint64_t)n_sites * (uint64_t)n_cells * 2u;
-    const bool k32 = key_span < (1ull << 32) && !getenv("LS_GENO_KEYS64");
-    const size_t ksz = k32 ? 4 : 8;
-    LS_CK(ctx->gs_hits_a.ensure((size_t)nh * ksz));
-    LS_CK(ctx->gs_hits_b.ensure((size_t)nh * ksz));
-    LS_CK(ctx->gs_flag.ensure((size_t)(nh + 1) * 4));
-    // pass 2: the hits themselves
-    a.hit_cnt = nullptr;
-    a.hit_off = ctx->gs_cnt.as<uint32_t>();
-    a.hits = ctx->gs_hits_a.as<uint64_t>();
-    a.hits32 = ctx->gs_hits_a.as<uint32_t>();
-    LS_CK(cudaMemsetAsync(d_cnt, 0, 8, st));
-    const int key_bits = ls_bits_for(key_span);
-    uint64_t *sorted = nullptr;
-    uint32_t *sorted32 = nullptr;
+    GenoArgs a = geno_args(ctx, n_sites, n_cells, params);
     a.sentinel = key_span;
-    if (k32) {
-      genotype_kernel<3><<<grid, 256, 0, st>>>(a);
-      LS_CK(ls_radix_sort_keys32(ctx->gs_hits_a.as<uint32_t>(), ctx->gs_hits_b.as<uint32_t>(), nh, key_bits, ctx->rs_hist,
-                                 &sorted32, ctx->num_sms, st, &launches));
-      hit_flag_kernel<uint32_t><<<(unsigned)((nh + 1 + 255) / 256), 256, 0, st>>>(sorted32, nh, (uint32_t)key_span, ctx->gs_flag.as<uint32_t>());
-    } else {
-      genotype_kernel<2><<<grid, 256, 0, st>>>(a);
-      LS_CK(ls_radix_sort_keys(ctx->gs_hits_a.as<uint64_t>(), ctx->gs_hits_b.as<uint64_t>(), nh, key_bits, ctx->rs_hist, &sorted,
-                               ctx->num_sms, st, &launches));
-      hit_flag_kernel<uint64_t><<<(unsigned)((nh + 1 + 255) / 256), 256, 0, st>>>(sorted, nh, key_span, ctx->gs_flag.as<uint32_t>());
-    }
-    LS_CK(ls_scan_exclusive_u32(ctx->gs_flag.as<uint32_t>(), ctx->gs_flag.as<uint32_t>(), nh + 1, d_ntup, ctx->scan_tmp, st));
-    LS_CK(cudaMemcpyAsync(h, d_cnt, 32, cudaMemcpyDeviceToHost, st));
-    LS_CK(cudaStreamSynchronize(st));
-    nt = (int64_t)h[2];
-    S.n_events = (int64_t)h[0];  // real hits
-    LS_CK(ctx->gs_tup.ensure((size_t)nt * 5 * 4 + 16));
-    LS_CK(ctx->gs_p.ensure((size_t)nt * 8 + 16));
-    int32_t *t_site = ctx->gs_tup.as<int32_t>(), *t_cell = t_site + nt, *t_dp = t_cell + nt, *t_alt = t_dp + nt,
-            *t_k = t_alt + nt;
-    const uint8_t *d_skip = skip_p ? ctx->gs_skip.as<uint8_t>() : nullptr;
-    if (k32)
-      hit_reduce_kernel<uint32_t><<<(unsigned)((nh + 255) / 256), 256, 0, st>>>(sorted32, nh, (uint32_t)key_span, ctx->gs_flag.as<uint32_t>(), n_cells,
-                                                                                d_skip, t_site, t_cell, t_dp, t_alt, t_k);
+    if (key_span < (1ull << 32) && !getenv("LS_GENO_KEYS64"))
+      rc = hits_to_tuples<uint32_t>(ctx, a, nh, skip_p != nullptr, d, h, launches);
     else
-      hit_reduce_kernel<uint64_t><<<(unsigned)((nh + 255) / 256), 256, 0, st>>>(sorted, nh, key_span, ctx->gs_flag.as<uint32_t>(), n_cells,
-                                                                                d_skip, t_site, t_cell, t_dp, t_alt, t_k);
-    launches += 4;
-    LS_CK(cudaGetLastError());
-    LS_CK(cudaEventRecord(ctx->ev[1], st));
-    // K2 on the device: p = betabinom.sf(Alt - eps, Dp, alpha, beta) for the pairs with a query
-    rc = ls_betabinom_device(ctx, t_k, t_dp, alpha, beta, ctx->gs_p.as<double>(), nt, d_nbig);
+      rc = hits_to_tuples<uint64_t>(ctx, a, nh, skip_p != nullptr, d, h, launches);
+    if (rc != LS_OK) return rc;
+  }
+  const int64_t nt = (int64_t)h.n_tuples;
+  LS_CK(cudaEventRecord(ctx->ev[1], st));
+  if (nh > 0) {  // Phase 3, K2 on the device: p = betabinom.sf(Alt - eps, Dp, alpha, beta) for the pairs with a query
+    const int32_t *t_dp = gs.tup.as<int32_t>() + 2 * nt, *t_k = t_dp + 2 * nt;
+    rc = ls_betabinom_device(ctx, t_k, t_dp, alpha, beta, gs.p.as<double>(), nt, &d->n_big);
     if (rc != LS_OK) return rc;
     launches += nt > 4 * 65 * 65 ? 4 : 2;  // constants + tails (+ the (k, n) table and its queries)
-  } else {
-    LS_CK(cudaEventRecord(ctx->ev[1], st));
   }
   LS_CK(cudaEventRecord(ctx->ev[2], st));
   LS_CK(cudaStreamSynchronize(st));
   LS_CK(cudaEventElapsedTime(&S.ms_count, ctx->ev[0], ctx->ev[1]));
-  LS_CK(cudaEventElapsedTime(&S.ms_sort, ctx->ev[1], ctx->ev[2]));  // here: the beta-binomial kernel
+  LS_CK(cudaEventElapsedTime(&S.ms_sort, ctx->ev[1], ctx->ev[2]));
   LS_CK(cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[2]));
+  S.n_events = (int64_t)h.n_events;
   S.n_segments = nt;
   S.count_launches = launches;
-  ctx->n_tuples = nt;
-  ctx->have_tuples = true;
+  gs.n_tuples = nt;
+  gs.have_tuples = true;
   ctx->n_drop = 0;
   if (n_tuples) *n_tuples = nt;
   if (stats) *stats = S;
@@ -518,20 +518,21 @@ extern "C" int ls_genotype_sparse_run(ls_ctx *ctx, const int32_t *site_tid, cons
 extern "C" int ls_genotype_sparse_fetch(ls_ctx *ctx, ls_geno_tuples *out) {
   if (!ctx) return LS_E_ARG;
   if (!out) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_fetch: out is null");
-  if (!ctx->have_tuples) LS_FAIL(LS_E_STATE, "ls_genotype_sparse_fetch: ls_genotype_sparse_run has not completed");
-  const int64_t nt = ctx->n_tuples;
+  const GenoState &gs = ctx->geno;
+  if (!gs.have_tuples) LS_FAIL(LS_E_STATE, "ls_genotype_sparse_fetch: ls_genotype_sparse_run has not completed");
+  const int64_t nt = gs.n_tuples;
   out->n_tuples = nt;
   if (nt == 0) return LS_OK;
   if (out->capacity < nt) LS_FAIL(LS_E_CAPACITY, "ls_genotype_sparse_fetch: capacity < n_tuples");
   if (!out->site || !out->cell || !out->dp || !out->alt || !out->p) LS_FAIL(LS_E_ARG, "ls_genotype_sparse_fetch: null array");
   LS_CK(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  const int32_t *t = ctx->gs_tup.as<int32_t>();
+  const int32_t *t = gs.tup.as<int32_t>();
   LS_CK(cudaMemcpyAsync(out->site, t, (size_t)nt * 4, cudaMemcpyDeviceToHost, st));
   LS_CK(cudaMemcpyAsync(out->cell, t + nt, (size_t)nt * 4, cudaMemcpyDeviceToHost, st));
   LS_CK(cudaMemcpyAsync(out->dp, t + 2 * nt, (size_t)nt * 4, cudaMemcpyDeviceToHost, st));
   LS_CK(cudaMemcpyAsync(out->alt, t + 3 * nt, (size_t)nt * 4, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaMemcpyAsync(out->p, ctx->gs_p.p, (size_t)nt * 8, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaMemcpyAsync(out->p, gs.p.p, (size_t)nt * 8, cudaMemcpyDeviceToHost, st));
   LS_CK(cudaStreamSynchronize(st));
   // pairs whose Alt count is past the in-register kernel's range (marked p = -1): the staged path
   std::vector<int64_t> big;
@@ -544,7 +545,7 @@ extern "C" int ls_genotype_sparse_fetch(ls_ctx *ctx, ls_geno_tuples *out) {
       k[j] = out->alt[big[j]];
       nn[j] = out->dp[big[j]];
     }
-    int rc = ls_betabinom_sf(ctx, k.data(), nn.data(), ctx->gs_alpha, ctx->gs_beta, pp.data(), (int64_t)big.size(), nullptr);
+    int rc = ls_betabinom_sf(ctx, k.data(), nn.data(), gs.alpha, gs.beta, pp.data(), (int64_t)big.size(), nullptr);
     if (rc != LS_OK) return rc;
     for (size_t j = 0; j < big.size(); ++j) out->p[big[j]] = pp[j];
   }
@@ -555,9 +556,8 @@ extern "C" int ls_genotype_count(ls_ctx *ctx, const int32_t *site_tid, const int
                                  const uint8_t *alt_class, int64_t n_sites, int32_t n_cells,
                                  const ls_geno_params *params, int32_t *dp, int32_t *alt, ls_run_stats *stats) {
   if (!ctx) return LS_E_ARG;
-  if (!params) LS_FAIL(LS_E_ARG, "ls_genotype_count: params is null");
-  if (!ctx->have_batch) LS_FAIL(LS_E_STATE, "ls_genotype_count: no batch uploaded");
-  if (n_sites < 0 || n_cells < 0) LS_FAIL(LS_E_ARG, "ls_genotype_count: negative size");
+  int rc = geno_check(ctx, "ls_genotype_count", params, n_sites, n_cells);
+  if (rc != LS_OK) return rc;
   ls_run_stats S;
   memset(&S, 0, sizeof S);
   if (n_sites == 0 || n_cells == 0) {
@@ -565,44 +565,34 @@ extern "C" int ls_genotype_count(ls_ctx *ctx, const int32_t *site_tid, const int
     return LS_OK;
   }
   if (!site_tid || !site_pos || !alt_class || !dp || !alt) LS_FAIL(LS_E_ARG, "ls_genotype_count: null array");
-  const int32_t bin = params->bin_size > 0 ? params->bin_size : 50000;
   GenoSites g;
-  int rc = geno_prepare_sites(ctx, site_tid, site_pos, n_sites, bin, g);
+  rc = geno_setup(ctx, site_tid, site_pos, alt_class, n_sites, params, g);
   if (rc != LS_OK) return rc;
-  LS_CK(cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
   rc = geno_depth_cap(ctx, g.btid, g.bstart, g.bend, params->min_mq, params->max_depth);
   if (rc != LS_OK) return rc;
+  GenoState &gs = ctx->geno;
+  cudaStream_t st = ctx->stream;
   const size_t cells = (size_t)n_sites * (size_t)n_cells;
-  LS_CK(ctx->g_a.ensure((size_t)n_sites * 8));
-  LS_CK(ctx->g_b.ensure((size_t)n_sites));
-  LS_CK(ctx->g_c.ensure(cells * 4));
-  LS_CK(ctx->g_d.ensure(cells * 4));
-  LS_CK(ctx->g_e.ensure((size_t)n_sites * 4));
-  LS_CK(ctx->counters.ensure(64));
-  LS_CK(cudaMemcpyAsync(ctx->g_a.p, g.keys.data(), (size_t)n_sites * 8, cudaMemcpyHostToDevice, st));
-  LS_CK(cudaMemcpyAsync(ctx->g_b.p, alt_class, (size_t)n_sites, cudaMemcpyHostToDevice, st));
-  LS_CK(cudaMemcpyAsync(ctx->g_e.p, g.sbin.data(), (size_t)n_sites * 4, cudaMemcpyHostToDevice, st));
+  LS_CK(gs.dp.ensure(cells * 4));
+  LS_CK(gs.alt.ensure(cells * 4));
   LS_CK(cudaEventRecord(ctx->ev[0], st));
-  LS_CK(cudaMemsetAsync(ctx->g_c.p, 0, cells * 4, st));
-  LS_CK(cudaMemsetAsync(ctx->g_d.p, 0, cells * 4, st));
-  LS_CK(cudaMemsetAsync(ctx->counters.p, 0, 64, st));
-  GenoArgs a;
-  geno_fill_args(ctx, a, n_sites, n_cells, params);
-  a.dp = ctx->g_c.as<int32_t>();
-  a.alt = ctx->g_d.as<int32_t>();
+  LS_CK(cudaMemsetAsync(gs.dp.p, 0, cells * 4, st));
+  LS_CK(cudaMemsetAsync(gs.alt.p, 0, cells * 4, st));
+  GenoArgs a = geno_args(ctx, n_sites, n_cells, params);
+  a.dp = gs.dp.as<int32_t>();
+  a.alt = gs.alt.as<int32_t>();
   LS_CK(cudaEventRecord(ctx->ev[1], st));
-  if (ctx->n_reads > 0) genotype_kernel<0><<<(unsigned)((ctx->n_reads + 255) / 256), 256, 0, st>>>(a);
+  if (ctx->n_reads > 0) genotype_kernel<void><<<(unsigned)((ctx->n_reads + 255) / 256), 256, 0, st>>>(a);
   LS_CK(cudaGetLastError());
   LS_CK(cudaEventRecord(ctx->ev[2], st));
-  LS_CK(cudaMemcpyAsync(dp, ctx->g_c.p, cells * 4, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaMemcpyAsync(alt, ctx->g_d.p, cells * 4, cudaMemcpyDeviceToHost, st));
-  unsigned long long nev = 0;
-  LS_CK(cudaMemcpyAsync(&nev, ctx->counters.p, 8, cudaMemcpyDeviceToHost, st));
-  LS_CK(cudaStreamSynchronize(st));
+  LS_CK(cudaMemcpyAsync(dp, gs.dp.p, cells * 4, cudaMemcpyDeviceToHost, st));
+  LS_CK(cudaMemcpyAsync(alt, gs.alt.p, cells * 4, cudaMemcpyDeviceToHost, st));
+  GenoCounters h;
+  rc = read_counters(ctx, ctx->counters.as<GenoCounters>(), h);
+  if (rc != LS_OK) return rc;
   LS_CK(cudaEventElapsedTime(&S.ms_count, ctx->ev[1], ctx->ev[2]));
   LS_CK(cudaEventElapsedTime(&S.ms_total, ctx->ev[0], ctx->ev[2]));
-  S.n_events = (int64_t)nev;
+  S.n_events = (int64_t)h.n_events;
   S.count_launches = 1;
   ctx->n_drop = 0;
   if (stats) *stats = S;

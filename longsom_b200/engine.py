@@ -3,6 +3,7 @@
 Mirrors the reference's unit operations:
   Engine.pileup_count     <-> BaseCellCounter.run_interval          (BaseCellCounter.py:182-320)
   Engine.genotype_count   <-> SingleCellGenotype.run_interval loop  (SingleCellGenotype.py:114-178)
+  Engine.genotype_sparse  <-> the same loop + its betabinom.sf calls (SingleCellGenotype.py:114-218), touched pairs only
   Engine.betabinom_sf     <-> scipy.stats.betabinom.sf call sites   (BaseCellCalling.step1.py:196,201)
   Engine.site_mask        <-> step2.build_dict / GetExtraFilters    (BaseCellCalling.step2.py:124-221)
 Every method runs on the GPU; there is no CPU path behind any of them.
