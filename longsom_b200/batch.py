@@ -85,25 +85,24 @@ class ReadBatch:
                          self.seq4[b0 // 2:b1 // 2], self.qual[b0:b1])
 
     def select(self, idx):
-        """Sub-batch with the given (sorted) read indices; re-packs cigar / bases."""
+        """Sub-batch with the given (sorted) read indices; re-packs cigar / bases.  Every read keeps its base
+        padding, and each run of consecutive indices is copied as one slice."""
         idx = np.asarray(idx, dtype=np.int64)
         n = idx.shape[0]
-        nc = (self.cigar_off[idx + 1] - self.cigar_off[idx]).astype(np.int64)
+        co, bo = self.cigar_off.astype(np.int64), self.base_off.astype(np.int64)
         cigar_off = np.zeros(n + 1, np.uint32)
-        np.cumsum(nc, out=cigar_off[1:])
-        padded = ((self.l_qseq[idx].astype(np.int64) + 15) // 16) * 16
+        np.cumsum(co[idx + 1] - co[idx], out=cigar_off[1:])
         base_off = np.zeros(n + 1, np.uint64)
-        np.cumsum(padded, out=base_off[1:])
-        cigar = np.zeros(int(cigar_off[-1]), np.uint32)
-        seq4 = np.zeros(int(base_off[-1]) // 2, np.uint8)
-        qual = np.zeros(int(base_off[-1]), np.uint8)
-        for j, i in enumerate(idx):
-            cigar[cigar_off[j]:cigar_off[j + 1]] = self.cigar[self.cigar_off[i]:self.cigar_off[i + 1]]
-            bo, nb = int(self.base_off[i]), int(padded[j])
-            qual[int(base_off[j]):int(base_off[j]) + nb] = self.qual[bo:bo + nb]
-            seq4[int(base_off[j]) // 2:(int(base_off[j]) + nb) // 2] = self.seq4[bo // 2:(bo + nb) // 2]
+        np.cumsum(bo[idx + 1] - bo[idx], out=base_off[1:])
+        cut = np.nonzero(np.diff(idx) != 1)[0] + 1
+        lo = idx[np.concatenate([[0], cut])] if n else idx
+        hi = idx[np.concatenate([cut - 1, [n - 1]])] + 1 if n else idx
+
+        def gather(a, off, div=1):
+            parts = [a[off[s] // div:off[e] // div] for s, e in zip(lo.tolist(), hi.tolist())]
+            return np.concatenate(parts) if parts else a[:0].copy()
         return ReadBatch(self.tid[idx], self.pos[idx], self.flag[idx], self.mapq[idx], self.cell[idx], cigar_off,
-                         cigar, base_off, self.l_qseq[idx], seq4, qual)
+                         gather(self.cigar, co), base_off, self.l_qseq[idx], gather(self.seq4, bo, 2), gather(self.qual, bo))
 
 
 @dataclass

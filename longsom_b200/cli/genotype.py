@@ -6,7 +6,15 @@ GPU part: K1' (ls_genotype_sparse_run / _fetch) counts Dp / Alt of every touched
 pair of the run in one pass over the reads, and K2 evaluates on the device the beta-binomial
 tails of the pairs with ALT > 0; only the touched pairs come back, and the dense rows are
 expanded from them on the host.  The reference does this with one pysam pileup per 50 kb bin,
-a Python dict per (site, barcode) and one scipy call per pair (:114-218).  Host part kept byte-compatible: barcode cleaning, bin codes and temp-file order,
+a Python dict per (site, barcode) and one scipy call per pair (:114-218).
+
+The BAM streams by default (pipeline.stream_genotype): chunks of LONGSOM_CHUNK_MB of inflated BAM go
+through pinned staging buffers to one engine per LONGSOM_GPUS device, each chunk with the bins no
+later read can reach, so host memory stays bounded whatever the size of the tumour BAM.
+LONGSOM_STREAM=0 decodes the whole file and runs one call on the first device; both give the same
+pairs.  The rows are written into the long table bin by bin.
+
+Host part kept byte-compatible: barcode cleaning, bin codes and temp-file order,
 Python set iteration order of the sites inside a bin (:112,130), row formatting, and the pandas
 pivots with the natural-sorted index (:342-379)."""
 import argparse
@@ -23,7 +31,7 @@ import pandas as pd
 from .. import bamio
 from .._lib import CLASS_ID, LS_CLASS_NA
 from ..engine import Engine
-from ..pipeline import devices_from_env
+from ..pipeline import devices_from_env, stream_genotype
 
 _NUM = re.compile(r"(\d+)")
 
@@ -58,33 +66,10 @@ def build_dict_variants(variant_file, window):
     return d
 
 
-def genotype(args, hccv):
-    if args.tmp_dir != '.':
-        try:
-            os.mkdir(args.tmp_dir)
-            print("Directory ", args.tmp_dir, " created\n")
-        except FileExistsError:
-            print("Directory ", args.tmp_dir, " already exists\n")
-    else:
-        print("Not temp directory specified, using working directory as temp")
-    meta_dict = meta_to_dict(args.meta, args.tissue)
-    barcodes = list(meta_dict.keys())
-    bc_index = {b: i for i, b in enumerate(barcodes)}
-    bins = build_dict_variants(args.infile, args.bin)
-
-    # ---- candidate sites of every bin -------------------------------------------------------------
-    # the CUDA context comes up in the background while the BAM is decoded (the native decoder releases the GIL)
-    warm = {}
-
-    def _make_engine():
-        try:
-            warm["engine"] = Engine(devices_from_env()[0])
-        except Exception as e:
-            warm["error"] = e
-    warm_thread = threading.Thread(target=_make_engine, daemon=True)
-    warm_thread.start()
-    bam = bamio.read_bam(args.bam)
-    tid_of = {n: i for i, n in enumerate(bam.contig_names)}
+def candidate_sites(bins, contig_names):
+    """Site and bin setup: (bin_info, keys, site_tid, site_pos, alt_cls).  bin_info lists every bin of the variant file
+    as (chrom, Target_sites dict in file order); keys are the sorted (tid, pos0) of the sites on contigs of the BAM."""
+    tid_of = {n: i for i, n in enumerate(contig_names)}
     bin_info = []  # (chrom, Target_sites dict in file order)
     site_keys = {}
     for code, lines in bins.items():
@@ -101,28 +86,82 @@ def genotype(args, hccv):
     site_tid = np.array([k[0] for k in keys], np.int32)
     site_pos = np.array([k[1] for k in keys], np.int32)
     alt_cls = np.array([site_keys[k] for k in keys], np.uint8)
-    row_of = {k: i for i, k in enumerate(keys)}
+    return bin_info, keys, site_tid, site_pos, alt_cls
 
-    # ---- barcode -> column of the dense tensors ------------------------------------------------------
+
+def genotype(args, hccv):
+    if args.tmp_dir != '.':
+        try:
+            os.mkdir(args.tmp_dir)
+            print("Directory ", args.tmp_dir, " created\n")
+        except FileExistsError:
+            print("Directory ", args.tmp_dir, " already exists\n")
+    else:
+        print("Not temp directory specified, using working directory as temp")
+    meta_dict = meta_to_dict(args.meta, args.tissue)
+    barcodes = list(meta_dict.keys())
+    bc_index = {b: i for i, b in enumerate(barcodes)}
+    bins = build_dict_variants(args.infile, args.bin)
+    devices = devices_from_env()
+    stream = os.environ.get("LONGSOM_STREAM", "1") != "0"
+    if stream:
+        bs = bamio.BamStream(args.bam)  # the header only: the reads are decoded chunk by chunk below
+        contig_names = bs.contig_names
+        bs.close()
+    else:
+        # the CUDA context comes up in the background while the BAM is decoded (the native decoder releases the GIL)
+        warm = {}
+
+        def _make_engine():
+            try:
+                warm["engine"] = Engine(devices[0])
+            except Exception as e:
+                warm["error"] = e
+        warm_thread = threading.Thread(target=_make_engine, daemon=True)
+        warm_thread.start()
+        bam = bamio.read_bam(args.bam)
+        contig_names = bam.contig_names
+    bin_info, keys, site_tid, site_pos, alt_cls = candidate_sites(bins, contig_names)
+
+    # ---- touched (site, cell) pairs ------------------------------------------------------------------
+    # only the touched pairs come back, each with its beta-binomial tail already evaluated on the device (ALT > 0, not
+    # the chrM shortcut); the dense rows of the reference are expanded from them below
     if hccv:
         # HCCVSingleCellGenotype.py:163-169 looks the RAW tag up in the cleaned metadata keys
-        raw_to_cell = np.array([bc_index.get(b, -1) for b in bam.barcodes], np.int32)
+        cell_of = lambda b: bc_index.get(b, -1)
     else:
-        raw_to_cell = np.array([bc_index.get(b.split("-")[0], -1) for b in bam.barcodes], np.int32)
-    batch = bam.with_cells(raw_to_cell) if len(bam.barcodes) else bam.batch
+        cell_of = lambda b: bc_index.get(b.split("-")[0], -1)
     n_cells = len(barcodes)
-    warm_thread.join()
-    if "error" in warm:
-        raise warm["error"]
-    with warm["engine"] as eng:
-        eng.upload(batch, None)
-        # only the touched (site, cell) pairs come back, each with its beta-binomial tail already evaluated on the
-        # device (ALT > 0, not the chrM shortcut); the dense rows of the reference are expanded from them below
-        chrM_rows = np.array([bam.contig_names[t] == 'chrM' for t in site_tid], bool) if len(keys) else np.zeros(0, bool)
-        skip = chrM_rows.astype(np.uint8) if args.chrM_contaminant == 'True' else None
-        t_site, t_cell, t_dp, t_alt, t_p = eng.genotype_sparse(
-            site_tid, site_pos, alt_cls, n_cells, args.alpha2, args.beta2, skip_p=skip, min_bq=args.min_bq,
-            min_mq=args.min_mq, max_depth=200000, alt_only=(args.alt_flag != 'All'), bin_size=args.bin)
+    chrM_rows = np.array([contig_names[t] == 'chrM' for t in site_tid], bool) if len(keys) else np.zeros(0, bool)
+    skip = chrM_rows.astype(np.uint8) if args.chrM_contaminant == 'True' else None
+    params = dict(min_bq=args.min_bq, min_mq=args.min_mq, max_depth=200000, alt_only=(args.alt_flag != 'All'))
+    if stream:
+        # default: chunks of the BAM through pinned staging buffers, over every LONGSOM_GPUS device (bounded host
+        # memory); the workers' CUDA contexts come up while the first chunk is decoded.  LONGSOM_STREAM=0 decodes the
+        # whole file and runs one call on the first device
+        tuples = stream_genotype(args.bam, (site_tid, site_pos, alt_cls), args.bin, n_cells, cell_of, params, args.alpha2,
+                                 args.beta2, skip, devices, make_engine=Engine)
+    else:
+        raw_to_cell = np.array([cell_of(b) for b in bam.barcodes], np.int32)
+        batch = bam.with_cells(raw_to_cell) if len(bam.barcodes) else bam.batch
+        warm_thread.join()
+        if "error" in warm:
+            raise warm["error"]
+        with warm["engine"] as eng:
+            eng.upload(batch, None)
+            tuples = eng.genotype_sparse(site_tid, site_pos, alt_cls, n_cells, args.alpha2, args.beta2, skip_p=skip,
+                                         bin_size=args.bin, **params)
+        del bam, batch
+    return write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict)
+
+
+def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict):
+    """Row assembly: the dense rows of every bin, expanded from the touched pairs, written straight into the long table
+    bin after bin in the reference's (chrom name, lo) order, so that no more than one bin's text is held at a time."""
+    tid_of = {n: i for i, n in enumerate(contig_names)}
+    row_of = {k: i for i, k in enumerate(keys)}
+    n_cells = len(barcodes)
+    t_site, t_cell, t_dp, t_alt, t_p = tuples
     t_p = np.round(t_p, 4)
     bounds = np.searchsorted(t_site, np.arange(len(keys) + 1))
     native = os.environ.get("LONGSOM_GENO_NATIVE", "1") != "0"
@@ -146,11 +185,8 @@ def genotype(args, hccv):
         t_p = np.ascontiguousarray(t_p, np.float64)
         cell_text = (C.c_char_p * max(1, n_cells))(*[(bc + '\t' + meta_dict[bc]).encode() for bc in barcodes])
 
-    # ---- rows, in the reference's order ------------------------------------------------------------
-    blocks = {}
-    for chrom, target in bin_info:
+    def bin_rows(chrom, target):
         sites = set(target.keys())  # same construction as the reference => same iteration order
-        lo, hi = min(sites), max(sites)
         if native:
             # the dense rows are expanded from the touched pairs by the native writer (csrc/host/ls_genorows.cpp)
             order = list(sites)  # CELLS dict comprehension iterates the set (:130)
@@ -176,11 +212,10 @@ def genotype(args, hccv):
             if n < 0:
                 raise RuntimeError("ls_geno_rows failed (%d)" % n)
             try:
-                blocks[(str(chrom), lo)] = [C.string_at(text.value, n)] if n else []
+                return [C.string_at(text.value, n)] if n else []
             finally:
-                if n >= 0 and text.value:
+                if text.value:
                     host.ls_geno_rows_free(text)
-            continue
         rows = []
         for POS in sites:  # CELLS dict comprehension iterates the set (:130)
             Ref_exp, Alt_exp, Cell_type_exp, Num_cells_exp = target[POS]
@@ -211,8 +246,12 @@ def genotype(args, hccv):
                     BIN = 1 if MUTATED == "PASS" else (3 if MUTATED == "NoCoverage" else 0)
                     group += [str(BIN), str(chrom) + ':' + str(POS + 1) + ':' + Alt_exp.split(',')[0]]
                 rows.append(('\t'.join(group) + '\n').encode())
-        # temp file CHROM_min_max; a later bin with the same name overwrites an earlier one (:117-120)
-        blocks[(str(chrom), lo)] = rows
+        return rows
+
+    # temp file CHROM_min_max; a later bin with the same name overwrites an earlier one (:117-120)
+    blocks = {}
+    for chrom, target in bin_info:
+        blocks[(str(chrom), min(target))] = (chrom, target)
     header = ['#CHROM', 'Start', 'End', 'REF', 'ALT_expected', 'Cell_type_expected', 'Num_cells_expected', 'CB',
               'Cell_type_observed', 'Dp', 'ALT', 'VAF', 'BetaBin', 'MutationStatus']
     if not hccv:
@@ -221,9 +260,8 @@ def genotype(args, hccv):
     if blocks:
         with open(long_path, 'wb') as out:
             out.write(('\t'.join(header) + '\n').encode())
-            for chrom in sorted({k[0] for k in blocks}):
-                for start in sorted(k[1] for k in blocks if k[0] == chrom):
-                    out.writelines(blocks[(chrom, start)])
+            for key in sorted(blocks):
+                out.writelines(bin_rows(*blocks[key]))
     else:
         print('No temporary files found')
     return long_path

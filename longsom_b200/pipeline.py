@@ -1,5 +1,6 @@
 """Host-side orchestration shared by the drop-in CLIs: BAM -> ReadBatch, barcode -> cell ids,
-window pruning, per-GPU sharding (no collective) and the BaseCellCounter TSV writer.
+window pruning, per-GPU sharding (no collective), the BaseCellCounter TSV writer and the streamed BAM sources of
+the counter (stream_count) and of the genotype scripts (stream_genotype).
 
 Reference counterparts: BaseCellCounter.main / run_interval / concatenate_sort_temp_files_and_write
 (BaseCellCounter.py:22-79,182-320,344-409).  GPU selection cannot be a CLI flag (the Snakemake
@@ -253,7 +254,9 @@ def count_shards_pipelined(shards, params: CountParams, outs, device=0, lanes=2,
 # ---- streaming BaseCellCounter: BAM chunks -> pinned staging -> GPU -> per-contig row files ---------------------------
 class PinnedSlot:
     """One staging buffer set in pinned host memory (ls_host_alloc): the BAM decoder writes where the H2D copy reads.
-    Arrays grow on demand and are reused for every chunk that goes through the slot."""
+    Arrays grow on demand and are reused for every chunk that goes through the slot.  Where the host refuses pinned
+    memory (no CUDA device, or the locked-memory limit) an array is pageable, and the upload stages it through the
+    driver's own pinned buffers."""
     FIELDS = (("tid", np.int32, "n"), ("pos", np.int32, "n"), ("flag", np.uint16, "n"), ("mapq", np.uint8, "n"),
               ("cell", np.int32, "n"), ("l_qseq", np.int32, "n"), ("cigar_off", np.uint32, "n1"),
               ("base_off", np.uint64, "n1"), ("cigar", np.uint32, "c"), ("seq4", np.uint8, "b2"), ("qual", np.uint8, "b"))
@@ -267,14 +270,15 @@ class PinnedSlot:
         if self.caps.get(name, 0) >= count:
             return
         if name in self.ptrs:
-            self.lib.ls_host_free(self.ptrs[name])
+            self.lib.ls_host_free(self.ptrs.pop(name))
         want = int(count * 1.25) + 1024
         nbytes = want * np.dtype(dtype).itemsize
         p = C.c_void_p()
-        if self.lib.ls_host_alloc(C.c_size_t(nbytes), C.byref(p)) != 0:
-            raise MemoryError("ls_host_alloc(%d) failed" % nbytes)
-        self.ptrs[name] = p
         self.caps[name] = want
+        if self.lib.ls_host_alloc(C.c_size_t(nbytes), C.byref(p)) != 0:
+            self.arrays[name] = np.empty(want, dtype)
+            return
+        self.ptrs[name] = p
         self.arrays[name] = np.frombuffer((C.c_uint8 * nbytes).from_address(p.value), dtype=dtype, count=want)
 
     def __call__(self, n, nc, nb):
@@ -555,6 +559,186 @@ def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, 
             state["out"].close()
             if os.path.exists(out_file):
                 os.remove(out_file)
+
+
+# ---- streaming genotype scripts: BAM chunks -> pinned staging -> K1' + K2 per chunk -> touched pairs ------------------
+def genotype_bins(site_tid, site_pos, bin_size):
+    """The pileup() calls of a genotype run as ls_genotype derives them from the sorted site table: one per run of sites
+    with the same contig and floor(POS / bin_size) of the 1-based POS, over [first pos - 1, last pos + 1) (0-based).
+    Returns (first, start, end): first[b] is the first site row of bin b and first[-1] the number of sites; start / end
+    are the keys tid << 32 | position of the bin's region."""
+    tid = np.asarray(site_tid, np.int64)
+    pos = np.asarray(site_pos, np.int64)
+    code = (pos + 1) // (bin_size if bin_size > 0 else 50000)
+    new = np.ones(pos.shape[0], bool)
+    new[1:] = (tid[1:] != tid[:-1]) | (code[1:] != code[:-1])
+    first = np.append(np.nonzero(new)[0], pos.shape[0])
+    lo, hi = first[:-1], first[1:] - 1
+    return first, (tid[lo] << 32) | np.maximum(pos[lo] - 1, 0), (tid[hi] << 32) | (pos[hi] + 1)
+
+
+def read_keys(batch: ReadBatch, ends):
+    """(start, end) keys tid << 32 | position of every read; the end is at least pos + 1, as the fetch of a pileup() call
+    sees it (bam_endpos)."""
+    tid = batch.tid.astype(np.int64) << 32
+    pos = batch.pos.astype(np.int64)
+    return tid | pos, tid | np.maximum(ends, pos + 1)
+
+
+def plan_genotype_chunk(read_start, read_end, bin_start, bin_end, first_bin, last):
+    """One chunk of a streamed genotype run.  read_start / read_end: read_keys() of the chunk's reads in coordinate
+    order (the carried reads first); bin_start / bin_end: region keys of genotype_bins(); first_bin: the first bin no
+    earlier chunk completed; last: start key of the chunk's last read, or None when no mapped read follows.
+    A bin is complete once last >= its end: every later read starts at or after `last`, so none can overlap it.
+    Returns (done, send, carry): bins [first_bin, done) are complete; `send` indexes the reads that overlap one of
+    them, which are all the records their pileup() calls fetch; `carry` indexes the reads whose end passes the start of
+    bin `done`, the first incomplete one, and which go in front of the next chunk."""
+    nb = bin_end.shape[0]
+    done = nb if last is None else max(first_bin, int(np.searchsorted(bin_end, last, side="right")))
+    # the first bin from first_bin on that ends after the read starts; bins are sorted, so it is the only one to test
+    j = np.maximum(np.searchsorted(bin_end, read_start, side="right"), first_bin)
+    send = np.nonzero((j < done) & (bin_start[np.minimum(j, max(nb - 1, 0))] < read_end))[0] if done > first_bin \
+        else np.zeros(0, np.int64)
+    carry = np.nonzero(read_end > bin_start[done])[0] if done < nb else np.zeros(0, np.int64)
+    return done, send, carry
+
+
+def stream_genotype(bam_path, sites, bins, n_cells, cell_map, geno_params, alpha, beta, skip_p, devices, chunk_bytes=None,
+                    stats_out=None, make_engine=None):
+    """Touched (site, cell) pairs of SingleCellGenotype / HCCVSingleCellGenotype over a BAM of any size with bounded host
+    memory: the same (site, cell, dp, alt, p) arrays, ordered by site, that one Engine.genotype_sparse call over the
+    whole file returns.
+      sites       : (site_tid, site_pos, alt_class), sorted and unique, tids of the BAM header;
+      bins        : the bin size of the scripts' --bin; the pileup() calls are genotype_bins();
+      cell_map    : barcode text of a CB tag -> column in [0, n_cells), or -1;
+      geno_params : the other keyword arguments of genotype_sparse (min_bq, min_mq, max_depth, alt_only);
+      skip_p      : per site, 1 where no tail is evaluated (None: none);
+      chunk_bytes : inflated BAM per chunk (default LONGSOM_CHUNK_MB, 256 MB);
+      make_engine : device -> engine of a worker (default take_engine).
+    A decoder thread fills pinned slots with the next chunk behind the reads carried from the previous one and plans it
+    (plan_genotype_chunk).  One worker per entry of `devices`, each with its own engine, uploads the reads that overlap
+    the chunk's complete bins and runs genotype_sparse on the contiguous slice of the site table those bins hold.  A
+    chunk then holds every record the whole-file call fetches for those bins, in the same order, so the depth cap drops
+    the same records.  Sites no read reaches get no pairs.  stats_out, if given, receives one dict per device call."""
+    import queue
+    site_tid, site_pos, alt_cls = (np.ascontiguousarray(a, t) for a, t in zip(sites, (np.int32, np.int32, np.uint8)))
+    skip = None if skip_p is None else np.ascontiguousarray(skip_p, np.uint8)
+    first, bstart, bend = genotype_bins(site_tid, site_pos, bins)
+    empty = (np.zeros(0, np.int32),) * 4 + (np.zeros(0, np.float64),)
+    if bend.shape[0] == 0:
+        return empty
+    devices = devices or [0]
+    chunk_bytes = int(chunk_bytes or float(os.environ.get("LONGSOM_CHUNK_MB", "256")) * (1 << 20))
+    bs = bamio.BamStream(bam_path)
+    slots = [PinnedSlot() for _ in range(len(devices) + 1)]
+    free_slots = queue.Queue()
+    for sl in slots:
+        free_slots.put(sl)
+    todo, done_q = queue.Queue(maxsize=len(slots)), queue.Queue()
+    errors = []
+    columns = {"of_raw": np.zeros(0, np.int32)}
+
+    def to_columns(raw):
+        """raw barcode ids of the stream -> columns; the table grows as new CB texts appear."""
+        old = columns["of_raw"]
+        if len(bs.barcodes) > old.shape[0]:
+            columns["of_raw"] = np.concatenate([old, np.array([cell_map(b) for b in bs.barcodes[old.shape[0]:]], np.int32)])
+        out = np.full(raw.shape[0], -1, np.int32)
+        m = raw >= 0
+        out[m] = columns["of_raw"][raw[m]]
+        return out
+
+    def decoder():
+        seq = 0
+        try:
+            bi, carry, carry_ends = 0, None, None
+            while bi < bend.shape[0] and not errors:
+                slot = free_slots.get()
+                got = bs.next_chunk(chunk_bytes, slot, carry, carry_ends)
+                if got is None:
+                    free_slots.put(slot)
+                    if carry is None:
+                        break
+                    slot, batch, ends, n_carried, last = None, carry, carry_ends, carry.n_reads, None
+                else:
+                    batch, n_new, ends = got
+                    n_carried = batch.n_reads - n_new
+                    # unplaced reads (tid -1) close a coordinate-sorted BAM: no mapped read follows them
+                    last = None if batch.tid[-1] < 0 else (int(batch.tid[-1]) << 32) | int(batch.pos[-1])
+                rs, re_ = read_keys(batch, ends)
+                bj, send, keep = plan_genotype_chunk(rs, re_, bstart, bend, bi, last)
+                carry, carry_ends = (batch.select(keep), ends[keep]) if keep.shape[0] else (None, None)
+                if send.shape[0]:
+                    sub = batch.slice(send[0], send[-1] + 1) if send[-1] - send[0] + 1 == send.shape[0] else batch.select(send)
+                    sub.cell = to_columns(sub.cell)
+                    todo.put((seq, sub, int(first[bi]), int(first[bj]), slot, n_carried))
+                    seq += 1
+                elif slot is not None:
+                    free_slots.put(slot)
+                bi = bj
+                if last is None:
+                    break
+        except Exception as ex:  # surfaced by the caller
+            errors.append(ex)
+        finally:
+            for _ in devices:
+                todo.put(None)
+
+    def device_worker(dev):
+        eng = None
+        try:
+            eng = (make_engine or take_engine)(dev)
+        except Exception as ex:
+            errors.append(ex)
+        try:
+            while True:
+                item = todo.get()
+                if item is None:
+                    break
+                seq, batch, lo, hi, slot, n_carried = item
+                try:
+                    if not errors:  # after an error the queue is only drained, so that the decoder never blocks
+                        eng.upload(batch, None)
+                        site, cell, dp, alt, p = eng.genotype_sparse(
+                            site_tid[lo:hi], site_pos[lo:hi], alt_cls[lo:hi], n_cells, alpha, beta,
+                            skip_p=None if skip is None else skip[lo:hi], bin_size=bins, **geno_params)
+                        site += lo  # chunk-local site rows -> rows of the whole table
+                        if stats_out is not None:
+                            stats_out.append(dict(device=dev, n_reads=batch.n_reads, n_carried=n_carried, site_lo=lo,
+                                                  site_hi=hi, **eng.last_stats))
+                        done_q.put((seq, (site, cell, dp, alt, p)))
+                except Exception as ex:
+                    errors.append(ex)
+                finally:
+                    if slot is not None:
+                        free_slots.put(slot)
+        finally:
+            if eng is not None:
+                eng.close()
+            done_q.put(None)
+
+    threads = [threading.Thread(target=decoder, daemon=True)] + [
+        threading.Thread(target=device_worker, args=(d,), daemon=True) for d in devices]
+    for t in threads:
+        t.start()
+    parts, live = {}, len(devices)
+    while live:
+        item = done_q.get()
+        if item is None:
+            live -= 1
+        else:
+            parts[item[0]] = item[1]
+    for t in threads:
+        t.join()
+    for sl in slots:
+        sl.free()
+    bs.close()
+    if errors:
+        raise errors[0]
+    if not parts:
+        return empty
+    # chunks cover disjoint, increasing site slices: in chunk order the pairs are ordered by (site, cell)
+    return tuple(np.concatenate([parts[s][k] for s in sorted(parts)]) for k in range(5))
 
 
 def format_counter_lines(chrom, pos, ref, counts):
