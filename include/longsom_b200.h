@@ -229,6 +229,48 @@ int ls_site_table_load(ls_ctx *ctx, int table, const uint64_t *keys, int64_t n_k
 int ls_site_table_lookup(ls_ctx *ctx, int table, const uint64_t *query, int64_t m, uint8_t *hit,
                          ls_run_stats *stats);
 
+/* ---- genotype matrices ------------------------------------------------------------------------
+ * Replaces the pandas pivots of SingleCellGenotype.py:351-379 (pivot_long_dataframe + sort_chr_index): the
+ * DpMatrix / AltMatrix / VAFMatrix / BinaryMatrix rows, written as text straight from the touched pairs.
+ *   load : the pairs in matrix coordinates (row = output row rank, col = output column rank), sorted on the device
+ *          by (row, col) and kept resident until the next load.  A duplicate (row, col) is LS_E_ARG.
+ *   text : the rows row_lo .. row_lo + *rows_done - 1 of one matrix kind, as many whole rows as fit in capacity
+ *          bytes, each "label <tab> entry <tab> ... entry \n" (no header line).  A row longer than capacity is
+ *          LS_E_CAPACITY.
+ * Entries, as pandas prints them:
+ *   SNV row, touched pair     Dp, Alt as integers; VAF str(round(Alt / Dp, 4)) ('.' when Dp = 0); Binary the
+ *                             long table's BinMutationStatus: 3 when Dp = 0, 0 when Alt = 0, chrM shortcut rows
+ *                             1 when the rounded VAF >= 0.3, else 1 when p < pvalue, else 0
+ *   SNV row, untouched        0, 0, '.', 3; empty in a col_absent column
+ *   fusion row, a pair        1, 1, 1, 1
+ *   fusion row, no pair       empty
+ * With float_mode set (some entry of the matrix is absent) Dp, Alt and Binary print as floats ("2.0").          */
+#define LS_GENO_MATRIX_DP 0
+#define LS_GENO_MATRIX_ALT 1
+#define LS_GENO_MATRIX_VAF 2
+#define LS_GENO_MATRIX_BINARY 3
+#define LS_GENO_ROW_CHRM 1   /* the chrM shortcut applies to this row (--chrM_contaminant True) */
+#define LS_GENO_ROW_FUSION 2 /* a fusion row: every pair prints 1, every other entry is absent */
+typedef struct ls_geno_matrix_in {
+  int64_t n_rows;
+  int64_t n_pairs;
+  int32_t n_cols;
+  int32_t float_mode;
+  const int32_t *row;          /* [n_pairs] */
+  const int32_t *col;          /* [n_pairs] */
+  const int32_t *dp;           /* [n_pairs] */
+  const int32_t *alt;          /* [n_pairs] */
+  const double *p;             /* [n_pairs] beta-binomial tail rounded to four places (numpy.round), NaN if none */
+  const char *labels;          /* printed row labels back to back, in row order */
+  const int64_t *label_off;    /* [n_rows+1] */
+  const uint8_t *row_flags;    /* [n_rows] LS_GENO_ROW_* */
+  const uint8_t *col_absent;   /* [n_cols] 1: the column is absent from SNV rows (a fusion barcode); may be NULL */
+  double pvalue;               /* --pvalue */
+} ls_geno_matrix_in;
+int ls_geno_matrix_load(ls_ctx *ctx, const ls_geno_matrix_in *in);
+int ls_geno_matrix_text(ls_ctx *ctx, int kind, int64_t row_lo, char *out, int64_t capacity, int64_t *rows_done,
+                        int64_t *bytes);
+
 /* ---- device-resident handles for benchmarking (inputs already in HBM) ----------------------- */
 int ls_device_synchronize(ls_ctx *ctx);
 /* PCI address ("0000:1b:00.0") of a CUDA device ordinal, for NUMA placement of the host staging buffers; no context */

@@ -22,7 +22,10 @@ ABI_SYMBOLS = [
     "ls_pileup_upload", "ls_pileup_run", "ls_pileup_compact", "ls_pileup_fetch", "ls_pileup_count", "ls_genotype_count",
     "ls_genotype_sparse_run", "ls_genotype_sparse_fetch",
     "ls_betabinom_sf", "ls_site_mask", "ls_site_table_load", "ls_site_table_lookup", "ls_device_synchronize", "ls_device_pci_bus_id", "ls_flush_l2",
+    "ls_geno_matrix_load", "ls_geno_matrix_text",
 ]
+LS_GENO_MATRIX_DP, LS_GENO_MATRIX_ALT, LS_GENO_MATRIX_VAF, LS_GENO_MATRIX_BINARY = 0, 1, 2, 3
+LS_GENO_ROW_CHRM, LS_GENO_ROW_FUSION = 1, 2
 
 
 class LsReadBatch(C.Structure):
@@ -71,6 +74,13 @@ class LsSiteCounts(C.Structure):
                 ("ref", C.c_void_p), ("counts", C.c_void_p)]
 
 
+class LsGenoMatrixIn(C.Structure):
+    _fields_ = [("n_rows", C.c_int64), ("n_pairs", C.c_int64), ("n_cols", C.c_int32), ("float_mode", C.c_int32),
+                ("row", C.c_void_p), ("col", C.c_void_p), ("dp", C.c_void_p), ("alt", C.c_void_p), ("p", C.c_void_p),
+                ("labels", C.c_void_p), ("label_off", C.c_void_p), ("row_flags", C.c_void_p), ("col_absent", C.c_void_p),
+                ("pvalue", C.c_double)]
+
+
 class LongSomError(RuntimeError):
     pass
 
@@ -114,6 +124,8 @@ def load():
     lib.ls_site_table_lookup.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     lib.ls_site_mask.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
                                  P(LsRunStats)]
+    lib.ls_geno_matrix_load.argtypes = [C.c_void_p, P(LsGenoMatrixIn)]
+    lib.ls_geno_matrix_text.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_int64, P(C.c_int64), P(C.c_int64)]
     lib.ls_device_synchronize.argtypes = [C.c_void_p]
     lib.ls_flush_l2.argtypes = [C.c_void_p]
     for name in ABI_SYMBOLS:

@@ -15,21 +15,26 @@ LONGSOM_STREAM=0 decodes the whole file and runs one call on the first device; b
 pairs.  The rows are written into the long table bin by bin.
 
 Host part kept byte-compatible: barcode cleaning, bin codes and temp-file order,
-Python set iteration order of the sites inside a bin (:112,130), row formatting, and the pandas
-pivots with the natural-sorted index (:342-379)."""
+Python set iteration order of the sites inside a bin (:112,130) and row formatting.  The four matrices
+(:342-379) are formatted on the device from the same touched pairs (write_matrices); the reference's
+pandas pivots stay for the inputs the device writer refuses."""
 import argparse
+import ctypes as C
 import math
 import os
 import re
 import sys
 import threading
 import timeit
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import pandas as pd
+from pandas._libs.parsers import STR_NA_VALUES
 
 from .. import bamio
-from .._lib import CLASS_ID, LS_CLASS_NA
+from .._lib import (CLASS_ID, LS_CLASS_NA, LS_GENO_MATRIX_ALT, LS_GENO_MATRIX_BINARY, LS_GENO_MATRIX_DP,
+                    LS_GENO_MATRIX_VAF, LS_GENO_ROW_CHRM, LS_GENO_ROW_FUSION, LS_E_ARG, LongSomError)
 from ..engine import Engine
 from ..pipeline import devices_from_env, stream_genotype
 
@@ -155,6 +160,15 @@ def genotype(args, hccv):
     return write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict)
 
 
+class MatrixSource:
+    """What the matrix writer takes from the long table: its path, its bins (after the CHROM_min_max overwrite rule),
+    the touched pairs (p rounded as printed) and the barcodes of its CB column."""
+
+    def __init__(self, long_path, blocks, keys, contig_names, tuples, barcodes, meta_dict):
+        self.long_path, self.blocks, self.keys, self.contig_names = long_path, blocks, keys, contig_names
+        self.tuples, self.barcodes, self.meta_dict = tuples, barcodes, meta_dict
+
+
 def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict):
     """Row assembly: the dense rows of every bin, expanded from the touched pairs, written straight into the long table
     bin after bin in the reference's (chrom name, lo) order, so that no more than one bin's text is held at a time."""
@@ -163,6 +177,7 @@ def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes,
     n_cells = len(barcodes)
     t_site, t_cell, t_dp, t_alt, t_p = tuples
     t_p = np.round(t_p, 4)
+    tuples = (t_site, t_cell, t_dp, t_alt, t_p)
     bounds = np.searchsorted(t_site, np.arange(len(keys) + 1))
     native = os.environ.get("LONGSOM_GENO_NATIVE", "1") != "0"
     touched = [None] * len(keys)
@@ -264,7 +279,8 @@ def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes,
                 out.writelines(bin_rows(*blocks[key]))
     else:
         print('No temporary files found')
-    return long_path
+    return MatrixSource(long_path if blocks else None, [blocks[k] for k in sorted(blocks)], keys, contig_names, tuples,
+                        barcodes, meta_dict)
 
 
 def collect_cells_with_fusions(fusion_file):
@@ -278,11 +294,20 @@ def collect_cells_with_fusions(fusion_file):
     return pd.DataFrame(lines)
 
 
+def chr_index_order(labels):
+    """Row order of the matrices (:342-348): chrM sorts last (renamed to chrZ for a stable natural sort), fusions
+    ('zzz:') after everything.  Returns the renamed labels, the order of the rows and the labels printed in that order
+    (chrZ, literal or not, prints as chrM; the 'zzz:' prefix is dropped)."""
+    keyed = [i.replace('chrM', 'chrZ') for i in labels]
+    order = sorted(range(len(keyed)), key=lambda i: natural_key(keyed[i]))
+    return keyed, order, [keyed[i].replace('chrZ', 'chrM').replace('zzz:', '') for i in order]
+
+
 def sort_chr_index(df):
-    # chrM sorts last (renamed to chrZ for the natural sort), fusions ('zzz:') after everything (:342-348)
-    df.index = [i.replace('chrM', 'chrZ') for i in df.index]
-    df = df.reindex(sorted(df.index, key=natural_key))
-    df.index = [i.replace('chrZ', 'chrM').replace('zzz:', '') for i in df.index]
+    keyed, order, printed = chr_index_order(df.index)
+    df.index = keyed
+    df = df.reindex([keyed[i] for i in order])
+    df.index = printed
     return df
 
 
@@ -295,6 +320,178 @@ def pivot_long_dataframe(out_prefix, fusions):
         m = long_df.pivot(index='INDEX', columns='CB', values=values)
         m = sort_chr_index(m)
         m.to_csv(out_prefix + '.' + name + '.tsv', sep='\t', index=True)
+
+
+# ---- the four matrices, written on the device --------------------------------------------------------------------
+_CSV_SPECIAL = ('\t', '\n', '\r', '"')
+_BOOL_TOKENS = {'True', 'TRUE', 'true', 'False', 'FALSE', 'false'}
+MATRIX_KINDS = (('DpMatrix', LS_GENO_MATRIX_DP), ('AltMatrix', LS_GENO_MATRIX_ALT), ('VAFMatrix', LS_GENO_MATRIX_VAF),
+                ('BinaryMatrix', LS_GENO_MATRIX_BINARY))
+MATRIX_BLOCK_BYTES = 64 << 20
+
+
+def prints_as_itself(s):
+    """True when a value pandas reads from the long table comes back as the same string whatever the other values of
+    its column (read_csv infers types chunk by chunk, so one numeric, boolean or NA-like value can change its own type)
+    and to_csv prints it unquoted."""
+    if not isinstance(s, str) or s in STR_NA_VALUES or s in _BOOL_TOKENS or any(c in s for c in _CSV_SPECIAL):
+        return False
+    try:
+        float(s)
+    except ValueError:
+        return True
+    return False
+
+
+class MatrixLayout:
+    """Rows, columns and pairs of the four matrices in output coordinates, as pivot_long_dataframe lays them out."""
+
+    def __init__(self, labels, columns, col_absent, float_mode, row_flags, row, col, dp, alt, p):
+        self.labels, self.columns, self.col_absent, self.float_mode = labels, columns, col_absent, float_mode
+        self.row_flags, self.row, self.col, self.dp, self.alt, self.p = row_flags, row, col, dp, alt, p
+
+
+def matrix_layout(src, fusions, chrM_contaminant):
+    """The layout of the matrices pivot_long_dataframe writes from the long table of `src` and the fusion rows of
+    collect_cells_with_fusions, or None for an input whose matrices only pandas can say (the reason is printed)."""
+    def refuse(why):
+        print('Matrices written by pandas: ' + why)
+        return None
+    if src.long_path is None:
+        return refuse('no long table')
+    barcodes = src.barcodes
+    if not barcodes:
+        return refuse('no barcodes')
+    if not all(prints_as_itself(b) for b in barcodes):
+        return refuse('a barcode pandas would not read back as itself')
+    fusion_labels, fusion_bcs = [], []  # 'zzz:' + #FusionName, BC
+    if not fusions.empty:
+        fusion_labels, fusion_bcs = list(fusions[15]), list(fusions[7])
+        if not all(isinstance(x, str) and not any(c in x for c in _CSV_SPECIAL) for x in fusion_labels + fusion_bcs):
+            return refuse('a fusion name or barcode that is not plain text')
+    # the long table's other text fields: a quote or carriage return there changes how read_csv splits the table
+    if any(('"' in x or '\r' in x) for x in src.meta_dict.values()):
+        return refuse('a cell type with a quote or carriage return')
+    tid_of = {n: i for i, n in enumerate(src.contig_names)}
+    row_of = {k: i for i, k in enumerate(src.keys)}
+    site_label = np.full(len(src.keys), -1, np.int64)
+    labels, chrm = [], []
+    for chrom, target in src.blocks:
+        for POS, fields in target.items():
+            if any(('"' in x or '\r' in x) for x in [str(chrom)] + [str(v) for v in fields]):
+                return refuse('a site field with a quote or carriage return')
+            r = row_of.get((tid_of.get(chrom, -1), POS))
+            if r is not None:
+                site_label[r] = len(labels)
+            labels.append(str(chrom) + ':' + str(POS + 1) + ':' + fields[1].split(',')[0])
+            chrm.append(chrM_contaminant == 'True' and str(chrom) == 'chrM')
+    n_snv = len(labels)
+    names = sorted(set(fusion_labels))
+    labels += names
+    if len(set(labels)) < len(labels):
+        return refuse('two rows with the same label')
+    lex = sorted(range(len(labels)), key=lambda i: labels[i])  # pivot's index order, then the stable natural sort
+    keyed, order, printed = chr_index_order([labels[i] for i in lex])
+    if len(set(keyed)) < len(keyed):
+        return refuse('two rows with the same label once chrM is renamed')
+    rank = np.empty(len(labels), np.int32)
+    rank[np.asarray(lex, np.int64)[np.asarray(order, np.int64)]] = np.arange(len(labels), dtype=np.int32)
+    columns = sorted(set(barcodes) | set(fusion_bcs))
+    col_of = {b: i for i, b in enumerate(columns)}
+    meta_cols = set(barcodes)
+    col_absent = np.array([b not in meta_cols for b in columns], np.uint8)
+
+    t_site, t_cell, t_dp, t_alt, t_p = src.tuples
+    srow = site_label[np.asarray(t_site, np.int64)] if len(t_site) else np.zeros(0, np.int64)
+    keep = srow >= 0
+    cell_col = np.array([col_of[b] for b in barcodes], np.int32)
+    row = [rank[srow[keep]]]
+    col = [cell_col[np.asarray(t_cell, np.int64)[keep]]]
+    dp, alt = [np.asarray(t_dp, np.int32)[keep]], [np.asarray(t_alt, np.int32)[keep]]
+    p = [np.asarray(t_p, np.float64)[keep]]
+    # the VAF column is read as text only when it holds a '.' (an SNV entry with Dp = 0)
+    if int(np.count_nonzero(dp[0] > 0)) >= n_snv * len(barcodes):
+        return refuse('every SNV entry is covered, so pandas reads VAF as numbers')
+    name_row = {n: n_snv + i for i, n in enumerate(names)}
+    fpairs = sorted({(name_row[n], col_of[b]) for n, b in zip(fusion_labels, fusion_bcs)})
+    if fpairs:
+        fr, fc = np.array(fpairs, np.int64).T
+        row.append(rank[fr])
+        col.append(fc.astype(np.int32))
+        dp.append(np.ones(len(fpairs), np.int32))
+        alt.append(np.ones(len(fpairs), np.int32))
+        p.append(np.full(len(fpairs), np.nan))
+    float_mode = bool(col_absent.any()) or len(fpairs) < len(names) * len(columns)
+    row_flags = np.zeros(len(labels), np.uint8)
+    row_flags[rank[:n_snv]] = np.where(np.array(chrm, bool), LS_GENO_ROW_CHRM, 0)
+    row_flags[rank[n_snv:]] = LS_GENO_ROW_FUSION
+    return MatrixLayout(printed, columns, col_absent, float_mode, row_flags, np.concatenate(row), np.concatenate(col),
+                        np.concatenate(dp), np.concatenate(alt), np.concatenate(p))
+
+
+def write_matrices(args, src, fusions):
+    """DpMatrix, AltMatrix, VAFMatrix and BinaryMatrix as pivot_long_dataframe writes them, formatted on the first
+    LONGSOM_GPUS device from the touched pairs in blocks of whole rows, so host memory does not grow with
+    n_sites x n_cells.  Runs after the long table is written.  Returns False, writing nothing, for an input it refuses
+    (matrix_layout); pivot_long_dataframe then writes the matrices, or raises as the reference does."""
+    if not hasattr(Engine, 'geno_matrix_load'):
+        return False  # a stand-in genotyping engine (the CPU oracle's) has no matrix writer: pandas writes them
+    lay = matrix_layout(src, fusions, args.chrM_contaminant)
+    if lay is None:
+        return False
+    with Engine(devices_from_env()[0]) as eng:
+        try:
+            eng.geno_matrix_load(lay.row, lay.col, lay.dp, lay.alt, lay.p, [x.encode() for x in lay.labels],
+                                 lay.row_flags, len(lay.columns), lay.col_absent, lay.float_mode, args.pvalue)
+        except LongSomError as e:
+            if e.code != LS_E_ARG:  # a duplicate (row, col): pandas raises on it as the reference does
+                raise
+            print('Matrices written by pandas: ' + str(e))
+            return False
+        # whole rows per block: the longest possible row fits any block
+        longest = max(len(x.encode()) for x in lay.labels) + 1 + 13 * len(lay.columns) + 16
+        cap = max(MATRIX_BLOCK_BYTES, longest)
+        bufs = [_PinnedBlock(eng, cap) for _ in range(2)]
+        header = ('\t' + '\t'.join(lay.columns) + '\n').encode()
+        try:
+            with ThreadPoolExecutor(1) as pool:
+                for name, kind in MATRIX_KINDS:
+                    with open(args.outfile + '.' + name + '.tsv', 'wb') as f:
+                        f.write(header)
+                        row, i, pending = 0, 0, None
+                        while row < len(lay.labels):
+                            # block i is written here while the file thread still writes block i ^ 1
+                            rows, nb = eng.geno_matrix_text(kind, row, bufs[i].addr, cap)
+                            if pending is not None:
+                                pending.result()
+                            pending = pool.submit(f.write, bufs[i].view[:nb])
+                            row += rows
+                            i ^= 1
+                        if pending is not None:
+                            pending.result()
+        finally:
+            for b in bufs:
+                b.free()
+    return True
+
+
+class _PinnedBlock:
+    """A block buffer in pinned host memory (pageable where the host refuses to pin it)."""
+
+    def __init__(self, eng, nbytes):
+        self._lib, self._ptr = eng._lib, C.c_void_p()
+        if self._lib.ls_host_alloc(C.c_size_t(nbytes), C.byref(self._ptr)) != 0:
+            self._ptr, self._keep = None, C.create_string_buffer(nbytes)
+            self.addr = C.addressof(self._keep)
+        else:
+            self.addr = self._ptr.value
+        self.view = memoryview((C.c_char * nbytes).from_address(self.addr)).cast('B')
+
+    def free(self):
+        self.view.release()
+        if self._ptr is not None:
+            self._lib.ls_host_free(self._ptr)
+            self._ptr = None
 
 
 def initialize_parser(hccv):
@@ -328,10 +525,11 @@ def main(argv=None, hccv=False):
     args = initialize_parser(hccv).parse_args(argv)
     start = timeit.default_timer()
     print("Outfile: " if hccv else "Outfile prefix: ", args.outfile, "\n")
-    genotype(args, hccv)
+    src = genotype(args, hccv)
     if not hccv:
         fusions = collect_cells_with_fusions(args.fusions) if args.fusions else pd.DataFrame()
-        pivot_long_dataframe(args.outfile, fusions)
+        if not write_matrices(args, src, fusions):
+            pivot_long_dataframe(args.outfile, fusions)
     print("Computation time: " + str(round(timeit.default_timer() - start)) + ' seconds')
 
 

@@ -128,6 +128,20 @@ struct GenoState {
   double alpha = 0.0, beta = 0.0;
 };
 
+// The genotype matrix writer's pairs, kept between ls_geno_matrix_load and the ls_geno_matrix_text calls
+struct GenoMatrixState {
+  DBuf keys_a, keys_b, vals_a, vals_b;  // (row, col) keys and the radix sort's second buffers
+  DBuf in_dp, in_alt, in_p;             // pairs in the caller's order
+  DBuf col, dp, alt, p;                 // pairs sorted by (row, col)
+  DBuf row_start;                       // [n_rows+1] first pair of each row
+  DBuf labels, label_off, row_flags, col_absent;
+  DBuf lens, offs, out, result;         // per text call: row lengths, their scan, the block's text, rows / bytes
+  int64_t n_rows = 0, n_pairs = 0;
+  int32_t n_cols = 0, n_present = 0, float_mode = 0;
+  double pvalue = 0.0;
+  bool loaded = false;
+};
+
 // What a replay of ls_pileup_run takes from the last run on the batch that it can stand for
 struct ReplaySnapshot {
   bool valid = false;
@@ -183,6 +197,7 @@ struct ls_ctx {
   int64_t site_tab_n[LS_SITE_TABLES + 1] = {};
   bool site_tab_ok[LS_SITE_TABLES + 1] = {};
   GenoState geno;  // K1'
+  GenoMatrixState gm;  // genotype matrix writer
 };
 
 #define LS_CK(call)                                                                        \

@@ -6,6 +6,7 @@ Mirrors the reference's unit operations:
   Engine.genotype_sparse  <-> the same loop + its betabinom.sf calls (SingleCellGenotype.py:114-218), touched pairs only
   Engine.betabinom_sf     <-> scipy.stats.betabinom.sf call sites   (BaseCellCalling.step1.py:196,201)
   Engine.site_mask        <-> step2.build_dict / GetExtraFilters    (BaseCellCalling.step2.py:124-221)
+  Engine.geno_matrix_*    <-> the pandas pivots of SingleCellGenotype (SingleCellGenotype.py:351-379)
 Every method runs on the GPU; there is no CPU path behind any of them.
 """
 import ctypes as C
@@ -60,7 +61,9 @@ class Engine:
     def _check(self, rc, what):
         if rc != L.LS_OK:
             msg = self._lib.ls_last_error(self._ctx)
-            raise L.LongSomError("%s failed (%d): %s" % (what, rc, msg.decode() if msg else ""))
+            err = L.LongSomError("%s failed (%d): %s" % (what, rc, msg.decode() if msg else ""))
+            err.code = rc
+            raise err
 
     # ---- K1 ------------------------------------------------------------------------------
     def upload(self, batch: ReadBatch, windows: Windows = None):
@@ -147,6 +150,35 @@ class Engine:
         t = L.LsGenoTuples(m, 0, vp(site), vp(cell), vp(dp), vp(alt), vp(p))
         self._check(self._lib.ls_genotype_sparse_fetch(self._ctx, C.byref(t)), "ls_genotype_sparse_fetch")
         return site, cell, dp, alt, p
+
+    # ---- genotype matrices ---------------------------------------------------------------
+    def geno_matrix_load(self, row, col, dp, alt, p, labels, row_flags, n_cols, col_absent=None, float_mode=False,
+                         pvalue=0.01):
+        """Pairs of the Dp / Alt / VAF / Binary matrices in matrix coordinates (row rank, column rank), kept on the
+        device for geno_matrix_text.  labels: the printed row labels (bytes), in row order; row_flags: LS_GENO_ROW_*;
+        col_absent: 1 for the columns SNV rows do not have; p: the beta-binomial tail rounded to four places."""
+        row, col = np.ascontiguousarray(row, np.int32), np.ascontiguousarray(col, np.int32)
+        dp, alt = np.ascontiguousarray(dp, np.int32), np.ascontiguousarray(alt, np.int32)
+        p = np.ascontiguousarray(p, np.float64)
+        row_flags = np.ascontiguousarray(row_flags, np.uint8)
+        lens = np.fromiter((len(x) for x in labels), np.int64, len(labels))
+        label_off = np.zeros(len(labels) + 1, np.int64)
+        np.cumsum(lens, out=label_off[1:])
+        blob = b"".join(labels)
+        absent = None if col_absent is None else np.ascontiguousarray(col_absent, np.uint8)
+        vp = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None and a.size else None
+        s = L.LsGenoMatrixIn(len(labels), row.shape[0], int(n_cols), 1 if float_mode else 0, vp(row), vp(col), vp(dp),
+                             vp(alt), vp(p), C.cast(C.c_char_p(blob), C.c_void_p), vp(label_off), vp(row_flags),
+                             vp(absent), float(pvalue))
+        self._check(self._lib.ls_geno_matrix_load(self._ctx, C.byref(s)), "ls_geno_matrix_load")
+
+    def geno_matrix_text(self, kind, row_lo, out, capacity):
+        """Text of the whole rows row_lo.. of matrix `kind` (LS_GENO_MATRIX_*) that fit in `capacity` bytes at address
+        `out`: (rows written, bytes)."""
+        rows, nb = C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.ls_geno_matrix_text(self._ctx, int(kind), int(row_lo), out, int(capacity), C.byref(rows),
+                                                  C.byref(nb)), "ls_geno_matrix_text")
+        return int(rows.value), int(nb.value)
 
     # ---- K2 ------------------------------------------------------------------------------
     def betabinom_sf(self, k, n, a, b):
