@@ -271,6 +271,56 @@ int ls_geno_matrix_load(ls_ctx *ctx, const ls_geno_matrix_in *in);
 int ls_geno_matrix_text(ls_ctx *ctx, int kind, int64_t row_lo, char *out, int64_t capacity, int64_t *rows_done,
                         int64_t *bytes);
 
+/* ---- genotype long table ----------------------------------------------------------------------
+ * Replaces the row loops of SingleCellGenotype.py:128-214 / HCCVSingleCellGenotype.py:126-212 (the dense long table,
+ * one row per candidate site x metadata barcode), written as text straight from the touched pairs.  The text equals
+ * the host writer's (ls_geno_rows).
+ *   load : the output sites in the order their rows are written, each with its range of the touched pairs, and the
+ *          texts of the rows; kept resident until the next load.  LS_E_ARG for a pair's cell outside [0, n_cells),
+ *          cells not strictly increasing inside a site's range, a range outside [0, n_pairs] or with lo > hi, a pair
+ *          with alt outside [0, dp], a p neither NaN nor below 4e5 in magnitude, or a null array that is needed.
+ *          The alt and p rules go beyond the host writer, which prints such pairs; they keep every number within the
+ *          device's 32-bit digit formatting.  K1' counts alt only with dp and K2's tails lie in [0, 1], so the CLIs
+ *          never meet them.
+ *   text : the rows of the sites site_lo .. site_lo + *sites_done - 1, as many whole sites as fit in capacity bytes
+ *          (no header line).  A site longer than capacity is LS_E_CAPACITY; site_lo == n_sites gives (0, 0).
+ *   times: device time of the text calls since the load, from events: the write kernels and the device-to-host
+ *          copies, with the number of blocks and their bytes.
+ * For site s and cell c = 0 .. n_cells-1, one row:
+ *   prefix[s] \t cell_text[c] \t Dp \t Alt \t VAF \t BetaBin \t MutationStatus [\t BinMutationStatus \t index[s]] \n
+ * (the two bracketed columns only when hccv is 0), with the pair (Dp, Alt, p) of (s, c):
+ *   untouched, or Dp = 0         0 \t 0 \t . \t . \t NoCoverage, BinMutationStatus 3
+ *   Dp > 0, Alt = 0              VAF 0.0, BetaBin '.', NoAltReads, 0
+ *   Alt > 0, LS_GENO_ROW_CHRM    VAF str(round(Alt / Dp, 4)), BetaBin '.', LowVAFChrM when that VAF < 0.3 else PASS
+ *   Alt > 0, other sites         VAF as above, BetaBin str(p) ('nan' for NaN), PASS when p < pvalue else
+ *                                BetaBin_problem
+ *   BinMutationStatus            1 for PASS, 3 for NoCoverage, 0 otherwise                                          */
+typedef struct ls_geno_long_in {
+  int64_t n_sites;             /* output sites, in the order their rows are written */
+  int32_t n_cells;             /* may be 0: every site then has no rows */
+  int32_t hccv;                /* 1: 14 columns, no BinMutationStatus / INDEX */
+  int64_t n_pairs;
+  const int32_t *cell;         /* [n_pairs] touched pairs, sorted by cell inside each site's range */
+  const int32_t *dp;           /* [n_pairs] */
+  const int32_t *alt;          /* [n_pairs] */
+  const double *p;             /* [n_pairs] rounded to four places (numpy.round), NaN where none */
+  const int64_t *hit_lo;       /* [n_sites] the site's range of the pair arrays (lo == hi: untouched) */
+  const int64_t *hit_hi;       /* [n_sites] */
+  const uint8_t *site_flags;   /* [n_sites] LS_GENO_ROW_CHRM */
+  const char *prefix;          /* the seven leading columns of each site, tab-joined, back to back */
+  const int64_t *prefix_off;   /* [n_sites+1] */
+  const char *index;           /* INDEX column of each site; NULL when hccv */
+  const int64_t *index_off;    /* [n_sites+1]; NULL when hccv */
+  const char *cell_text;       /* "barcode\tcell type" of each cell */
+  const int64_t *cell_off;     /* [n_cells+1] */
+  double pvalue;               /* --pvalue */
+} ls_geno_long_in;
+int ls_geno_long_load(ls_ctx *ctx, const ls_geno_long_in *in);
+int ls_geno_long_text(ls_ctx *ctx, int64_t site_lo, char *out, int64_t capacity, int64_t *sites_done, int64_t *bytes);
+int ls_geno_long_times(ls_ctx *ctx, double *ms_text, double *ms_copy, int64_t *blocks, int64_t *bytes);
+/* frees the long table's device buffers (a later text call is LS_E_STATE until the next load) */
+int ls_geno_long_release(ls_ctx *ctx);
+
 /* ---- device-resident handles for benchmarking (inputs already in HBM) ----------------------- */
 int ls_device_synchronize(ls_ctx *ctx);
 /* PCI address ("0000:1b:00.0") of a CUDA device ordinal, for NUMA placement of the host staging buffers; no context */

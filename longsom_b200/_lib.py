@@ -22,7 +22,8 @@ ABI_SYMBOLS = [
     "ls_pileup_upload", "ls_pileup_run", "ls_pileup_compact", "ls_pileup_fetch", "ls_pileup_count", "ls_genotype_count",
     "ls_genotype_sparse_run", "ls_genotype_sparse_fetch",
     "ls_betabinom_sf", "ls_site_mask", "ls_site_table_load", "ls_site_table_lookup", "ls_device_synchronize", "ls_device_pci_bus_id", "ls_flush_l2",
-    "ls_geno_matrix_load", "ls_geno_matrix_text",
+    "ls_geno_matrix_load", "ls_geno_matrix_text", "ls_geno_long_load", "ls_geno_long_text", "ls_geno_long_times",
+    "ls_geno_long_release",
 ]
 LS_GENO_MATRIX_DP, LS_GENO_MATRIX_ALT, LS_GENO_MATRIX_VAF, LS_GENO_MATRIX_BINARY = 0, 1, 2, 3
 LS_GENO_ROW_CHRM, LS_GENO_ROW_FUSION = 1, 2
@@ -81,6 +82,14 @@ class LsGenoMatrixIn(C.Structure):
                 ("pvalue", C.c_double)]
 
 
+class LsGenoLongIn(C.Structure):
+    _fields_ = [("n_sites", C.c_int64), ("n_cells", C.c_int32), ("hccv", C.c_int32), ("n_pairs", C.c_int64),
+                ("cell", C.c_void_p), ("dp", C.c_void_p), ("alt", C.c_void_p), ("p", C.c_void_p), ("hit_lo", C.c_void_p),
+                ("hit_hi", C.c_void_p), ("site_flags", C.c_void_p), ("prefix", C.c_void_p), ("prefix_off", C.c_void_p),
+                ("index", C.c_void_p), ("index_off", C.c_void_p), ("cell_text", C.c_void_p), ("cell_off", C.c_void_p),
+                ("pvalue", C.c_double)]
+
+
 class LongSomError(RuntimeError):
     pass
 
@@ -126,6 +135,10 @@ def load():
                                  P(LsRunStats)]
     lib.ls_geno_matrix_load.argtypes = [C.c_void_p, P(LsGenoMatrixIn)]
     lib.ls_geno_matrix_text.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_int64, P(C.c_int64), P(C.c_int64)]
+    lib.ls_geno_long_load.argtypes = [C.c_void_p, P(LsGenoLongIn)]
+    lib.ls_geno_long_text.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, P(C.c_int64), P(C.c_int64)]
+    lib.ls_geno_long_times.argtypes = [C.c_void_p, P(C.c_double), P(C.c_double), P(C.c_int64), P(C.c_int64)]
+    lib.ls_geno_long_release.argtypes = [C.c_void_p]
     lib.ls_device_synchronize.argtypes = [C.c_void_p]
     lib.ls_flush_l2.argtypes = [C.c_void_p]
     for name in ABI_SYMBOLS:

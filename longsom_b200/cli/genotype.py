@@ -4,15 +4,18 @@ workflow/scripts/CellTypeReannotation/HCCVSingleCellGenotype.py).
 
 GPU part: K1' (ls_genotype_sparse_run / _fetch) counts Dp / Alt of every touched (site, cell)
 pair of the run in one pass over the reads, and K2 evaluates on the device the beta-binomial
-tails of the pairs with ALT > 0; only the touched pairs come back, and the dense rows are
-expanded from them on the host.  The reference does this with one pysam pileup per 50 kb bin,
-a Python dict per (site, barcode) and one scipy call per pair (:114-218).
+tails of the pairs with ALT > 0; only the touched pairs come back, and the dense rows of the
+long table are expanded from them on the device (ls_geno_long_*, write_long_table).  The reference
+does this with one pysam pileup per 50 kb bin, a Python dict per (site, barcode) and one scipy
+call per pair (:114-218).
 
 The BAM streams by default (pipeline.stream_genotype): chunks of LONGSOM_CHUNK_MB of inflated BAM go
 through pinned staging buffers to one engine per LONGSOM_GPUS device, each chunk with the bins no
 later read can reach, so host memory stays bounded whatever the size of the tumour BAM.
 LONGSOM_STREAM=0 decodes the whole file and runs one call on the first device; both give the same
-pairs.  The rows are written into the long table bin by bin.
+pairs.  The long table's rows are written in blocks of whole sites, two pinned blocks in flight, so its
+text is never held whole either; the host writer (ls_geno_rows) takes the place of the device
+writer when the genotyping engine is a stand-in without one.
 
 Host part kept byte-compatible: barcode cleaning, bin codes and temp-file order,
 Python set iteration order of the sites inside a bin (:112,130) and row formatting.  The four matrices
@@ -25,8 +28,10 @@ import os
 import re
 import sys
 import threading
+import time
 import timeit
 from concurrent.futures import ThreadPoolExecutor
+from contextlib import nullcontext
 
 import numpy as np
 import pandas as pd
@@ -95,6 +100,7 @@ def candidate_sites(bins, contig_names):
 
 
 def genotype(args, hccv):
+    """The long table of one run: (MatrixSource, the engine that wrote it or None); the caller closes the engine."""
     if args.tmp_dir != '.':
         try:
             os.mkdir(args.tmp_dir)
@@ -157,24 +163,69 @@ def genotype(args, hccv):
             tuples = eng.genotype_sparse(site_tid, site_pos, alt_cls, n_cells, args.alpha2, args.beta2, skip_p=skip,
                                          bin_size=args.bin, **params)
         del bam, batch
-    return write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict)
+    # the long table is formatted on the first device by the library's writer; a stand-in genotyping engine (the CPU
+    # oracle's) has none, and the host writer formats it
+    eng = Engine(devices[0]) if hasattr(Engine, 'geno_long_load') else None
+    try:
+        return write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict, eng), eng
+    except BaseException:
+        if eng is not None:
+            eng.close()
+        raise
 
 
 class MatrixSource:
     """What the matrix writer takes from the long table: its path, its bins (after the CHROM_min_max overwrite rule),
-    the touched pairs (p rounded as printed) and the barcodes of its CB column."""
+    the touched pairs (p rounded as printed) and the barcodes of its CB column.  long_stats: the device writer's times
+    (long_rows_device), None when the host wrote the table."""
 
-    def __init__(self, long_path, blocks, keys, contig_names, tuples, barcodes, meta_dict):
+    def __init__(self, long_path, blocks, keys, contig_names, tuples, barcodes, meta_dict, long_stats=None):
         self.long_path, self.blocks, self.keys, self.contig_names = long_path, blocks, keys, contig_names
-        self.tuples, self.barcodes, self.meta_dict = tuples, barcodes, meta_dict
+        self.tuples, self.barcodes, self.meta_dict, self.long_stats = tuples, barcodes, meta_dict, long_stats
 
 
-def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict):
+LONG_BLOCK_BYTES = 64 << 20
+LONG_TAIL_MAX = 57  # Dp .. MutationStatus of a row at most: two 10-digit counts, "0.xxxx", "-xxxxxx.xxxx", BetaBin_problem
+
+
+class LongLayout:
+    """The long table's sites in output order: per site its prefix (the seven leading columns), index (the INDEX
+    column), chrM flag (the chrM shortcut applies; LS_GENO_ROW_CHRM) and range hit_lo .. hit_hi of the touched pairs.
+    The sites of bin b are bin_start[b] .. bin_start[b + 1] - 1."""
+
+    def __init__(self, prefix, index, chrm, hit_lo, hit_hi, bin_start):
+        self.prefix, self.index, self.chrm, self.hit_lo, self.hit_hi = prefix, index, chrm, hit_lo, hit_hi
+        self.bin_start = bin_start
+
+
+def long_layout(args, blocks, tid_of, row_of, bounds):
+    """The LongLayout of the bins `blocks` (in their (chrom name, lo) order) over the touched pairs split by site at
+    `bounds`.  Inside a bin the sites come in the reference's Python set order (:112,130)."""
+    prefix, index, chrm, hlo, hhi, bin_start = [], [], [], [], [], []
+    for key in sorted(blocks):
+        chrom, target = blocks[key]
+        bin_start.append(len(prefix))
+        for POS in set(target.keys()):  # CELLS dict comprehension iterates the set (:130)
+            Ref_exp, Alt_exp, Cell_type_exp, Num_cells_exp = target[POS]
+            prefix.append('\t'.join([str(chrom), str(POS + 1), str(POS + 1), Ref_exp, Alt_exp, str(Cell_type_exp),
+                                     str(Num_cells_exp)]).encode())
+            index.append((str(chrom) + ':' + str(POS + 1) + ':' + Alt_exp.split(',')[0]).encode())
+            chrm.append(LS_GENO_ROW_CHRM if (args.chrM_contaminant == 'True' and str(chrom) == 'chrM') else 0)
+            r = row_of.get((tid_of.get(chrom, -1), POS))
+            hlo.append(bounds[r] if r is not None else 0)
+            hhi.append(bounds[r + 1] if r is not None else 0)
+    bin_start.append(len(prefix))
+    return LongLayout(prefix, index, np.array(chrm, np.uint8), np.array(hlo, np.int64), np.array(hhi, np.int64),
+                      bin_start)
+
+
+def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes, meta_dict, engine=None):
     """Row assembly: the dense rows of every bin, expanded from the touched pairs, written straight into the long table
-    bin after bin in the reference's (chrom name, lo) order, so that no more than one bin's text is held at a time."""
+    in the reference's (chrom name, lo) bin order.  With an engine the rows are formatted on its device in blocks of
+    whole sites (long_rows_device); without one the host writer formats them bin after bin (long_rows_host).  Either
+    way no more than two blocks or one bin of text are held at a time."""
     tid_of = {n: i for i, n in enumerate(contig_names)}
     row_of = {k: i for i, k in enumerate(keys)}
-    n_cells = len(barcodes)
     t_site, t_cell, t_dp, t_alt, t_p = tuples
     t_p = np.round(t_p, 4)
     tuples = (t_site, t_cell, t_dp, t_alt, t_p)
@@ -188,49 +239,9 @@ def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes,
             lo_, hi_ = int(bounds[r]), int(bounds[r + 1])
             if hi_ > lo_:
                 touched[r] = {tc[i]: (td[i], ta[i], tp[i]) for i in range(lo_, hi_)}
-    else:
-        import ctypes as C
-        host = bamio._load_host()
-        host.ls_geno_rows.restype = C.c_int64
-        host.ls_geno_rows.argtypes = [C.c_int32] + [C.c_void_p] * 9 + [C.c_int32, C.c_void_p, C.c_int32, C.c_double, C.c_void_p]
-        host.ls_geno_rows_free.argtypes = [C.c_void_p]
-        t_cell = np.ascontiguousarray(t_cell, np.int32)
-        t_dp = np.ascontiguousarray(t_dp, np.int32)
-        t_alt = np.ascontiguousarray(t_alt, np.int32)
-        t_p = np.ascontiguousarray(t_p, np.float64)
-        cell_text = (C.c_char_p * max(1, n_cells))(*[(bc + '\t' + meta_dict[bc]).encode() for bc in barcodes])
 
     def bin_rows(chrom, target):
         sites = set(target.keys())  # same construction as the reference => same iteration order
-        if native:
-            # the dense rows are expanded from the touched pairs by the native writer (csrc/host/ls_genorows.cpp)
-            order = list(sites)  # CELLS dict comprehension iterates the set (:130)
-            ns = len(order)
-            prefix, index = [], []
-            chrm = np.zeros(ns, np.uint8)
-            hlo, hhi = np.zeros(ns, np.int64), np.zeros(ns, np.int64)
-            for j, POS in enumerate(order):
-                Ref_exp, Alt_exp, Cell_type_exp, Num_cells_exp = target[POS]
-                prefix.append('\t'.join([str(chrom), str(POS + 1), str(POS + 1), Ref_exp, Alt_exp, str(Cell_type_exp),
-                                         str(Num_cells_exp)]).encode())
-                index.append((str(chrom) + ':' + str(POS + 1) + ':' + Alt_exp.split(',')[0]).encode())
-                chrm[j] = 1 if (args.chrM_contaminant == 'True' and str(chrom) == 'chrM') else 0
-                r = row_of.get((tid_of.get(chrom, -1), POS))
-                if r is not None:
-                    hlo[j], hhi[j] = bounds[r], bounds[r + 1]
-            pre_a = (C.c_char_p * max(1, ns))(*prefix)
-            idx_a = None if hccv else (C.c_char_p * max(1, ns))(*index)
-            text = C.c_void_p()
-            n = host.ls_geno_rows(ns, pre_a, idx_a, chrm.ctypes.data, hlo.ctypes.data, hhi.ctypes.data, t_cell.ctypes.data,
-                                  t_dp.ctypes.data, t_alt.ctypes.data, t_p.ctypes.data, n_cells, cell_text, 1 if hccv else 0,
-                                  float(args.pvalue), C.byref(text))
-            if n < 0:
-                raise RuntimeError("ls_geno_rows failed (%d)" % n)
-            try:
-                return [C.string_at(text.value, n)] if n else []
-            finally:
-                if text.value:
-                    host.ls_geno_rows_free(text)
         rows = []
         for POS in sites:  # CELLS dict comprehension iterates the set (:130)
             Ref_exp, Alt_exp, Cell_type_exp, Num_cells_exp = target[POS]
@@ -272,15 +283,80 @@ def write_long_table(args, hccv, bin_info, keys, contig_names, tuples, barcodes,
     if not hccv:
         header += ['BinMutationStatus', 'INDEX']
     long_path = args.outfile if hccv else args.outfile + '.SingleCellGenotype.tsv'
+    stats = None
     if blocks:
         with open(long_path, 'wb') as out:
             out.write(('\t'.join(header) + '\n').encode())
-            for key in sorted(blocks):
-                out.writelines(bin_rows(*blocks[key]))
+            if not native:
+                for key in sorted(blocks):
+                    out.writelines(bin_rows(*blocks[key]))
+            else:
+                lay = long_layout(args, blocks, tid_of, row_of, bounds)
+                cell_text = [(bc + '\t' + meta_dict[bc]).encode() for bc in barcodes]
+                if engine is not None:
+                    stats = long_rows_device(engine, out, lay, tuples, cell_text, hccv, args.pvalue)
+                else:
+                    long_rows_host(out, lay, tuples, cell_text, hccv, args.pvalue)
     else:
         print('No temporary files found')
     return MatrixSource(long_path if blocks else None, [blocks[k] for k in sorted(blocks)], keys, contig_names, tuples,
-                        barcodes, meta_dict)
+                        barcodes, meta_dict, stats)
+
+
+def long_rows_host(out, lay, tuples, cell_text, hccv, pvalue):
+    """The rows of `lay` to file `out` through the host writer (csrc/host/ls_genorows.cpp), one bin's text at a time."""
+    host = bamio._load_host()
+    host.ls_geno_rows.restype = C.c_int64
+    host.ls_geno_rows.argtypes = [C.c_int32] + [C.c_void_p] * 9 + [C.c_int32, C.c_void_p, C.c_int32, C.c_double, C.c_void_p]
+    host.ls_geno_rows_free.argtypes = [C.c_void_p]
+    _, t_cell, t_dp, t_alt, t_p = tuples
+    t_cell = np.ascontiguousarray(t_cell, np.int32)
+    t_dp = np.ascontiguousarray(t_dp, np.int32)
+    t_alt = np.ascontiguousarray(t_alt, np.int32)
+    t_p = np.ascontiguousarray(t_p, np.float64)
+    n_cells = len(cell_text)
+    cells = (C.c_char_p * max(1, n_cells))(*cell_text)
+    for s0, s1 in zip(lay.bin_start[:-1], lay.bin_start[1:]):
+        ns = s1 - s0
+        pre_a = (C.c_char_p * ns)(*lay.prefix[s0:s1])
+        idx_a = None if hccv else (C.c_char_p * ns)(*lay.index[s0:s1])
+        text = C.c_void_p()
+        n = host.ls_geno_rows(ns, pre_a, idx_a, lay.chrm[s0:].ctypes.data, lay.hit_lo[s0:].ctypes.data,
+                              lay.hit_hi[s0:].ctypes.data, t_cell.ctypes.data, t_dp.ctypes.data, t_alt.ctypes.data,
+                              t_p.ctypes.data, n_cells, cells, 1 if hccv else 0, float(pvalue), C.byref(text))
+        if n < 0:
+            raise RuntimeError("ls_geno_rows failed (%d)" % n)
+        try:
+            if n:
+                out.write(C.string_at(text.value, n))
+        finally:
+            if text.value:
+                host.ls_geno_rows_free(text)
+
+
+def long_rows_device(eng, out, lay, tuples, cell_text, hccv, pvalue):
+    """The rows of `lay` to file `out`, formatted on the engine's device (ls_genolong.cu) in blocks of whole sites
+    through two pinned buffers.  Returns the device times of the text calls (Engine.geno_long_times) and the seconds
+    the file writes took (write_s)."""
+    _, t_cell, t_dp, t_alt, t_p = tuples
+    eng.geno_long_load(t_cell, t_dp, t_alt, t_p, lay.hit_lo, lay.hit_hi, lay.chrm, lay.prefix,
+                       None if hccv else lay.index, cell_text, hccv, pvalue)
+    # whole sites per block: the longest possible site fits any block
+    n_cells = len(cell_text)
+    fixed = np.fromiter((len(x) for x in lay.prefix), np.int64, len(lay.prefix)) + 3 + 18
+    if not hccv:
+        fixed += 3 + np.fromiter((len(x) for x in lay.index), np.int64, len(lay.index))
+    longest = fixed * n_cells + sum(len(x) for x in cell_text) + (LONG_TAIL_MAX - 18) * (lay.hit_hi - lay.hit_lo)
+    cap = max(LONG_BLOCK_BYTES, int(longest.max()) if len(longest) else 0)
+    bufs = [_PinnedBlock(eng, cap) for _ in range(2)]
+    try:
+        write_s = write_blocks(out, eng.geno_long_text, len(lay.prefix), bufs, cap)
+        times = eng.geno_long_times()
+    finally:
+        for b in bufs:
+            b.free()
+        eng.geno_long_release()  # the matrix stage that follows on the same engine does not hold the table's buffers
+    return dict(times, write_s=write_s)
 
 
 def collect_cells_with_fusions(fusion_file):
@@ -429,7 +505,7 @@ def matrix_layout(src, fusions, chrM_contaminant):
                         np.concatenate(dp), np.concatenate(alt), np.concatenate(p))
 
 
-def write_matrices(args, src, fusions):
+def write_matrices(args, src, fusions, engine=None):
     """DpMatrix, AltMatrix, VAFMatrix and BinaryMatrix as pivot_long_dataframe writes them, formatted on the first
     LONGSOM_GPUS device from the touched pairs in blocks of whole rows, so host memory does not grow with
     n_sites x n_cells.  Runs after the long table is written.  Returns False, writing nothing, for an input it refuses
@@ -439,7 +515,8 @@ def write_matrices(args, src, fusions):
     lay = matrix_layout(src, fusions, args.chrM_contaminant)
     if lay is None:
         return False
-    with Engine(devices_from_env()[0]) as eng:
+    # the caller's engine when it passes one (main: the long table's), else one of our own
+    with nullcontext(engine) if engine is not None else Engine(devices_from_env()[0]) as eng:
         try:
             eng.geno_matrix_load(lay.row, lay.col, lay.dp, lay.alt, lay.p, [x.encode() for x in lay.labels],
                                  lay.row_flags, len(lay.columns), lay.col_absent, lay.float_mode, args.pvalue)
@@ -454,25 +531,37 @@ def write_matrices(args, src, fusions):
         bufs = [_PinnedBlock(eng, cap) for _ in range(2)]
         header = ('\t' + '\t'.join(lay.columns) + '\n').encode()
         try:
-            with ThreadPoolExecutor(1) as pool:
-                for name, kind in MATRIX_KINDS:
-                    with open(args.outfile + '.' + name + '.tsv', 'wb') as f:
-                        f.write(header)
-                        row, i, pending = 0, 0, None
-                        while row < len(lay.labels):
-                            # block i is written here while the file thread still writes block i ^ 1
-                            rows, nb = eng.geno_matrix_text(kind, row, bufs[i].addr, cap)
-                            if pending is not None:
-                                pending.result()
-                            pending = pool.submit(f.write, bufs[i].view[:nb])
-                            row += rows
-                            i ^= 1
-                        if pending is not None:
-                            pending.result()
+            for name, kind in MATRIX_KINDS:
+                with open(args.outfile + '.' + name + '.tsv', 'wb') as f:
+                    f.write(header)
+                    write_blocks(f, lambda row, addr, n, kind=kind: eng.geno_matrix_text(kind, row, addr, n),
+                                 len(lay.labels), bufs, cap)
         finally:
             for b in bufs:
                 b.free()
     return True
+
+
+def write_blocks(f, text, n, bufs, cap):
+    """Units (rows or sites) 0 .. n-1 to file f in blocks: text(lo, addr, cap) formats as many whole units from lo as
+    fit in cap bytes at addr and returns (units, bytes).  Block i is formatted into bufs[i] while the file thread still
+    writes block i ^ 1.  Returns the seconds the file writes took."""
+    def put(view):
+        t = time.perf_counter()
+        f.write(view)
+        return time.perf_counter() - t
+    spent, lo, i, pending = 0.0, 0, 0, None
+    with ThreadPoolExecutor(1) as pool:
+        while lo < n:
+            units, nb = text(lo, bufs[i].addr, cap)
+            if pending is not None:
+                spent += pending.result()
+            pending = pool.submit(put, bufs[i].view[:nb])
+            lo += units
+            i ^= 1
+        if pending is not None:
+            spent += pending.result()
+    return spent
 
 
 class _PinnedBlock:
@@ -525,11 +614,15 @@ def main(argv=None, hccv=False):
     args = initialize_parser(hccv).parse_args(argv)
     start = timeit.default_timer()
     print("Outfile: " if hccv else "Outfile prefix: ", args.outfile, "\n")
-    src = genotype(args, hccv)
-    if not hccv:
-        fusions = collect_cells_with_fusions(args.fusions) if args.fusions else pd.DataFrame()
-        if not write_matrices(args, src, fusions):
-            pivot_long_dataframe(args.outfile, fusions)
+    src, eng = genotype(args, hccv)
+    try:
+        if not hccv:
+            fusions = collect_cells_with_fusions(args.fusions) if args.fusions else pd.DataFrame()
+            if not write_matrices(args, src, fusions, engine=eng):
+                pivot_long_dataframe(args.outfile, fusions)
+    finally:
+        if eng is not None:
+            eng.close()
     print("Computation time: " + str(round(timeit.default_timer() - start)) + ' seconds')
 
 

@@ -142,6 +142,30 @@ struct GenoMatrixState {
   bool loaded = false;
 };
 
+// The genotype long table's layout, kept between ls_geno_long_load and the ls_geno_long_text calls
+struct GenoLongState {
+  DBuf cell, dp, alt, p;                         // [n_pairs] the touched pairs as given
+  DBuf hit_lo, hit_hi, flags;                    // [n_sites] each output site's range of the pairs, LS_GENO_ROW_*
+  DBuf tail_base, tail_cum;                      // per site, from tail_base[s]: its pairs' tail lengths, scanned
+  DBuf site_len, site_off;                       // [n_sites] text bytes of a site; [n_sites+1] their scan
+  DBuf prefix, prefix_off, index, index_off, cell_text, cell_off;  // offsets rebased to 0
+  DBuf out, result;                              // per text call: the block's text; load: the input error flags
+  std::vector<int64_t> h_site_off;               // [n_sites+1] host copy of site_off: plans the blocks
+  int64_t n_sites = 0, n_pairs = 0;
+  int32_t n_cells = 0, hccv = 0;
+  double pvalue = 0.0;
+  double ms_text = 0.0, ms_copy = 0.0;           // device time of the text calls since the load (events)
+  int64_t blocks = 0, bytes = 0;                 // blocks and bytes written since the load
+  bool loaded = false;
+  void release() {
+    for (DBuf *b : {&cell, &dp, &alt, &p, &hit_lo, &hit_hi, &flags, &tail_base, &tail_cum, &site_len, &site_off, &prefix,
+                    &prefix_off, &index, &index_off, &cell_text, &cell_off, &out, &result})
+      b->release();
+    std::vector<int64_t>().swap(h_site_off);
+    loaded = false;
+  }
+};
+
 // What a replay of ls_pileup_run takes from the last run on the batch that it can stand for
 struct ReplaySnapshot {
   bool valid = false;
@@ -198,6 +222,7 @@ struct ls_ctx {
   bool site_tab_ok[LS_SITE_TABLES + 1] = {};
   GenoState geno;  // K1'
   GenoMatrixState gm;  // genotype matrix writer
+  GenoLongState gl;    // genotype long-table writer
 };
 
 #define LS_CK(call)                                                                        \

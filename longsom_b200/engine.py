@@ -7,6 +7,7 @@ Mirrors the reference's unit operations:
   Engine.betabinom_sf     <-> scipy.stats.betabinom.sf call sites   (BaseCellCalling.step1.py:196,201)
   Engine.site_mask        <-> step2.build_dict / GetExtraFilters    (BaseCellCalling.step2.py:124-221)
   Engine.geno_matrix_*    <-> the pandas pivots of SingleCellGenotype (SingleCellGenotype.py:351-379)
+  Engine.geno_long_*      <-> the long-table row loops of both genotype scripts (SingleCellGenotype.py:128-214)
 Every method runs on the GPU; there is no CPU path behind any of them.
 """
 import ctypes as C
@@ -179,6 +180,52 @@ class Engine:
         self._check(self._lib.ls_geno_matrix_text(self._ctx, int(kind), int(row_lo), out, int(capacity), C.byref(rows),
                                                   C.byref(nb)), "ls_geno_matrix_text")
         return int(rows.value), int(nb.value)
+
+    # ---- genotype long table -------------------------------------------------------------
+    def geno_long_load(self, cell, dp, alt, p, hit_lo, hit_hi, site_flags, prefix, index, cell_text, hccv=False,
+                       pvalue=0.01):
+        """The long table's layout, kept on the device for geno_long_text: the touched pairs (cell, dp, alt, p rounded
+        to four places; sorted by cell inside each site's range), and per output site, in row order, its pair range
+        hit_lo .. hit_hi, LS_GENO_ROW_CHRM flag, prefix (the seven leading columns, bytes) and index (the INDEX column,
+        bytes; None when hccv).  cell_text: b"barcode\\tcell type" of each cell."""
+        cell, dp, alt = (np.ascontiguousarray(x, np.int32) for x in (cell, dp, alt))
+        p = np.ascontiguousarray(p, np.float64)
+        hit_lo, hit_hi = np.ascontiguousarray(hit_lo, np.int64), np.ascontiguousarray(hit_hi, np.int64)
+        site_flags = np.ascontiguousarray(site_flags, np.uint8)
+
+        def packed(texts):
+            off = np.zeros(len(texts) + 1, np.int64)
+            np.cumsum(np.fromiter((len(x) for x in texts), np.int64, len(texts)), out=off[1:])
+            return b"".join(texts), off
+        pre, pre_off = packed(prefix)
+        idx, idx_off = packed(index) if not hccv else (b"", None)
+        ct, ct_off = packed(cell_text)
+        vp = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None and a.size else None
+        bp = lambda b: C.cast(C.c_char_p(b), C.c_void_p)
+        s = L.LsGenoLongIn(len(hit_lo), len(cell_text), 1 if hccv else 0, cell.shape[0], vp(cell), vp(dp), vp(alt), vp(p),
+                           vp(hit_lo), vp(hit_hi), vp(site_flags), bp(pre), vp(pre_off), bp(idx) if not hccv else None,
+                           vp(idx_off), bp(ct), vp(ct_off), float(pvalue))
+        self._check(self._lib.ls_geno_long_load(self._ctx, C.byref(s)), "ls_geno_long_load")
+
+    def geno_long_text(self, site_lo, out, capacity):
+        """Text of the whole sites site_lo.. of the loaded long table that fit in `capacity` bytes at address `out`:
+        (sites written, bytes)."""
+        sites, nb = C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.ls_geno_long_text(self._ctx, int(site_lo), out, int(capacity), C.byref(sites),
+                                                C.byref(nb)), "ls_geno_long_text")
+        return int(sites.value), int(nb.value)
+
+    def geno_long_times(self):
+        """Device time of the geno_long_text calls since the last load, from events: {ms_text, ms_copy, blocks,
+        bytes}."""
+        t, c, n, b = C.c_double(0), C.c_double(0), C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.ls_geno_long_times(self._ctx, C.byref(t), C.byref(c), C.byref(n), C.byref(b)),
+                    "ls_geno_long_times")
+        return dict(ms_text=t.value, ms_copy=c.value, blocks=n.value, bytes=b.value)
+
+    def geno_long_release(self):
+        """Frees the device buffers of the loaded long table."""
+        self._check(self._lib.ls_geno_long_release(self._ctx), "ls_geno_long_release")
 
     # ---- K2 ------------------------------------------------------------------------------
     def betabinom_sf(self, k, n, a, b):
