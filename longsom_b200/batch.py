@@ -75,14 +75,17 @@ class ReadBatch:
                    ("tid", "pos", "flag", "mapq", "cell", "cigar_off", "cigar", "base_off", "l_qseq", "seq4", "qual"))
 
     def slice(self, lo, hi):
-        """Sub-batch of the consecutive reads [lo, hi): array slices with rebased offsets (no per-read work)."""
+        """Sub-batch of the consecutive reads [lo, hi): array slices with rebased offsets (no per-read work).  Offsets
+        that start at 0 stay views, so that a slice of pinned staging memory is uploaded from pinned memory."""
         lo, hi = int(lo), int(hi)
         c0, c1 = int(self.cigar_off[lo]), int(self.cigar_off[hi])
         b0, b1 = int(self.base_off[lo]), int(self.base_off[hi])
+        cigar_off, base_off = self.cigar_off[lo:hi + 1], self.base_off[lo:hi + 1]
+        if c0 or b0:
+            cigar_off, base_off = (cigar_off - np.uint32(c0)).astype(np.uint32), (base_off - np.uint64(b0)).astype(np.uint64)
         return ReadBatch(self.tid[lo:hi], self.pos[lo:hi], self.flag[lo:hi], self.mapq[lo:hi], self.cell[lo:hi],
-                         (self.cigar_off[lo:hi + 1] - np.uint32(c0)).astype(np.uint32), self.cigar[c0:c1],
-                         (self.base_off[lo:hi + 1] - np.uint64(b0)).astype(np.uint64), self.l_qseq[lo:hi],
-                         self.seq4[b0 // 2:b1 // 2], self.qual[b0:b1])
+                         cigar_off, self.cigar[c0:c1], base_off, self.l_qseq[lo:hi], self.seq4[b0 // 2:b1 // 2],
+                         self.qual[b0:b1])
 
     def select(self, idx):
         """Sub-batch with the given (sorted) read indices; re-packs cigar / bases.  Every read keeps its base

@@ -3,7 +3,7 @@
 //
 // Replaces, for the drop-in BaseCellCounter, the per-window `pysam.AlignmentFile.pileup` fetches of
 // workflow/scripts/SNVCalling/BaseCellCounter.py:190-191,344-409 (the reference streams windows through a process
-// pool; here the reads stream through chunks and the windows are completed on the fly, see pipeline.stream_count).
+// pool; here the reads stream through chunks and the windows are completed on the fly, see pipeline.stream_chunks).
 //
 //   h = ls_bams_open(path, threads)                    header + contigs
 //   n = ls_bams_next(h, target_bytes, &n_cigar, &n_bases)   the next chunk: ~target_bytes inflated (members in parallel),

@@ -1,6 +1,6 @@
 """Host-side orchestration shared by the drop-in CLIs: BAM -> ReadBatch, barcode -> cell ids,
-window pruning, per-GPU sharding (no collective), the BaseCellCounter TSV writer and the streamed BAM sources of
-the counter (stream_count) and of the genotype scripts (stream_genotype).
+window pruning, per-GPU sharding (no collective), the BaseCellCounter TSV writer and the streamed BAM (stream_chunks)
+under the counter (stream_count) and the genotype scripts (stream_genotype).
 
 Reference counterparts: BaseCellCounter.main / run_interval / concatenate_sort_temp_files_and_write
 (BaseCellCounter.py:22-79,182-320,344-409).  GPU selection cannot be a CLI flag (the Snakemake
@@ -127,6 +127,14 @@ def read_ends(batch: ReadBatch):
     return batch.pos.astype(np.int64) + span
 
 
+def read_keys(batch: ReadBatch, ends):
+    """(start, end) keys tid << 32 | position of every read; the end is at least pos + 1, as the fetch of a pileup() call
+    sees it (bam_endpos)."""
+    tid = batch.tid.astype(np.int64) << 32
+    pos = batch.pos.astype(np.int64)
+    return tid | pos, tid | np.maximum(ends, pos + 1)
+
+
 def clean_barcodes_split(raw):
     """BaseCellCounter / SingleCellGenotype: barcode = CB.split('-')[0] (BaseCellCounter.py:246)."""
     return [b.split("-")[0] for b in raw]
@@ -152,8 +160,7 @@ def prune_and_sort_windows(named_windows, bam_names, batch, ends):
     iv = sorted((tid_of[c], s, e) for c, s, e in named_windows if c in tid_of and e > s)
     if not iv or batch.n_reads == 0:
         return []
-    rk_lo = (batch.tid.astype(np.int64) << 32) | batch.pos.astype(np.int64)
-    rk_hi = (batch.tid.astype(np.int64) << 32) | np.maximum(ends, batch.pos.astype(np.int64) + 1)
+    rk_lo, rk_hi = read_keys(batch, ends)
     run_max = np.maximum.accumulate(rk_hi)
     wk_lo = np.array([(t << 32) | s for t, s, e in iv], np.int64)
     wk_hi = np.array([(t << 32) | e for t, s, e in iv], np.int64)
@@ -198,9 +205,8 @@ def window_shards(batch: ReadBatch, windows: Windows, n_shards):
     nw = windows.n_windows
     if nw == 0 or batch.n_reads == 0 or n_shards <= 1:
         return [(batch, windows)]
-    ends = read_ends(batch)
-    rk_lo = (batch.tid.astype(np.int64) << 32) | batch.pos.astype(np.int64)
-    rk_hi = np.maximum.accumulate((batch.tid.astype(np.int64) << 32) | np.maximum(ends, batch.pos.astype(np.int64) + 1))
+    rk_lo, rk_hi = read_keys(batch, read_ends(batch))
+    rk_hi = np.maximum.accumulate(rk_hi)
     wk_lo = (windows.tid.astype(np.int64) << 32) | windows.start.astype(np.int64)
     wk_hi = (windows.tid.astype(np.int64) << 32) | windows.end.astype(np.int64)
     idx = np.minimum(np.searchsorted(wk_hi, rk_lo, side="right"), nw - 1)
@@ -251,7 +257,7 @@ def count_shards_pipelined(shards, params: CountParams, outs, device=0, lanes=2,
     return n_sites
 
 
-# ---- streaming BaseCellCounter: BAM chunks -> pinned staging -> GPU -> per-contig row files ---------------------------
+# ---- streamed BAM: chunks -> pinned staging -> one worker per device -> results in chunk order ------------------------
 class PinnedSlot:
     """One staging buffer set in pinned host memory (ls_host_alloc): the BAM decoder writes where the H2D copy reads.
     Arrays grow on demand and are reused for every chunk that goes through the slot.  Where the host refuses pinned
@@ -307,174 +313,192 @@ def _peak_rss_gb():
     return resource.getrusage(resource.RUSAGE_SELF).ru_maxrss / 1e6
 
 
-def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, ID, devices=None, chunk_bytes=None,
-                 stats_out=None):
-    """BaseCellCounter over a BAM of any size with bounded host memory (reference: the per-window pool of
-    BaseCellCounter.py:344-409).  Three stages run concurrently:
-      decoder : next ~chunk_bytes of the BAM -> pinned slot (behind the reads carried over from the previous chunk);
-                decides which windows are COMPLETE (no later read can reach them: reads are coordinate sorted) and which
-                reads must be carried on because they overlap a window that is not;
-      device  : ls_pileup_count on (carried + chunk reads, complete windows), one chunk per engine at a time;
-      writer  : native TSV rows appended to one file per contig; the files are concatenated in the reference's order
-                (contig name, start) at the end.
-    Returns the number of sites written."""
+def plan_chunk(read_start, read_end, region_start, region_end, first_region, last):
+    """One chunk of a streamed run.  read_start / read_end: read_keys() of the chunk's reads in coordinate order (the
+    carried reads first); region_start / region_end: keys of the regions, sorted by start and disjoint, so that their
+    ends are sorted too; first_region: the first region no earlier chunk completed; last: start key of the chunk's
+    last read, or None when no mapped read follows.
+    A region is complete once last >= its end: every later read starts at or after `last`, so none can overlap it.
+    Returns (done, send, carry): regions [first_region, done) are complete; `send` indexes the reads that overlap one
+    of them, which are all the records a fetch of those regions returns; `carry` indexes the reads whose end passes the
+    start of region `done`, the first incomplete one, and which go in front of the next chunk."""
+    nb = region_end.shape[0]
+    done = nb if last is None else max(first_region, int(np.searchsorted(region_end, last, side="right")))
+    # the first region from first_region on that ends after the read starts; regions are sorted, so it is the only
+    # one to test
+    j = np.maximum(np.searchsorted(region_end, read_start, side="right"), first_region)
+    send = np.nonzero((j < done) & (region_start[np.minimum(j, max(nb - 1, 0))] < read_end))[0] if done > first_region \
+        else np.zeros(0, np.int64)
+    carry = np.nonzero(read_end > region_start[done])[0] if done < nb else np.zeros(0, np.int64)
+    return done, send, carry
+
+
+plan_genotype_chunk = plan_chunk  # the genotype scripts' name: their regions are the genotype_bins()
+
+
+def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, chunk_bytes=None, make_engine=None):
+    """Streams a coordinate-sorted BAM of any size through regions with bounded host memory.
+      region_start, region_end : keys tid << 32 | position of the regions, as plan_chunk() takes them;
+      cell_map    : barcode text of a CB tag -> cell id, or -1; read once per barcode, on the decoder thread;
+      run         : run(engine, batch, ends, lo, done) -> result, for a chunk that completes regions [lo, done): batch
+                    holds the reads that overlap them, with cell ids, and ends their exclusive reference ends;
+      chunk_bytes : inflated BAM per chunk (default LONGSOM_CHUNK_MB, 256 MB);
+      make_engine : device -> engine of a worker (default take_engine).
+    A decoder thread fills len(devices) + 1 pinned slots in turn with the next chunk behind the reads carried from the
+    previous one and plans it (plan_chunk).  One worker per entry of `devices`, each with its own engine, calls `run`.
+    Yields (result, lo, done, stats) in chunk order; stats holds the device, n_reads (reads sent), n_carried (reads
+    the chunk carried in) and the engine's last_stats.  After the first error the workers only drain the queue, and
+    the error is raised once every thread has stopped.  Closing the generator stops the stream the same way."""
     import queue
-    import shutil
     devices = devices or [0]
     chunk_bytes = int(chunk_bytes or float(os.environ.get("LONGSOM_CHUNK_MB", "256")) * (1 << 20))
     bs = bamio.BamStream(bam_path)
-    tid_of = {n: i for i, n in enumerate(bs.contig_names)}
-    win = sorted((tid_of[c], s, e) for c, s, e in named_windows if c in tid_of and e > s)
-    wk_end = np.array([(t << 32) | e for t, s, e in win], np.int64)
-    wk_start = np.array([(t << 32) | s for t, s, e in win], np.int64)
-    n_slots = len(devices) + 1
-    free_slots = queue.Queue()
-    slots = [PinnedSlot() for _ in range(n_slots)]
+    slots = [PinnedSlot() for _ in range(len(devices) + 1)]
+    free_slots, todo, done_q = queue.Queue(), queue.Queue(maxsize=len(slots)), queue.Queue()
     for sl in slots:
         free_slots.put(sl)
-    todo, done = queue.Queue(maxsize=n_slots), queue.Queue()
-    errors = []
-    fasta_lock = threading.Lock()
-    busy = {"decode": 0.0, "host_glue": 0.0, "device": 0.0, "writer": 0.0}
-    clean_map = {"ids": np.zeros(0, np.int32), "table": {}, "names": []}
-
-    def cell_ids(raw, barcodes):
-        """raw barcode ids of the stream -> dense ids of cleaned barcodes (CB.split('-')[0], BaseCellCounter.py:246)."""
-        ids = clean_map["ids"]
-        if len(barcodes) > ids.shape[0]:
-            new = np.zeros(len(barcodes), np.int32)
-            new[:ids.shape[0]] = ids
-            for i in range(ids.shape[0], len(barcodes)):
-                c = barcodes[i].split("-")[0]
-                j = clean_map["table"].get(c)
-                if j is None:
-                    j = len(clean_map["names"])
-                    clean_map["table"][c] = j
-                    clean_map["names"].append(c)
-                new[i] = j
-            clean_map["ids"] = ids = new
-        out = np.full(raw.shape[0], -1, np.int32)
-        m = raw >= 0
-        out[m] = ids[raw[m]]
-        return out
+    errors, stop = [], threading.Event()
 
     def decoder():
+        seq, lo, carry, carry_ends, cell_of_raw = 0, 0, None, None, np.zeros(0, np.int32)
         try:
-            wi, seq, carry, carry_ends = 0, 0, None, None
-            while True:
+            while lo < region_end.shape[0] and not errors and not stop.is_set():
                 slot = free_slots.get()
-                t_a = time.time()
                 got = bs.next_chunk(chunk_bytes, slot, carry, carry_ends)
-                busy["decode"] += time.time() - t_a
-                t_a = time.time()
                 if got is None:
                     free_slots.put(slot)
-                    batch, last, ends = carry, None, carry_ends
-                    if batch is None or batch.n_reads == 0 or wi >= len(win):
+                    if carry is None:
                         break
-                    slot = None
+                    slot, batch, ends, n_carried, last = None, carry, carry_ends, carry.n_reads, None
                 else:
-                    batch, _n_new, ends = got
-                    last = (int(batch.tid[-1]) << 32) | int(batch.pos[-1])
-                # windows no future read can overlap: every later read starts at or after `last`
-                wj = len(win) if last is None else int(np.searchsorted(wk_end, last, side="right"))
-                wj = max(wj, wi)
-                rk_end = (batch.tid.astype(np.int64) << 32) | np.maximum(ends, batch.pos.astype(np.int64) + 1)
-                if wj > wi:
-                    iv = prune_and_sort_windows([(bs.contig_names[t], s, e) for t, s, e in win[wi:wj]], bs.contig_names, batch, ends)
-                    if iv:
-                        b2 = ReadBatch(batch.tid, batch.pos, batch.flag, batch.mapq, cell_ids(batch.cell, bs.barcodes),
-                                       batch.cigar_off, batch.cigar, batch.base_off, batch.l_qseq, batch.seq4, batch.qual)
-                        todo.put((seq, b2, iv, slot, win[wj][0] if wj < len(win) else (1 << 30)))
-                        seq += 1
-                        slot_in_use = True
-                    else:
-                        slot_in_use = False
-                else:
-                    slot_in_use = False
-                wi = wj
-                if last is None:
-                    if slot is not None and not slot_in_use:
-                        free_slots.put(slot)
-                    break
-                # reads that overlap a window which is not complete yet travel with the next chunk
-                if wi < len(win):
-                    keep = np.nonzero(rk_end > wk_start[wi])[0]
-                    carry = batch.select(keep) if keep.shape[0] else None
-                    carry_ends = ends[keep] if keep.shape[0] else None
-                else:
-                    carry, carry_ends = None, None
-                if not slot_in_use:
+                    batch, n_new, ends = got
+                    n_carried = batch.n_reads - n_new
+                    # unplaced reads (tid -1) close a coordinate-sorted BAM: no mapped read follows them
+                    last = None if batch.tid[-1] < 0 else (int(batch.tid[-1]) << 32) | int(batch.pos[-1])
+                done, send, keep = plan_chunk(*read_keys(batch, ends), region_start, region_end, lo, last)
+                carry, carry_ends = (batch.select(keep), ends[keep]) if keep.shape[0] else (None, None)
+                if send.shape[0]:
+                    sub = batch.slice(send[0], send[-1] + 1) if send[-1] - send[0] + 1 == send.shape[0] else batch.select(send)
+                    if len(bs.barcodes) > cell_of_raw.shape[0]:  # the table grows as new CB texts appear
+                        new = [cell_map(b) for b in bs.barcodes[cell_of_raw.shape[0]:]]
+                        cell_of_raw = np.concatenate([cell_of_raw, np.array(new, np.int32)])
+                    cell = np.full(sub.n_reads, -1, np.int32)
+                    tagged = sub.cell >= 0
+                    cell[tagged] = cell_of_raw[sub.cell[tagged]]
+                    sub.cell = cell
+                    todo.put((seq, sub, ends[send], n_carried, lo, done, slot))
+                    seq += 1
+                elif slot is not None:
                     free_slots.put(slot)
-                busy["host_glue"] += time.time() - t_a
-                if wi >= len(win):
+                lo = done
+                if last is None:
                     break
-        except Exception as ex:  # surfaced by the caller
+        except Exception as ex:  # raised by the generator
             errors.append(ex)
         finally:
             for _ in devices:
                 todo.put(None)
 
-    def device_worker(dev):
+    def worker(dev):
+        eng = None
         try:
-            eng = take_engine(dev)
-            try:
-                while True:
-                    item = todo.get()
-                    if item is None:
-                        break
-                    seq, batch, iv, slot, complete_tid = item
-                    t_a = time.time()
-                    with fasta_lock:
-                        contig_seq = {t: fasta.contig(bs.contig_names[t]) for t in sorted({w[0] for w in iv})}
-                    w = Windows.from_intervals(iv, contig_seq)
-                    sites = eng.pileup_count(batch, w, params)
-                    if stats_out is not None:
-                        stats_out.append(dict(device=dev, **eng.last_stats))
-                    if slot is not None:
-                        free_slots.put(slot)
-                    busy["device"] += time.time() - t_a
-                    done.put((seq, sites, complete_tid))
-            finally:
-                eng.close()
+            eng = (make_engine or take_engine)(dev)
         except Exception as ex:
             errors.append(ex)
+        try:
+            while True:
+                item = todo.get()
+                if item is None:
+                    break
+                seq, batch, ends, n_carried, lo, done, slot = item
+                try:
+                    if not errors and not stop.is_set():  # otherwise the queue is only drained: the decoder never blocks
+                        res = run(eng, batch, ends, lo, done)
+                        done_q.put((seq, (res, lo, done, dict(device=dev, n_reads=batch.n_reads, n_carried=n_carried,
+                                                               **eng.last_stats))))
+                except Exception as ex:
+                    errors.append(ex)
+                finally:
+                    if slot is not None:
+                        free_slots.put(slot)
         finally:
-            done.put(None)
+            if eng is not None:
+                eng.close()
+            done_q.put(None)
 
-    threads = [threading.Thread(target=decoder, daemon=True)] + [threading.Thread(target=device_worker, args=(d,), daemon=True)
-                                                                 for d in devices]
+    threads = [threading.Thread(target=decoder, daemon=True)] + [
+        threading.Thread(target=worker, args=(d,), daemon=True) for d in devices]
     for t in threads:
         t.start()
-    # writer (this thread): chunks in sequence order, rows appended to one temporary file per contig
-    host = bamio._load_host()
-    host.ls_write_counter_rows.argtypes = [C.c_char_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
-                                           C.c_int, C.c_int]
-    host.ls_write_counter_rows.restype = C.c_int
-    parts, pending, want, live, n_sites = {}, {}, 0, len(devices), 0
-    nthreads = min(16, len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1))
-    # The table lists the contigs in NAME order (collect_result sorts the window files by name), the BAM delivers them
-    # in header order: rows go to one part file per contig, and a part is appended to the output as soon as every
-    # contig before it in name order is complete -- at the end only the last few contigs are left to copy.
-    order = sorted({t for t, _s, _e in win}, key=lambda t: bs.contig_names[t])
-    state = {"out": None, "next": 0, "complete_tid": -1}
-    busy["concat"] = 0.0
+    try:
+        pending, want, live = {}, 0, len(devices)
+        while live:
+            item = done_q.get()
+            if item is None:
+                live -= 1
+                continue
+            pending[item[0]] = item[1]
+            while want in pending and not errors:
+                yield pending.pop(want)
+                want += 1
+        if errors:
+            raise errors[0]
+    finally:
+        stop.set()
+        for t in threads:
+            t.join()
+        for sl in slots:
+            sl.free()
+        bs.close()
 
-    def append_ready(everything=False):
-        t_cat = time.time()
-        while state["next"] < len(order) and (everything or order[state["next"]] < state["complete_tid"]):
-            t = order[state["next"]]
-            state["next"] += 1
-            path = parts.pop(t, None)
+
+def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, ID, devices=None, chunk_bytes=None,
+                 stats_out=None):
+    """BaseCellCounter over a BAM of any size with bounded host memory (reference: the per-window pool of
+    BaseCellCounter.py:344-409).  The windows are the regions of stream_chunks: a chunk runs ls_pileup_count on those
+    of its complete windows that a read reaches, and this thread appends the rows to one file per contig.  The table
+    lists the contigs in NAME order (collect_result sorts the window files by name), the BAM delivers them in header
+    order: a contig's file is appended to the table as soon as every contig before it in name order is complete, so at
+    the end only the last few are left to copy.  Returns the number of sites written; stats_out, if given, receives
+    the stats of every chunk."""
+    import contextlib
+    import shutil
+    bs = bamio.BamStream(bam_path)  # the header only: stream_chunks decodes the reads
+    names = bs.contig_names
+    bs.close()
+    tid_of = {n: i for i, n in enumerate(names)}
+    win = sorted((tid_of[c], s, e) for c, s, e in named_windows if c in tid_of and e > s)
+    order = sorted({t for t, _s, _e in win}, key=lambda t: names[t])
+    fasta_lock = threading.Lock()
+    busy = {"device": 0.0, "writer": 0.0, "concat": 0.0}
+    cells = {}  # cleaned barcode (CB.split('-')[0], BaseCellCounter.py:246) -> dense id in first-appearance order
+
+    def run(eng, batch, ends, lo, done):
+        t0 = time.time()
+        iv = prune_and_sort_windows([(names[t], s, e) for t, s, e in win[lo:done]], names, batch, ends)
+        with fasta_lock:
+            contig_seq = {t: fasta.contig(names[t]) for t in sorted({w[0] for w in iv})}
+        sites = eng.pileup_count(batch, Windows.from_intervals(iv, contig_seq), params)
+        busy["device"] += time.time() - t0
+        return sites
+
+    parts, out, next_part, n_sites = {}, None, 0, 0
+
+    def append_ready(complete_tid):
+        """Appends the files of the contigs that come next in name order and lie before complete_tid in the BAM."""
+        nonlocal out, next_part
+        t0 = time.time()
+        while next_part < len(order) and order[next_part] < complete_tid:
+            path = parts.pop(order[next_part], None)
+            next_part += 1
             if path is None:
                 continue
-            if state["out"] is None:
-                state["out"] = open(out_file, "wb")
-                state["out"].write(("##fileDate=%s\n" % time.strftime("%d/%m/%Y")).encode())
-                state["out"].write((COUNTER_CONCEPTS + "\n").encode())
-                state["out"].write(("\t".join(["#CHROM", "POS", "REF", "INFO", str(ID)]) + "\n").encode())
-                state["out"].flush()
-            out = state["out"]
+            if out is None:
+                out = open(out_file, "wb")
+                out.write(("##fileDate=%s\n" % time.strftime("%d/%m/%Y")).encode())
+                out.write((COUNTER_CONCEPTS + "\n").encode())
+                out.write(("\t".join(["#CHROM", "POS", "REF", "INFO", str(ID)]) + "\n").encode())
+                out.flush()
             with open(path, "rb") as f:
                 left = os.fstat(f.fileno()).st_size
                 try:  # in-kernel copy
@@ -490,78 +514,44 @@ def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, 
                     shutil.copyfileobj(f, out, 1 << 24)
                     out.flush()
             os.remove(path)
-        busy["concat"] += time.time() - t_cat
+        busy["concat"] += time.time() - t0
 
-    while live:
-        item = done.get()
-        if item is None:
-            live -= 1
-            continue
-        pending[item[0]] = (item[1], item[2])
-        t_w = time.time()
-        while want in pending:
-            sites, complete_tid = pending.pop(want)
-            want += 1
-            n_sites += sites.n_sites
-            for t in np.unique(sites.tid).tolist():
-                lo, hi = int(np.searchsorted(sites.tid, t, "left")), int(np.searchsorted(sites.tid, t, "right"))
-                path = parts.setdefault(t, "%s.part.%d.%d" % (out_file, os.getpid(), t))
-                pos = np.ascontiguousarray(sites.pos[lo:hi])
-                ref = np.ascontiguousarray(sites.ref[lo:hi])
-                cnt = np.ascontiguousarray(sites.counts[lo:hi])
-                rc = host.ls_write_counter_rows(os.fsencode(path), bs.contig_names[t].encode(), pos.ctypes.data, ref.ctypes.data,
-                                                cnt.ctypes.data, hi - lo, nthreads, 1)
-                if rc != 0:
-                    errors.append(IOError("ls_write_counter_rows(%s) failed: %d" % (path, rc)))
-            state["complete_tid"] = max(state["complete_tid"], complete_tid)
-            if not errors:
-                append_ready()
-        busy["writer"] += time.time() - t_w
-    for t in threads:
-        t.join()
-    for sl in slots:
-        sl.free()
-    bs.close()
+    wk_start = np.array([(t << 32) | s for t, s, e in win], np.int64)
+    wk_end = np.array([(t << 32) | e for t, s, e in win], np.int64)
+    cell_map = lambda b: cells.setdefault(b.split("-")[0], len(cells))
     try:
-        if errors:
-            raise errors[0]
+        with contextlib.closing(stream_chunks(bam_path, wk_start, wk_end, devices, cell_map, run, chunk_bytes)) as chunks:
+            for sites, _lo, done, stats in chunks:
+                t0 = time.time()
+                if stats_out is not None:
+                    stats_out.append(stats)
+                n_sites += sites.n_sites
+                for t in np.unique(sites.tid).tolist():
+                    path = parts.setdefault(t, "%s.part.%d.%d" % (out_file, os.getpid(), t))
+                    write_counter_rows(path, names[t], sites, t)
+                busy["writer"] += time.time() - t0
+                append_ready(win[done][0] if done < len(win) else len(names))
         if n_sites == 0:
             print("No temporary files found")
             return 0
-        append_ready(everything=True)
-        if state["out"] is not None:
-            state["out"].close()
-            state["out"] = None
+        append_ready(len(names))
+        out.close()
+        out = None
         if os.environ.get("LS_STREAM_TIMING"):
-            import resource
             print("[stream_count] busy seconds: " + ", ".join("%s %.2f" % kv for kv in sorted(busy.items())) +
                   "; peak RSS of this process %.2f GB" % _peak_rss_gb(), file=sys.stderr)
-            if os.environ.get("LS_STREAM_TIMING") == "2":   # what the resident set is made of (largest mappings)
-                try:
-                    maps, cur = [], None
-                    with open("/proc/self/smaps") as f:
-                        for line in f:
-                            if "-" in line.split(" ", 1)[0] and ":" not in line.split(" ", 1)[0]:
-                                cur = line.split()
-                            elif line.startswith("Rss:") and cur is not None:
-                                maps.append((int(line.split()[1]), cur[5] if len(cur) > 5 else "[anon]", cur[0]))
-                    maps.sort(reverse=True)
-                    print("[stream_count] largest resident mappings (MB): " +
-                          "; ".join("%d %s" % (kb // 1024, name) for kb, name, _ in maps[:10]), file=sys.stderr)
-                except OSError:
-                    pass
         return n_sites
     finally:
         for path in parts.values():
             if os.path.exists(path):
                 os.remove(path)
-        if state["out"] is not None:   # an error after the first contigs were appended: no partial table is left behind
-            state["out"].close()
+        if out is not None:   # an error after the first contigs were appended: no partial table is left behind
+            out.close()
             if os.path.exists(out_file):
                 os.remove(out_file)
 
 
-# ---- streaming genotype scripts: BAM chunks -> pinned staging -> K1' + K2 per chunk -> touched pairs ------------------
+# ---- streaming genotype scripts: BAM chunks -> K1' + K2 per chunk -> touched pairs -----------------------------------
 def genotype_bins(site_tid, site_pos, bin_size):
     """The pileup() calls of a genotype run as ls_genotype derives them from the sorted site table: one per run of sites
     with the same contig and floor(POS / bin_size) of the 1-based POS, over [first pos - 1, last pos + 1) (0-based).
@@ -577,32 +567,6 @@ def genotype_bins(site_tid, site_pos, bin_size):
     return first, (tid[lo] << 32) | np.maximum(pos[lo] - 1, 0), (tid[hi] << 32) | (pos[hi] + 1)
 
 
-def read_keys(batch: ReadBatch, ends):
-    """(start, end) keys tid << 32 | position of every read; the end is at least pos + 1, as the fetch of a pileup() call
-    sees it (bam_endpos)."""
-    tid = batch.tid.astype(np.int64) << 32
-    pos = batch.pos.astype(np.int64)
-    return tid | pos, tid | np.maximum(ends, pos + 1)
-
-
-def plan_genotype_chunk(read_start, read_end, bin_start, bin_end, first_bin, last):
-    """One chunk of a streamed genotype run.  read_start / read_end: read_keys() of the chunk's reads in coordinate
-    order (the carried reads first); bin_start / bin_end: region keys of genotype_bins(); first_bin: the first bin no
-    earlier chunk completed; last: start key of the chunk's last read, or None when no mapped read follows.
-    A bin is complete once last >= its end: every later read starts at or after `last`, so none can overlap it.
-    Returns (done, send, carry): bins [first_bin, done) are complete; `send` indexes the reads that overlap one of
-    them, which are all the records their pileup() calls fetch; `carry` indexes the reads whose end passes the start of
-    bin `done`, the first incomplete one, and which go in front of the next chunk."""
-    nb = bin_end.shape[0]
-    done = nb if last is None else max(first_bin, int(np.searchsorted(bin_end, last, side="right")))
-    # the first bin from first_bin on that ends after the read starts; bins are sorted, so it is the only one to test
-    j = np.maximum(np.searchsorted(bin_end, read_start, side="right"), first_bin)
-    send = np.nonzero((j < done) & (bin_start[np.minimum(j, max(nb - 1, 0))] < read_end))[0] if done > first_bin \
-        else np.zeros(0, np.int64)
-    carry = np.nonzero(read_end > bin_start[done])[0] if done < nb else np.zeros(0, np.int64)
-    return done, send, carry
-
-
 def stream_genotype(bam_path, sites, bins, n_cells, cell_map, geno_params, alpha, beta, skip_p, devices, chunk_bytes=None,
                     stats_out=None, make_engine=None):
     """Touched (site, cell) pairs of SingleCellGenotype / HCCVSingleCellGenotype over a BAM of any size with bounded host
@@ -613,132 +577,39 @@ def stream_genotype(bam_path, sites, bins, n_cells, cell_map, geno_params, alpha
       cell_map    : barcode text of a CB tag -> column in [0, n_cells), or -1;
       geno_params : the other keyword arguments of genotype_sparse (min_bq, min_mq, max_depth, alt_only);
       skip_p      : per site, 1 where no tail is evaluated (None: none);
-      chunk_bytes : inflated BAM per chunk (default LONGSOM_CHUNK_MB, 256 MB);
-      make_engine : device -> engine of a worker (default take_engine).
-    A decoder thread fills pinned slots with the next chunk behind the reads carried from the previous one and plans it
-    (plan_genotype_chunk).  One worker per entry of `devices`, each with its own engine, uploads the reads that overlap
-    the chunk's complete bins and runs genotype_sparse on the contiguous slice of the site table those bins hold.  A
-    chunk then holds every record the whole-file call fetches for those bins, in the same order, so the depth cap drops
-    the same records.  Sites no read reaches get no pairs.  stats_out, if given, receives one dict per device call."""
-    import queue
+      chunk_bytes, make_engine : as stream_chunks takes them.
+    The bins are the regions of stream_chunks: a chunk uploads the reads that overlap its complete bins and runs
+    genotype_sparse on the contiguous slice of the site table those bins hold.  A chunk then holds every record the
+    whole-file call fetches for those bins, in the same order, so the depth cap drops the same records.  Sites no read
+    reaches get no pairs.  stats_out, if given, receives the stats of every chunk with its site rows [site_lo, site_hi)."""
+    import contextlib
     site_tid, site_pos, alt_cls = (np.ascontiguousarray(a, t) for a, t in zip(sites, (np.int32, np.int32, np.uint8)))
     skip = None if skip_p is None else np.ascontiguousarray(skip_p, np.uint8)
     first, bstart, bend = genotype_bins(site_tid, site_pos, bins)
     empty = (np.zeros(0, np.int32),) * 4 + (np.zeros(0, np.float64),)
     if bend.shape[0] == 0:
         return empty
-    devices = devices or [0]
-    chunk_bytes = int(chunk_bytes or float(os.environ.get("LONGSOM_CHUNK_MB", "256")) * (1 << 20))
-    bs = bamio.BamStream(bam_path)
-    slots = [PinnedSlot() for _ in range(len(devices) + 1)]
-    free_slots = queue.Queue()
-    for sl in slots:
-        free_slots.put(sl)
-    todo, done_q = queue.Queue(maxsize=len(slots)), queue.Queue()
-    errors = []
-    columns = {"of_raw": np.zeros(0, np.int32)}
 
-    def to_columns(raw):
-        """raw barcode ids of the stream -> columns; the table grows as new CB texts appear."""
-        old = columns["of_raw"]
-        if len(bs.barcodes) > old.shape[0]:
-            columns["of_raw"] = np.concatenate([old, np.array([cell_map(b) for b in bs.barcodes[old.shape[0]:]], np.int32)])
-        out = np.full(raw.shape[0], -1, np.int32)
-        m = raw >= 0
-        out[m] = columns["of_raw"][raw[m]]
-        return out
+    def run(eng, batch, _ends, lo, done):
+        lo, hi = int(first[lo]), int(first[done])
+        eng.upload(batch, None)
+        site, cell, dp, alt, p = eng.genotype_sparse(site_tid[lo:hi], site_pos[lo:hi], alt_cls[lo:hi], n_cells, alpha,
+                                                     beta, skip_p=None if skip is None else skip[lo:hi], bin_size=bins,
+                                                     **geno_params)
+        site += lo  # chunk-local site rows -> rows of the whole table
+        return site, cell, dp, alt, p
 
-    def decoder():
-        seq = 0
-        try:
-            bi, carry, carry_ends = 0, None, None
-            while bi < bend.shape[0] and not errors:
-                slot = free_slots.get()
-                got = bs.next_chunk(chunk_bytes, slot, carry, carry_ends)
-                if got is None:
-                    free_slots.put(slot)
-                    if carry is None:
-                        break
-                    slot, batch, ends, n_carried, last = None, carry, carry_ends, carry.n_reads, None
-                else:
-                    batch, n_new, ends = got
-                    n_carried = batch.n_reads - n_new
-                    # unplaced reads (tid -1) close a coordinate-sorted BAM: no mapped read follows them
-                    last = None if batch.tid[-1] < 0 else (int(batch.tid[-1]) << 32) | int(batch.pos[-1])
-                rs, re_ = read_keys(batch, ends)
-                bj, send, keep = plan_genotype_chunk(rs, re_, bstart, bend, bi, last)
-                carry, carry_ends = (batch.select(keep), ends[keep]) if keep.shape[0] else (None, None)
-                if send.shape[0]:
-                    sub = batch.slice(send[0], send[-1] + 1) if send[-1] - send[0] + 1 == send.shape[0] else batch.select(send)
-                    sub.cell = to_columns(sub.cell)
-                    todo.put((seq, sub, int(first[bi]), int(first[bj]), slot, n_carried))
-                    seq += 1
-                elif slot is not None:
-                    free_slots.put(slot)
-                bi = bj
-                if last is None:
-                    break
-        except Exception as ex:  # surfaced by the caller
-            errors.append(ex)
-        finally:
-            for _ in devices:
-                todo.put(None)
-
-    def device_worker(dev):
-        eng = None
-        try:
-            eng = (make_engine or take_engine)(dev)
-        except Exception as ex:
-            errors.append(ex)
-        try:
-            while True:
-                item = todo.get()
-                if item is None:
-                    break
-                seq, batch, lo, hi, slot, n_carried = item
-                try:
-                    if not errors:  # after an error the queue is only drained, so that the decoder never blocks
-                        eng.upload(batch, None)
-                        site, cell, dp, alt, p = eng.genotype_sparse(
-                            site_tid[lo:hi], site_pos[lo:hi], alt_cls[lo:hi], n_cells, alpha, beta,
-                            skip_p=None if skip is None else skip[lo:hi], bin_size=bins, **geno_params)
-                        site += lo  # chunk-local site rows -> rows of the whole table
-                        if stats_out is not None:
-                            stats_out.append(dict(device=dev, n_reads=batch.n_reads, n_carried=n_carried, site_lo=lo,
-                                                  site_hi=hi, **eng.last_stats))
-                        done_q.put((seq, (site, cell, dp, alt, p)))
-                except Exception as ex:
-                    errors.append(ex)
-                finally:
-                    if slot is not None:
-                        free_slots.put(slot)
-        finally:
-            if eng is not None:
-                eng.close()
-            done_q.put(None)
-
-    threads = [threading.Thread(target=decoder, daemon=True)] + [
-        threading.Thread(target=device_worker, args=(d,), daemon=True) for d in devices]
-    for t in threads:
-        t.start()
-    parts, live = {}, len(devices)
-    while live:
-        item = done_q.get()
-        if item is None:
-            live -= 1
-        else:
-            parts[item[0]] = item[1]
-    for t in threads:
-        t.join()
-    for sl in slots:
-        sl.free()
-    bs.close()
-    if errors:
-        raise errors[0]
+    parts = []
+    with contextlib.closing(stream_chunks(bam_path, bstart, bend, devices, cell_map, run, chunk_bytes,
+                                          make_engine)) as chunks:
+        for tup, lo, done, stats in chunks:
+            parts.append(tup)
+            if stats_out is not None:
+                stats_out.append(dict(stats, site_lo=int(first[lo]), site_hi=int(first[done])))
     if not parts:
         return empty
     # chunks cover disjoint, increasing site slices: in chunk order the pairs are ordered by (site, cell)
-    return tuple(np.concatenate([parts[s][k] for s in sorted(parts)]) for k in range(5))
+    return tuple(np.concatenate([p[k] for p in parts]) for k in range(5))
 
 
 def format_counter_lines(chrom, pos, ref, counts):
@@ -768,22 +639,27 @@ def write_counter_tsv(out_file, ID, sites: SiteCounts, bam_names):
         out.write("##fileDate=%s\n" % time.strftime("%d/%m/%Y"))
         out.write(COUNTER_CONCEPTS + "\n")
         out.write("\t".join(["#CHROM", "POS", "REF", "INFO", str(ID)]) + "\n")
+    for t in sorted(np.unique(sites.tid).tolist(), key=lambda t: bam_names[t]):
+        write_counter_rows(out_file, bam_names[t], sites, t)
+    return True
+
+
+def write_counter_rows(path, chrom, sites: SiteCounts, tid):
+    """Appends the TSV rows of contig `tid` to path with the native formatter (ls_write_counter_rows).  The rows of one
+    contig are contiguous: sites are ordered by window = (tid, start)."""
     host = bamio._load_host()
     host.ls_write_counter_rows.argtypes = [C.c_char_p, C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                            C.c_int, C.c_int]
     host.ls_write_counter_rows.restype = C.c_int
-    tids = np.unique(sites.tid)
-    for t in sorted(tids.tolist(), key=lambda t: bam_names[t]):
-        # rows of one contig are contiguous (sites are ordered by window = (tid, start)) -> native formatter
-        lo, hi = int(np.searchsorted(sites.tid, t, "left")), int(np.searchsorted(sites.tid, t, "right"))
-        pos = np.ascontiguousarray(sites.pos[lo:hi])
-        ref = np.ascontiguousarray(sites.ref[lo:hi])
-        cnt = np.ascontiguousarray(sites.counts[lo:hi])
-        rc = host.ls_write_counter_rows(os.fsencode(out_file), bam_names[t].encode(), pos.ctypes.data, ref.ctypes.data,
-                                        cnt.ctypes.data, hi - lo, min(16, len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)), 1)
-        if rc != 0:
-            raise IOError("ls_write_counter_rows(%s) failed: %d" % (out_file, rc))
-    return True
+    lo, hi = int(np.searchsorted(sites.tid, tid, "left")), int(np.searchsorted(sites.tid, tid, "right"))
+    pos = np.ascontiguousarray(sites.pos[lo:hi])
+    ref = np.ascontiguousarray(sites.ref[lo:hi])
+    cnt = np.ascontiguousarray(sites.counts[lo:hi])
+    threads = min(16, len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1))
+    rc = host.ls_write_counter_rows(os.fsencode(path), chrom.encode(), pos.ctypes.data, ref.ctypes.data, cnt.ctypes.data,
+                                    hi - lo, threads, 1)
+    if rc != 0:
+        raise IOError("ls_write_counter_rows(%s) failed: %d" % (path, rc))
 
 
 def load_bam_for_counting(bam_path, mode="split"):
