@@ -59,7 +59,23 @@ const char *ls_bams_contig_name(void *h, int i);
 int32_t ls_bams_contig_len(void *h, int i);
 int32_t ls_bams_n_barcodes(void *h);
 const char *ls_bams_barcode(void *h, int i);
+/* Optional, after ls_bams_open and before the first ls_bams_next: the run only needs the records that overlap the n
+ * regions [beg[i], end[i]) of reference tid[i] (0-based, any order; regions that touch are merged).  The reader then
+ * reads and inflates only the BGZF members of the spans the BAM's .bai index lists for them (SAM spec 5.3), merged into
+ * disjoint spans in file order, and hands out exactly the records of those spans: every record that overlaps a region,
+ * and possibly others, in file order.  The index is <bam>.bai, else <bam without .bam>.bai; CSI is not read.
+ * Returns 1 when the index is used; 0 when there is none or it is refused, and the whole file is read as without the
+ * call: an index that cannot be parsed, whose reference count differs from the header's, that is older than the BAM
+ * (mtime: a stale index could change the records a region gets), or one of whose offsets is past the end of the file
+ * or not inside a BGZF member.  ls_bams_index_note() then gives the reason in one line (NULL while the index is used).
+ * -1 when called after ls_bams_next or on a handle in error. */
+int ls_bams_set_regions(void *h, int64_t n, const int32_t *tid, const int64_t *beg, const int64_t *end);
+const char *ls_bams_index_note(void *h);
 int64_t ls_bams_next(void *h, int64_t target_bytes, int64_t *n_cigar, int64_t *n_bases);
+/* Compressed BGZF member bytes read and bytes inflated to produce the chunk the last ls_bams_next returned (the call that
+ * returned 0 included).  With the index, the header's members are not counted; without it, they count in the first
+ * chunk. */
+void ls_bams_chunk_io(void *h, int64_t *compressed, int64_t *inflated);
 int ls_bams_fill(void *h, int32_t *tid, int32_t *pos, uint16_t *flag, uint8_t *mapq, int32_t *cb, int32_t *l_qseq,
                  uint32_t *cigar_off, uint64_t *base_off, uint32_t *cigar, uint8_t *seq4, uint8_t *qual);
 /* the same, plus ref_end[i] = pos + M/D/N/=/X lengths of read i (exclusive reference end; may be NULL) */

@@ -144,6 +144,11 @@ class BamStream:
             lib.ls_bams_contig_len.argtypes = [C.c_void_p, C.c_int]
             lib.ls_bams_barcode.restype = C.c_char_p
             lib.ls_bams_barcode.argtypes = [C.c_void_p, C.c_int]
+            lib.ls_bams_set_regions.restype = C.c_int
+            lib.ls_bams_set_regions.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
+            lib.ls_bams_index_note.restype = C.c_char_p
+            lib.ls_bams_index_note.argtypes = [C.c_void_p]
+            lib.ls_bams_chunk_io.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
             lib._bams_ready = True
         threads = threads or min(16, len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1))
         self.h = lib.ls_bams_open(os.fsencode(path), int(threads))
@@ -151,6 +156,20 @@ class BamStream:
         self.contig_names = [lib.ls_bams_contig_name(self.h, i).decode() for i in range(lib.ls_bams_n_contigs(self.h))]
         self.contig_lens = [lib.ls_bams_contig_len(self.h, i) for i in range(len(self.contig_names))]
         self.barcodes = []
+        self.compressed_bytes = self.inflated_bytes = 0  # of the chunks decoded so far
+
+    def set_regions(self, tid, beg, end):
+        """Read only the BGZF members the .bai lists for the regions [beg, end) of reference tid (arrays); call before
+        the first next_chunk.  Returns None when the index is used, else the one-line reason why the whole file is
+        read (see ls_bams_set_regions)."""
+        tid = np.ascontiguousarray(tid, np.int32)
+        beg = np.ascontiguousarray(beg, np.int64)
+        end = np.ascontiguousarray(end, np.int64)
+        rc = self.lib.ls_bams_set_regions(self.h, tid.shape[0], tid.ctypes.data, beg.ctypes.data, end.ctypes.data)
+        if rc < 0:
+            self._check()
+            raise ValueError("BamStream.set_regions: call it before the first next_chunk")
+        return None if rc == 1 else self.lib.ls_bams_index_note(self.h).decode(errors="replace")
 
     def _check(self):
         err = self.lib.ls_bams_error(self.h)
@@ -173,6 +192,10 @@ class BamStream:
         the carried reads in `head`)."""
         nc, nb = C.c_int64(0), C.c_int64(0)
         n = self.lib.ls_bams_next(self.h, int(target_bytes), C.byref(nc), C.byref(nb))
+        cb, ib = C.c_int64(0), C.c_int64(0)
+        self.lib.ls_bams_chunk_io(self.h, C.byref(cb), C.byref(ib))
+        self.compressed_bytes += cb.value
+        self.inflated_bytes += ib.value
         if n < 0:
             self._check()
             raise IOError("BAM stream: decode failed")

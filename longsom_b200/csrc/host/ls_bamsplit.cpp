@@ -32,6 +32,7 @@
 #include <unordered_map>
 #include <vector>
 
+#include "ls_bai.h"
 #include "ls_bgzf.h"
 
 using namespace lsbgzf;
@@ -100,16 +101,6 @@ static AuxHit find_aux(const uint8_t *p, const uint8_t *end, char t0, char t1) {
   return h;
 }
 
-static int reg2bin(int64_t beg, int64_t end) {
-  --end;
-  if (beg >> 14 == end >> 14) return (int)(((1 << 15) - 1) / 7 + (beg >> 14));
-  if (beg >> 17 == end >> 17) return (int)(((1 << 12) - 1) / 7 + (beg >> 17));
-  if (beg >> 20 == end >> 20) return (int)(((1 << 9) - 1) / 7 + (beg >> 20));
-  if (beg >> 23 == end >> 23) return (int)(((1 << 6) - 1) / 7 + (beg >> 23));
-  if (beg >> 26 == end >> 26) return (int)(((1 << 3) - 1) / 7 + (beg >> 26));
-  return 0;
-}
-
 static void put32(std::vector<uint8_t> &v, uint32_t x) {
   uint8_t b[4];
   wr32(b, x);
@@ -145,14 +136,14 @@ struct BaiBuilder {
       return;
     }
     Ref &r = refs[(size_t)tid];
-    const int b = reg2bin(beg, end);
+    const int b = lsbai::reg2bin(beg, end);
     auto &ch = r.bins[(uint32_t)b];
     if (b == r.last_bin && !ch.empty() && ch.back().second == u0)
       ch.back().second = u1;  // consecutive records of one bin form one chunk
     else
       ch.emplace_back(u0, u1);
     r.last_bin = b;
-    const size_t w0 = (size_t)(beg >> 14), w1 = (size_t)((end - 1) >> 14);
+    const size_t w0 = (size_t)(beg >> lsbai::kLinShift), w1 = (size_t)((end - 1) >> lsbai::kLinShift);
     if (r.lin.size() <= w1) r.lin.resize(w1 + 1, UINT64_MAX);
     for (size_t w = w0; w <= w1; ++w)
       if (r.lin[w] == UINT64_MAX) r.lin[w] = u0;
@@ -178,7 +169,7 @@ struct BaiBuilder {
         }
       }
       if (r.any) {
-        put32(bai, 37450u);
+        put32(bai, lsbai::kMetaBin);
         put32(bai, 2u);
         put64(bai, voff(r.off_beg));
         put64(bai, voff(r.off_end));

@@ -6,6 +6,8 @@
 // pool; here the reads stream through chunks and the windows are completed on the fly, see pipeline.stream_chunks).
 //
 //   h = ls_bams_open(path, threads)                    header + contigs
+//   ls_bams_set_regions(h, n, tid, beg, end)           optional: read only the BGZF members that the .bai lists for
+//                                                      these regions (see read_index for when the index is refused)
 //   n = ls_bams_next(h, target_bytes, &n_cigar, &n_bases)   the next chunk: ~target_bytes inflated (members in parallel),
 //                                                      complete records indexed; a record cut by the chunk end is
 //                                                      carried over.  The chunk AFTER it is inflated and indexed by a
@@ -14,13 +16,23 @@
 //                                                      memory of the CUDA library: the decoder writes where the H2D
 //                                                      copy reads)
 // Barcodes (CB:Z) are interned across chunks: ids are stable for the whole file.
+// The compressed input is a list of segments, whole BGZF members each: the whole file, or one per span of virtual
+// offsets the index gives for the regions.  A segment's first member is parsed from the span's in-block offset on and
+// its last member up to the span's end, so the inflated bytes are exactly the records of the spans, in file order.
 // Every length field is checked against the bytes that are actually there: a truncated or corrupt file is an error
 // string, never an out-of-bounds read.
 #include <zlib.h>
 
+#include "ls_bai.h"
 #include "ls_inflate.h"
 
+#include <fcntl.h>
+#include <sys/stat.h>
+#include <unistd.h>
+
+#include <algorithm>
 #include <atomic>
+#include <cerrno>
 #include <chrono>
 #include <cstdint>
 #include <cstdio>
@@ -43,6 +55,16 @@ struct Member {
   size_t coff;     // offset in the compressed buffer
   uint32_t csize, usize;
   size_t uoff;     // offset in the inflated buffer (after the carried bytes)
+  uint32_t skip, keep_end;  // the member's inflated bytes [skip, keep_end) are kept
+};
+
+// Compressed bytes [c0, c1) of the file, whole members.  The first member's inflated bytes start at `skip`; the member
+// at last_coff (if any) ends at last_keep.
+struct Segment {
+  uint64_t c0, c1;
+  uint32_t skip;
+  uint64_t last_coff;
+  uint32_t last_keep;
 };
 
 // Byte buffer that grows without zero-filling (a std::vector would clear 256 MB per chunk before inflate overwrites it)
@@ -76,6 +98,7 @@ struct Chunk {
   std::vector<int32_t> cb;
   int64_t n = 0;                      // complete records; -1 = error (err)
   int64_t n_cigar = 0, n_bases = 0;
+  int64_t comp_bytes = 0, infl_bytes = 0;  // compressed member bytes read and bytes inflated to produce the chunk
   int32_t n_barcodes = 0;             // size of the barcode table when the chunk was indexed
   std::string err;
 };
@@ -123,14 +146,22 @@ struct BarcodeTable {
 };
 
 struct Stream {
-  std::string err;
-  FILE *f = nullptr;
+  std::string err, path;
+  int fd = -1;
+  uint64_t file_size = 0;
   int threads = 1;
   double t_read = 0, t_inflate = 0, t_index = 0, t_tags = 0, t_intern = 0, t_fill = 0, t_wait = 0;  // LS_BAM_TIMING
-  bool header_done = false, eof = false;
+  bool header_done = false, started = false;
   std::vector<std::string> contig_names;
   std::vector<int32_t> contig_lens;
   BarcodeTable bar;
+  std::vector<Segment> segs;  // what is read, in file order
+  size_t seg = 0;             // the segment being read
+  uint64_t rd_off = 0;        // next file offset of segs[seg] to read
+  uint64_t comp_file_off = 0; // file offset of comp[comp_lo]
+  std::string index_note = "regions not set";  // why the index is not used ("" when it is)
+  int64_t comp_bytes = 0, infl_bytes = 0;  // since the last chunk was produced
+  int64_t tot_comp = 0, tot_infl = 0;      // of the chunks handed out
   std::vector<uint8_t> comp;  // compressed bytes read but not yet consumed
   size_t comp_lo = 0;         // first unconsumed byte of comp
   Chunk ch[2];
@@ -194,10 +225,25 @@ const char *find_cb(const uint8_t *p, const uint8_t *end) {
 }
 
 
-// Make sure at least `want` unconsumed compressed bytes are buffered (or the file is exhausted).  Bytes below `pin`
-// (the first member of the call in progress, still to be inflated) are kept; returns how far the buffer was shifted.
+bool pread_all(int fd, uint8_t *dst, size_t n, uint64_t off) {
+  while (n) {
+    const ssize_t k = pread(fd, dst, n, (off_t)off);
+    if (k < 0 && errno == EINTR) continue;
+    if (k <= 0) return false;
+    dst += k;
+    n -= (size_t)k;
+    off += (uint64_t)k;
+  }
+  return true;
+}
+
+// Make sure at least `want` unconsumed compressed bytes of the current segment are buffered (or the segment is
+// exhausted).  Bytes below `pin` (the first member of the call in progress, still to be inflated) are kept; returns
+// how far the buffer was shifted.
 size_t refill(Stream *s, size_t want, size_t pin) {
-  if (s->comp.size() - s->comp_lo >= want || s->eof) return 0;
+  if (s->comp.size() - s->comp_lo >= want || s->seg >= s->segs.size()) return 0;
+  const Segment &g = s->segs[s->seg];
+  if (s->rd_off >= g.c1) return 0;
   size_t shift = 0;
   if (pin) {
     s->comp.erase(s->comp.begin(), s->comp.begin() + (ptrdiff_t)pin);
@@ -205,13 +251,19 @@ size_t refill(Stream *s, size_t want, size_t pin) {
     shift = pin;
   }
   const size_t have = s->comp.size();
-  const size_t grab = want > (size_t)(8u << 20) ? want : (size_t)(8u << 20);
+  // the header is read in small steps: with an index, what follows it is not needed
+  const size_t step = s->header_done ? (size_t)(8u << 20) : (size_t)(256u << 10);
+  const size_t grab = (size_t)std::min<uint64_t>(std::max(want, step), g.c1 - s->rd_off);
   s->comp.resize(have + grab);
   const double t0 = now_s();
-  const size_t got = fread(s->comp.data() + have, 1, grab, s->f);
+  const bool ok = pread_all(s->fd, s->comp.data() + have, grab, s->rd_off);
   s->t_read += now_s() - t0;
-  s->comp.resize(have + got);
-  if (got < grab) s->eof = true;
+  if (!ok) {  // the file is shorter than it was: what is buffered is all there is
+    s->comp.resize(have);
+    s->rd_off = g.c1;
+    return shift;
+  }
+  s->rd_off += grab;
   return shift;
 }
 
@@ -231,9 +283,14 @@ bool inflate_some(Stream *s, ByteBuf &raw, size_t target, std::string &err) {
   };
   for (;;) {
     if (!need(18)) {
-      if (s->comp.size() - s->comp_lo == 0) break;
-      err = "truncated BGZF member header";
-      return false;
+      if (s->comp.size() - s->comp_lo != 0) {
+        err = "truncated BGZF member header";
+        return false;
+      }
+      if (s->seg + 1 >= s->segs.size()) break;
+      ++s->seg;  // the next segment starts in an empty buffer
+      s->rd_off = s->comp_file_off = s->segs[s->seg].c0;
+      continue;
     }
     const uint8_t *p = s->comp.data() + s->comp_lo;
     if (p[0] != 0x1f || p[1] != 0x8b || !(p[3] & 4)) {
@@ -270,10 +327,20 @@ bool inflate_some(Stream *s, ByteBuf &raw, size_t target, std::string &err) {
       err = "corrupt BGZF block (ISIZE > 64 KiB)";
       return false;
     }
+    const Segment &g = s->segs[s->seg];
+    m.skip = s->comp_file_off == g.c0 ? g.skip : 0;
+    m.keep_end = s->comp_file_off == g.last_coff ? g.last_keep : m.usize;
+    if (m.skip > m.keep_end || m.keep_end > m.usize) {
+      err = "index offset past the end of a BGZF member";
+      return false;
+    }
     m.uoff = raw0 + usum;
     mem.push_back(m);
-    usum += m.usize;
+    usum += m.keep_end - m.skip;
+    s->comp_bytes += bsize;
+    s->infl_bytes += m.usize;
     s->comp_lo += bsize;
+    s->comp_file_off += bsize;
     if (usum >= target) break;
   }
   if (mem.empty()) return true;
@@ -286,6 +353,7 @@ bool inflate_some(Stream *s, ByteBuf &raw, size_t target, std::string &err) {
   std::atomic<size_t> next(0);
   std::atomic<int> bad(0);
   auto worker = [&]() {
+    std::vector<uint8_t> part;  // a member only partly kept is inflated here first
     z_stream zs;
     memset(&zs, 0, sizeof zs);
     if (inflateInit2(&zs, -15) != Z_OK) {
@@ -295,9 +363,17 @@ bool inflate_some(Stream *s, ByteBuf &raw, size_t target, std::string &err) {
     for (;;) {
       const size_t i = next.fetch_add(8);
       if (i >= mem.size()) break;
-      for (size_t j = i; j < i + 8 && j < mem.size(); ++j)
-        if (mem[j].usize && !inflate_block(zs, s->comp.data() + mem[j].coff, mem[j].csize, raw.p + mem[j].uoff, mem[j].usize))
-          bad = 1;
+      for (size_t j = i; j < i + 8 && j < mem.size(); ++j) {
+        const Member &m = mem[j];
+        if (!m.usize) continue;
+        if (m.skip == 0 && m.keep_end == m.usize) {
+          if (!inflate_block(zs, s->comp.data() + m.coff, m.csize, raw.p + m.uoff, m.usize)) bad = 1;
+          continue;
+        }
+        part.resize((size_t)m.usize + 8);
+        if (!inflate_block(zs, s->comp.data() + m.coff, m.csize, part.data(), m.usize)) bad = 1;
+        else memcpy(raw.p + m.uoff, part.data() + m.skip, m.keep_end - m.skip);
+      }
     }
     inflateEnd(&zs);
   };
@@ -362,6 +438,15 @@ void produce(Stream *s, Chunk &dst, const Chunk &prev, size_t target) {
   dst.recs.clear();
   dst.n = 0;
   dst.n_cigar = dst.n_bases = 0;
+  struct Account {  // the bytes read since the previous chunk are this chunk's, whichever way produce() returns
+    Stream *s;
+    Chunk &c;
+    ~Account() {
+      c.comp_bytes = s->comp_bytes;
+      c.infl_bytes = s->infl_bytes;
+      s->comp_bytes = s->infl_bytes = 0;
+    }
+  } account{s, dst};
   const size_t carry = prev.raw.n - prev.tail_lo;
   if (!dst.raw.resize(carry + 8)) {
     dst.err = "out of memory";
@@ -473,6 +558,105 @@ void produce(Stream *s, Chunk &dst, const Chunk &prev, size_t target) {
   s->t_intern += now_s() - t_x2;
 }
 
+// The BGZF member at file offset off: its compressed size and ISIZE; false when off is not at a whole member.
+bool member_at(const Stream *s, uint64_t off, uint32_t &bsize, uint32_t &isize) {
+  uint8_t hd[18], tl[4];
+  if (off + 26 > s->file_size || !pread_all(s->fd, hd, 18, off)) return false;
+  if (hd[0] != 0x1f || hd[1] != 0x8b || hd[2] != 8 || !(hd[3] & 4) || rd16(hd + 10) != 6 || hd[12] != 'B' ||
+      hd[13] != 'C' || rd16(hd + 14) != 2)
+    return false;
+  bsize = (uint32_t)rd16(hd + 16) + 1;
+  if (bsize < 26 || off + bsize > s->file_size || !pread_all(s->fd, tl, 4, off + bsize - 4)) return false;
+  isize = rd32(tl);
+  return isize <= 65536u;
+}
+
+// Reads <bam>.bai (or <bam without .bam>.bai) and turns the regions' queries into segments.  An index that is missing,
+// unreadable, older than the BAM, made for another header, or that points anywhere but into whole members of the file
+// is not used: false, with the reason in s->index_note.
+bool use_index(Stream *s, int64_t n, const int32_t *tid, const int64_t *beg, const int64_t *end,
+               std::vector<Segment> &segs) {
+  std::string bai = s->path + ".bai";
+  struct stat sb, si;
+  if (stat(bai.c_str(), &si) != 0 && s->path.size() > 4 && s->path.compare(s->path.size() - 4, 4, ".bam") == 0)
+    bai = s->path.substr(0, s->path.size() - 4) + ".bai";
+  if (stat(bai.c_str(), &si) != 0) {
+    s->index_note = "no .bai index";
+    return false;
+  }
+  if (fstat(s->fd, &sb) != 0 || si.st_mtim.tv_sec < sb.st_mtim.tv_sec ||
+      (si.st_mtim.tv_sec == sb.st_mtim.tv_sec && si.st_mtim.tv_nsec < sb.st_mtim.tv_nsec)) {
+    s->index_note = bai + " is older than the BAM";
+    return false;
+  }
+  std::vector<uint8_t> buf;
+  {
+    const int fd = open(bai.c_str(), O_RDONLY | O_CLOEXEC);
+    struct stat st;
+    bool ok = fd >= 0 && fstat(fd, &st) == 0;
+    if (ok) {
+      buf.resize((size_t)st.st_size);
+      ok = pread_all(fd, buf.data(), buf.size(), 0);
+    }
+    if (fd >= 0) close(fd);
+    if (!ok) {
+      s->index_note = "cannot read " + bai;
+      return false;
+    }
+  }
+  lsbai::Index idx;
+  std::string why;
+  if (!lsbai::parse(buf.data(), buf.size(), idx, why)) {
+    s->index_note = bai + ": " + why;
+    return false;
+  }
+  if (idx.refs.size() != s->contig_names.size()) {
+    s->index_note = bai + " lists " + std::to_string(idx.refs.size()) + " references, the BAM header " +
+                    std::to_string(s->contig_names.size());
+    return false;
+  }
+  // regions that overlap or touch are one query
+  std::vector<std::pair<int64_t, int64_t>> reg;  // (tid << 32 | beg, end)
+  for (int64_t i = 0; i < n; ++i)
+    if (tid[i] >= 0 && (size_t)tid[i] < idx.refs.size() && end[i] > beg[i] && end[i] > 0)
+      reg.emplace_back(((int64_t)tid[i] << 32) | std::max<int64_t>(beg[i], 0), end[i]);
+  std::sort(reg.begin(), reg.end());
+  std::vector<lsbai::Chunk> spans;
+  for (size_t i = 0; i < reg.size();) {
+    const int64_t t = reg[i].first >> 32, b = reg[i].first & 0xffffffffll;
+    int64_t e = reg[i].second;
+    size_t j = i + 1;
+    for (; j < reg.size() && (reg[j].first >> 32) == t && (reg[j].first & 0xffffffffll) <= e; ++j)
+      e = std::max(e, reg[j].second);
+    lsbai::query(idx.refs[(size_t)t], b, e, spans);
+    i = j;
+  }
+  lsbai::merge_spans(spans);
+  segs.clear();
+  for (const lsbai::Chunk &c : spans) {
+    const uint64_t c0 = c.first >> 16, c1 = c.second >> 16;
+    const uint32_t u0 = (uint32_t)(c.first & 0xffff), u1 = (uint32_t)(c.second & 0xffff);
+    uint32_t bsize = 0, isize = 0;
+    Segment g{c0, c1, u0, c1, u1};
+    if (!member_at(s, c0, bsize, isize) || u0 > isize || (!segs.empty() && c0 < segs.back().c1)) {
+      s->index_note = bai + ": a chunk starts outside the BAM's BGZF members";
+      return false;
+    }
+    if (u1) {
+      if (!member_at(s, c1, bsize, isize) || u1 > isize) {
+        s->index_note = bai + ": a chunk ends outside the BAM's BGZF members";
+        return false;
+      }
+      g.c1 = c1 + bsize;
+    } else if (c1 > s->file_size || (c1 < s->file_size && !member_at(s, c1, bsize, isize))) {
+      s->index_note = bai + ": a chunk ends outside the BAM's BGZF members";
+      return false;
+    }
+    segs.push_back(g);
+  }
+  return true;
+}
+
 }  // namespace
 
 extern "C" {
@@ -480,11 +664,15 @@ extern "C" {
 void *ls_bams_open(const char *path, int threads) {
   Stream *s = new Stream();
   s->threads = threads < 1 ? 1 : threads;
-  s->f = fopen(path, "rb");
-  if (!s->f) {
+  s->path = path;
+  s->fd = open(path, O_RDONLY | O_CLOEXEC);
+  struct stat st;
+  if (s->fd < 0 || fstat(s->fd, &st) != 0) {
     s->err = std::string("cannot open ") + path;
     return s;
   }
+  s->file_size = (uint64_t)st.st_size;
+  s->segs.push_back(Segment{0, s->file_size, 0, UINT64_MAX, 0});
   // the header may span several members; what follows it in the inflated bytes is the first chunk's carry
   Chunk &c0 = s->ch[0];
   size_t consumed = 0;
@@ -515,9 +703,11 @@ void ls_bams_close(void *h) {
   if (s->pf_running) s->pf.join();
   if (getenv("LS_BAM_TIMING"))
     fprintf(stderr, "[ls_bamstream] file read %.2f s, inflate %.2f s, record boundaries %.2f s, CB tags %.2f s, barcode ids + offsets "
-                    "%.2f s (all on the prefetch thread), fill %.2f s, caller waited %.2f s for prefetched chunks\n",
-            s->t_read, s->t_inflate, s->t_index, s->t_tags, s->t_intern, s->t_fill, s->t_wait);
-  if (s->f) fclose(s->f);
+                    "%.2f s (all on the prefetch thread), fill %.2f s, caller waited %.2f s for prefetched chunks; "
+                    "compressed bytes read %lld, inflated bytes %lld, index %s\n",
+            s->t_read, s->t_inflate, s->t_index, s->t_tags, s->t_intern, s->t_fill, s->t_wait, (long long)s->tot_comp,
+            (long long)s->tot_infl, s->index_note.empty() ? "used" : s->index_note.c_str());
+  if (s->fd >= 0) close(s->fd);
   delete s;
 }
 int32_t ls_bams_n_contigs(void *h) { return (int32_t)((Stream *)h)->contig_names.size(); }
@@ -532,6 +722,35 @@ const char *ls_bams_barcode(void *h, int i) {
   Stream *s = (Stream *)h;
   std::lock_guard<std::mutex> g(s->bar.mu);
   return s->bar.names[(size_t)i].c_str();
+}
+
+int ls_bams_set_regions(void *h, int64_t n, const int32_t *tid, const int64_t *beg, const int64_t *end) {
+  Stream *s = (Stream *)h;
+  if (!s->err.empty() || !s->header_done || s->started) return -1;
+  std::vector<Segment> segs;
+  if (!use_index(s, n, tid, beg, end, segs)) return 0;
+  // the bytes the header read past itself are not records of the regions
+  s->segs.swap(segs);
+  s->seg = 0;
+  s->rd_off = s->comp_file_off = s->segs.empty() ? 0 : s->segs[0].c0;
+  s->comp.clear();
+  s->comp_lo = 0;
+  s->comp_bytes = s->infl_bytes = 0;
+  Chunk &c0 = s->ch[0];
+  c0.raw.n = c0.tail_lo;
+  s->index_note.clear();
+  return 1;
+}
+
+const char *ls_bams_index_note(void *h) {
+  Stream *s = (Stream *)h;
+  return s->index_note.empty() ? nullptr : s->index_note.c_str();
+}
+
+void ls_bams_chunk_io(void *h, int64_t *compressed, int64_t *inflated) {
+  Stream *s = (Stream *)h;
+  *compressed = s->ch[s->cur].comp_bytes;
+  *inflated = s->ch[s->cur].infl_bytes;
 }
 
 // Next chunk: number of complete records (0 = end of file, -1 = error).  The records stay valid until the next call.
@@ -550,6 +769,9 @@ int64_t ls_bams_next(void *h, int64_t target_bytes, int64_t *n_cigar, int64_t *n
   }
   s->cur = 1 - s->cur;
   Chunk &c = s->ch[s->cur];
+  s->started = true;
+  s->tot_comp += c.comp_bytes;
+  s->tot_infl += c.infl_bytes;
   if (c.n < 0) {
     s->err = c.err.empty() ? "BAM stream: decode failed" : c.err;
     return -1;

@@ -346,13 +346,22 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
       make_engine : device -> engine of a worker (default take_engine).
     A decoder thread fills len(devices) + 1 pinned slots in turn with the next chunk behind the reads carried from the
     previous one and plans it (plan_chunk).  One worker per entry of `devices`, each with its own engine, calls `run`.
+    The reader is given the regions: where the BAM has a usable .bai it reads and inflates only the BGZF members the
+    index lists for them (bamio.BamStream.set_regions), which hold every record that overlaps a region, in file order;
+    plan_chunk drops the others.  Without one it reads the whole file.
     Yields (result, lo, done, stats) in chunk order; stats holds the device, n_reads (reads sent), n_carried (reads
-    the chunk carried in) and the engine's last_stats.  After the first error the workers only drain the queue, and
+    the chunk carried in), indexed (the .bai is used), compressed_bytes / inflated_bytes (what the reader read and
+    inflated since the previous yielded chunk) and the engine's last_stats.  After the first error the workers only drain the queue, and
     the error is raised once every thread has stopped.  Closing the generator stops the stream the same way."""
     import queue
     devices = devices or [0]
     chunk_bytes = int(chunk_bytes or float(os.environ.get("LONGSOM_CHUNK_MB", "256")) * (1 << 20))
     bs = bamio.BamStream(bam_path)
+    key_tid = (np.asarray(region_start, np.int64) >> 32).astype(np.int32)
+    index_note = bs.set_regions(key_tid, np.asarray(region_start, np.int64) & 0xffffffff,
+                                np.asarray(region_end, np.int64) & 0xffffffff)
+    if index_note is not None and not index_note.startswith("no .bai"):
+        print("[longsom] %s: index not used, reading the whole BAM: %s" % (bam_path, index_note), file=sys.stderr)
     slots = [PinnedSlot() for _ in range(len(devices) + 1)]
     free_slots, todo, done_q = queue.Queue(), queue.Queue(maxsize=len(slots)), queue.Queue()
     for sl in slots:
@@ -361,6 +370,7 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
 
     def decoder():
         seq, lo, carry, carry_ends, cell_of_raw = 0, 0, None, None, np.zeros(0, np.int32)
+        io_sent = (0, 0)  # reader bytes already reported with an earlier chunk
         try:
             while lo < region_end.shape[0] and not errors and not stop.is_set():
                 slot = free_slots.get()
@@ -386,7 +396,11 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
                     tagged = sub.cell >= 0
                     cell[tagged] = cell_of_raw[sub.cell[tagged]]
                     sub.cell = cell
-                    todo.put((seq, sub, ends[send], n_carried, lo, done, slot))
+                    io = (bs.compressed_bytes, bs.inflated_bytes)
+                    todo.put((seq, sub, ends[send], n_carried, lo, done, slot,
+                              dict(indexed=index_note is None, compressed_bytes=io[0] - io_sent[0],
+                                   inflated_bytes=io[1] - io_sent[1])))
+                    io_sent = io
                     seq += 1
                 elif slot is not None:
                     free_slots.put(slot)
@@ -410,12 +424,12 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
                 item = todo.get()
                 if item is None:
                     break
-                seq, batch, ends, n_carried, lo, done, slot = item
+                seq, batch, ends, n_carried, lo, done, slot, io = item
                 try:
                     if not errors and not stop.is_set():  # otherwise the queue is only drained: the decoder never blocks
                         res = run(eng, batch, ends, lo, done)
                         done_q.put((seq, (res, lo, done, dict(device=dev, n_reads=batch.n_reads, n_carried=n_carried,
-                                                               **eng.last_stats))))
+                                                               **io, **eng.last_stats))))
                 except Exception as ex:
                     errors.append(ex)
                 finally:
