@@ -162,6 +162,29 @@ int ls_pileup_fetch(ls_ctx *ctx, ls_site_counts *out);
 int ls_pileup_count(ls_ctx *ctx, const ls_read_batch *batch, const ls_windows *windows,
                     const ls_count_params *params, ls_site_counts *out, ls_run_stats *stats);
 
+/* ---- K1 table text ------------------------------------------------------------------------------
+ * The rows of BaseCellCounter's table (BaseCellCounter.py:297-309) written as text on the device from the compacted
+ * sites of the last run, in site order, instead of fetching the counts and formatting them on the host; the text
+ * equals ls_write_counter_rows' (longsom_host.h).  Per site:
+ *   chrom \t pos+1 \t REF \t DP|NC|CC|BC|BQ|BCf|BCr \t DP|NC|CC|BC|BQ|BCf|BCr values \n
+ * where each of the five vectors is six ':'-joined numbers and BC = BCf + BCr in uint32 (wrapping).
+ *   text_load : valid after ls_pileup_run (compacts first if that has not been done).  names: the contig names back to
+ *               back, indexed by tid through name_off[0 .. n_names]; each at most 65535 bytes.  Measures every row on
+ *               the device and writes each contig's site range [contig_lo[t], contig_hi[t]) (empty: lo == hi == 0).
+ *               LS_E_ARG for a site whose tid is outside [0, n_names) or sites not grouped by ascending tid.  A new
+ *               upload or run discards the load.
+ *   text      : the rows of the sites site_lo .. site_lo + *sites_done - 1 (below site_hi), as many whole rows as fit
+ *               in capacity bytes at out (a host buffer, pinned or not).  A row longer than capacity is LS_E_CAPACITY,
+ *               a call without a load since the last run LS_E_STATE; site_lo == site_hi gives (0, 0).            */
+/* The caller's site table (n_sites and the four arrays, ordered as a run orders them) in place of the last run's
+ * compacted sites, as if a run had produced it: text_load and fetch then work on it.  Lets a table whose counts no run
+ * can reach (sums near 2^32) be formatted; the next upload or run replaces it.                                     */
+int ls_pileup_sites_upload(ls_ctx *ctx, const ls_site_counts *sites);
+int ls_pileup_text_load(ls_ctx *ctx, const char *names, const int64_t *name_off, int32_t n_names, int64_t *contig_lo,
+                        int64_t *contig_hi);
+int ls_pileup_text(ls_ctx *ctx, int64_t site_lo, int64_t site_hi, char *out, int64_t capacity, int64_t *sites_done,
+                   int64_t *bytes);
+
 /* ---- K1': pileup at candidate sites, per (site, cell) ------------------------------------
  * Replaces SingleCellGenotype.run_interval's pileup loop (SingleCellGenotype.py:114-178) and
  * HCCVSingleCellGenotype.run_interval (:112-176).  Uses the batch of the last

@@ -23,7 +23,8 @@ ABI_SYMBOLS = [
     "ls_genotype_sparse_run", "ls_genotype_sparse_fetch",
     "ls_betabinom_sf", "ls_site_mask", "ls_site_table_load", "ls_site_table_lookup", "ls_device_synchronize", "ls_device_pci_bus_id", "ls_flush_l2",
     "ls_geno_matrix_load", "ls_geno_matrix_text", "ls_geno_long_load", "ls_geno_long_text", "ls_geno_long_times",
-    "ls_geno_long_release",
+    "ls_geno_long_release", "ls_pileup_text_load", "ls_pileup_text",
+    "ls_pileup_sites_upload",
 ]
 LS_GENO_MATRIX_DP, LS_GENO_MATRIX_ALT, LS_GENO_MATRIX_VAF, LS_GENO_MATRIX_BINARY = 0, 1, 2, 3
 LS_GENO_ROW_CHRM, LS_GENO_ROW_FUSION = 1, 2
@@ -121,6 +122,9 @@ def load():
     lib.ls_pileup_fetch.argtypes = [C.c_void_p, P(LsSiteCounts)]
     lib.ls_pileup_count.argtypes = [C.c_void_p, P(LsReadBatch), P(LsWindows), P(LsCountParams), P(LsSiteCounts),
                                     P(LsRunStats)]
+    lib.ls_pileup_sites_upload.argtypes = [C.c_void_p, P(LsSiteCounts)]
+    lib.ls_pileup_text_load.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+    lib.ls_pileup_text.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, P(C.c_int64), P(C.c_int64)]
     lib.ls_genotype_count.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                       P(LsGenoParams), C.c_void_p, C.c_void_p, P(LsRunStats)]
     lib.ls_genotype_sparse_run.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,

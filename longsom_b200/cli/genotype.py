@@ -28,9 +28,7 @@ import os
 import re
 import sys
 import threading
-import time
 import timeit
-from concurrent.futures import ThreadPoolExecutor
 from contextlib import nullcontext
 
 import numpy as np
@@ -40,6 +38,7 @@ from pandas._libs.parsers import STR_NA_VALUES
 from .. import bamio
 from .._lib import (CLASS_ID, LS_CLASS_NA, LS_GENO_MATRIX_ALT, LS_GENO_MATRIX_BINARY, LS_GENO_MATRIX_DP,
                     LS_GENO_MATRIX_VAF, LS_GENO_ROW_CHRM, LS_GENO_ROW_FUSION, LS_E_ARG, LongSomError)
+from ..blocks import PinnedBlock, write_blocks
 from ..engine import Engine
 from ..pipeline import devices_from_env, stream_genotype
 
@@ -348,7 +347,7 @@ def long_rows_device(eng, out, lay, tuples, cell_text, hccv, pvalue):
         fixed += 3 + np.fromiter((len(x) for x in lay.index), np.int64, len(lay.index))
     longest = fixed * n_cells + sum(len(x) for x in cell_text) + (LONG_TAIL_MAX - 18) * (lay.hit_hi - lay.hit_lo)
     cap = max(LONG_BLOCK_BYTES, int(longest.max()) if len(longest) else 0)
-    bufs = [_PinnedBlock(eng, cap) for _ in range(2)]
+    bufs = [PinnedBlock(eng, cap) for _ in range(2)]
     try:
         write_s = write_blocks(out, eng.geno_long_text, len(lay.prefix), bufs, cap)
         times = eng.geno_long_times()
@@ -528,7 +527,7 @@ def write_matrices(args, src, fusions, engine=None):
         # whole rows per block: the longest possible row fits any block
         longest = max(len(x.encode()) for x in lay.labels) + 1 + 13 * len(lay.columns) + 16
         cap = max(MATRIX_BLOCK_BYTES, longest)
-        bufs = [_PinnedBlock(eng, cap) for _ in range(2)]
+        bufs = [PinnedBlock(eng, cap) for _ in range(2)]
         header = ('\t' + '\t'.join(lay.columns) + '\n').encode()
         try:
             for name, kind in MATRIX_KINDS:
@@ -540,47 +539,6 @@ def write_matrices(args, src, fusions, engine=None):
             for b in bufs:
                 b.free()
     return True
-
-
-def write_blocks(f, text, n, bufs, cap):
-    """Units (rows or sites) 0 .. n-1 to file f in blocks: text(lo, addr, cap) formats as many whole units from lo as
-    fit in cap bytes at addr and returns (units, bytes).  Block i is formatted into bufs[i] while the file thread still
-    writes block i ^ 1.  Returns the seconds the file writes took."""
-    def put(view):
-        t = time.perf_counter()
-        f.write(view)
-        return time.perf_counter() - t
-    spent, lo, i, pending = 0.0, 0, 0, None
-    with ThreadPoolExecutor(1) as pool:
-        while lo < n:
-            units, nb = text(lo, bufs[i].addr, cap)
-            if pending is not None:
-                spent += pending.result()
-            pending = pool.submit(put, bufs[i].view[:nb])
-            lo += units
-            i ^= 1
-        if pending is not None:
-            spent += pending.result()
-    return spent
-
-
-class _PinnedBlock:
-    """A block buffer in pinned host memory (pageable where the host refuses to pin it)."""
-
-    def __init__(self, eng, nbytes):
-        self._lib, self._ptr = eng._lib, C.c_void_p()
-        if self._lib.ls_host_alloc(C.c_size_t(nbytes), C.byref(self._ptr)) != 0:
-            self._ptr, self._keep = None, C.create_string_buffer(nbytes)
-            self.addr = C.addressof(self._keep)
-        else:
-            self.addr = self._ptr.value
-        self.view = memoryview((C.c_char * nbytes).from_address(self.addr)).cast('B')
-
-    def free(self):
-        self.view.release()
-        if self._ptr is not None:
-            self._lib.ls_host_free(self._ptr)
-            self._ptr = None
 
 
 def initialize_parser(hccv):

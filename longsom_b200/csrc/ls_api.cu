@@ -143,6 +143,7 @@ extern "C" int ls_pileup_upload(ls_ctx *ctx, const ls_read_batch *b, const ls_wi
   if (!b) LS_FAIL(LS_E_ARG, "ls_pileup_upload: batch is null");
   ctx->have_batch = false;
   ctx->have_run = false;
+  ctx->ct.loaded = false;
   ctx->replay.valid = false;
   const int64_t n = b->n_reads;
   if (n < 0 || b->n_cigar < 0 || b->n_bases < 0) LS_FAIL(LS_E_ARG, "ls_pileup_upload: negative size");

@@ -166,6 +166,16 @@ struct GenoLongState {
   }
 };
 
+// The counter table's row offsets, kept between ls_pileup_text_load and the ls_pileup_text calls
+struct CounterTextState {
+  DBuf names, name_off;  // contig names back to back, [n_names+1] offsets rebased to 0
+  DBuf lens, off;        // [n_sites] row bytes; [n_sites+1] their 64-bit exclusive scan
+  DBuf range, result;    // [2][n_names] each contig's site range; load: input error flags, text: (last site, bytes)
+  DBuf out;              // per text call: the block's text
+  int64_t n_sites = 0;
+  bool loaded = false;   // cleared by ls_pileup_upload and ls_pileup_run
+};
+
 // What a replay of ls_pileup_run takes from the last run on the batch that it can stand for
 struct ReplaySnapshot {
   bool valid = false;
@@ -223,6 +233,7 @@ struct ls_ctx {
   GenoState geno;  // K1'
   GenoMatrixState gm;  // genotype matrix writer
   GenoLongState gl;    // genotype long-table writer
+  CounterTextState ct;  // counter table writer
 };
 
 #define LS_CK(call)                                                                        \
@@ -322,10 +333,14 @@ struct LsScanJob {
   uint32_t *out;
   int64_t n;
   uint64_t *total;  // may be null
+  uint64_t *out64 = nullptr;  // ls_scan_exclusive_u32_wide only: the 64-bit prefixes
 };
 cudaError_t ls_scan_exclusive_u32_multi(const LsScanJob *jobs, int n_jobs, DBuf &tmp, cudaStream_t st);
 cudaError_t ls_scan_exclusive_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n, uint64_t *d_total,
                                   DBuf &tmp, cudaStream_t st);
+// d_out[0 .. n]: exclusive prefix sums of d_in as 64-bit values, d_out[n] the total; every 2048 consecutive inputs
+// must sum below 2^32
+cudaError_t ls_scan_exclusive_u32_wide(const uint32_t *d_in, uint64_t *d_out, int64_t n, DBuf &tmp, cudaStream_t st);
 cudaError_t ls_radix_sort_pairs(uint64_t *keys_a, uint64_t *keys_b, uint32_t *vals_a, uint32_t *vals_b,
                                 int64_t n, int key_bits, DBuf &hist, uint64_t **sorted_keys,
                                 uint32_t **sorted_vals, int num_sms, cudaStream_t st, int *launches);

@@ -412,6 +412,7 @@ extern "C" int ls_pileup_run(ls_ctx *ctx, const ls_count_params *params, int64_t
   ctx->params = *params;
   ctx->have_run = false;
   ctx->compacted = false;
+  ctx->ct.loaded = false;
   ls_run_stats S;
   memset(&S, 0, sizeof S);
   int launches = 0;

@@ -51,7 +51,9 @@ struct ScanJobs {
   int64_t nb_max;
 };
 
-// blockIdx.y = the array (several independent scans share one launch)
+// blockIdx.y = the array (several independent scans share one launch).  WIDE: the prefixes go to job.out64 as 64-bit
+// values, for sums that may pass 2^32 (a chunk's own sum must still fit 32 bits)
+template <bool WIDE>
 __global__ void __launch_bounds__(SCAN_THREADS) scan_chained(ScanJobs jobs) {
   __shared__ uint32_t sm[SCAN_THREADS / 32 + 1];
   __shared__ uint32_t bid_s;
@@ -110,6 +112,15 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_chained(ScanJobs jobs) {
     }
   }
   __syncthreads();
+  if (WIDE) {
+    uint64_t e = pfx_s + ex;
+#pragma unroll
+    for (int i = 0; i < SCAN_ITEMS; ++i) {
+      if (base + i < n) job.out64[base + i] = e;
+      e += v[i];
+    }
+    return;
+  }
   ex += (uint32_t)pfx_s;
   if (base + SCAN_ITEMS <= n) {
     uint4 a, b;
@@ -306,9 +317,8 @@ cudaError_t radix_sort_impl(K *keys_a, K *keys_b, uint32_t *vals_a, uint32_t *va
   return cudaGetLastError();
 }
 
-}  // namespace
-
-cudaError_t ls_scan_exclusive_u32_multi(const LsScanJob *jobs, int n_jobs, DBuf &tmp, cudaStream_t st) {
+template <bool WIDE>
+cudaError_t scan_multi(const LsScanJob *jobs, int n_jobs, DBuf &tmp, cudaStream_t st) {
   if (n_jobs < 1 || n_jobs > LS_SCAN_MAX_JOBS) return cudaErrorInvalidValue;
   ScanJobs a;
   int64_t nb_max = 0;
@@ -322,6 +332,7 @@ cudaError_t ls_scan_exclusive_u32_multi(const LsScanJob *jobs, int n_jobs, DBuf 
       continue;
     }
     if ((reinterpret_cast<uintptr_t>(jobs[k].in) | reinterpret_cast<uintptr_t>(jobs[k].out)) & 15u) return cudaErrorMisalignedAddress;
+    if (WIDE != (jobs[k].out64 != nullptr)) return cudaErrorInvalidValue;
     a.j[live++] = jobs[k];
     const int64_t nb = (jobs[k].n + SCAN_CHUNK - 1) / SCAN_CHUNK;
     nb_max = nb > nb_max ? nb : nb_max;
@@ -336,8 +347,25 @@ cudaError_t ls_scan_exclusive_u32_multi(const LsScanJob *jobs, int n_jobs, DBuf 
   a.state = tmp.as<unsigned long long>();
   a.ticket = reinterpret_cast<unsigned int *>(tmp.as<unsigned long long>() + (size_t)live * (size_t)nb_max);
   a.nb_max = nb_max;
-  scan_chained<<<dim3((unsigned)nb_max, (unsigned)live), SCAN_THREADS, 0, st>>>(a);
+  scan_chained<WIDE><<<dim3((unsigned)nb_max, (unsigned)live), SCAN_THREADS, 0, st>>>(a);
   return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t ls_scan_exclusive_u32_multi(const LsScanJob *jobs, int n_jobs, DBuf &tmp, cudaStream_t st) {
+  return scan_multi<false>(jobs, n_jobs, tmp, st);
+}
+
+cudaError_t ls_scan_exclusive_u32_wide(const uint32_t *d_in, uint64_t *d_out, int64_t n, DBuf &tmp, cudaStream_t st) {
+  if (n <= 0) return cudaMemsetAsync(d_out, 0, sizeof(uint64_t), st);
+  LsScanJob j;
+  j.in = d_in;
+  j.out = nullptr;
+  j.n = n;
+  j.total = d_out + n;
+  j.out64 = d_out;
+  return scan_multi<true>(&j, 1, tmp, st);
 }
 
 cudaError_t ls_scan_exclusive_u32(const uint32_t *d_in, uint32_t *d_out, int64_t n, uint64_t *d_total, DBuf &tmp,

@@ -2,6 +2,7 @@
 
 Mirrors the reference's unit operations:
   Engine.pileup_count     <-> BaseCellCounter.run_interval          (BaseCellCounter.py:182-320)
+  Engine.pileup_count_text <-> the same, with its rows as text     (BaseCellCounter.py:297-309)
   Engine.genotype_count   <-> SingleCellGenotype.run_interval loop  (SingleCellGenotype.py:114-178)
   Engine.genotype_sparse  <-> the same loop + its betabinom.sf calls (SingleCellGenotype.py:114-218), touched pairs only
   Engine.betabinom_sf     <-> scipy.stats.betabinom.sf call sites   (BaseCellCalling.step1.py:196,201)
@@ -11,10 +12,12 @@ Mirrors the reference's unit operations:
 Every method runs on the GPU; there is no CPU path behind any of them.
 """
 import ctypes as C
+import time
 
 import numpy as np
 
 from . import _lib as L
+from .blocks import PinnedBlock, counter_block_bytes, counter_text
 from .batch import ReadBatch, SiteCounts, Windows
 
 
@@ -41,8 +44,12 @@ class Engine:
         self.device = device
         self.last_stats = None
         self._keep = None
+        self._blocks = []  # the two pinned blocks of pileup_count_text, kept across calls
 
     def close(self):
+        for b in getattr(self, "_blocks", ()):
+            b.free()
+        self._blocks = []
         if getattr(self, "_ctx", None):
             self._lib.ls_ctx_destroy(self._ctx)
             self._ctx = None
@@ -107,6 +114,51 @@ class Engine:
                                               C.byref(st)), "ls_pileup_count")
         self.last_stats = st.as_dict()
         return int(s.n_sites)
+
+    def pileup_sites_upload(self, sites: SiteCounts):
+        """Places a site table where a run leaves its compacted sites (ls_pileup_sites_upload), for the text writer."""
+        sites = SiteCounts(np.ascontiguousarray(sites.tid, np.int32), np.ascontiguousarray(sites.pos, np.int32),
+                           np.ascontiguousarray(sites.ref, np.uint8), np.ascontiguousarray(sites.counts, np.uint32))
+        s = sites.as_struct()
+        s.n_sites = sites.n_sites
+        self._keep = sites
+        self._check(self._lib.ls_pileup_sites_upload(self._ctx, C.byref(s)), "ls_pileup_sites_upload")
+
+    def pileup_text_load(self, names):
+        """Measures the rows of the last run's sites on the device (ls_pileup_text_load).  names: contig names (bytes)
+        indexed by tid.  Returns (lo, hi): int64 arrays, contig t's sites are [lo[t], hi[t])."""
+        off = np.zeros(len(names) + 1, np.int64)
+        np.cumsum(np.fromiter((len(x) for x in names), np.int64, len(names)), out=off[1:])
+        blob = b"".join(names)
+        lo, hi = np.zeros(len(names), np.int64), np.zeros(len(names), np.int64)
+        self._check(self._lib.ls_pileup_text_load(self._ctx, C.cast(C.c_char_p(blob), C.c_void_p), off.ctypes.data,
+                                                  len(names), lo.ctypes.data, hi.ctypes.data), "ls_pileup_text_load")
+        return lo, hi
+
+    def pileup_text(self, site_lo, site_hi, out, capacity):
+        """Rows of the whole sites site_lo.. (below site_hi) that fit in `capacity` bytes at address `out`: (sites
+        written, bytes)."""
+        sites, nb = C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.ls_pileup_text(self._ctx, int(site_lo), int(site_hi), out, int(capacity), C.byref(sites),
+                                             C.byref(nb)), "ls_pileup_text")
+        return int(sites.value), int(nb.value)
+
+    def pileup_count_text(self, batch: ReadBatch, windows: Windows, params: CountParams, names):
+        """upload + run + the rows as text, formatted on the device into the engine's two pinned blocks: {tid: text}
+        (memoryviews of host memory), each contig's rows in site order, as ls_write_counter_rows writes them.  names: contig names (bytes) indexed
+        by tid.  last_stats gains n_sites and text_s (the seconds of the text load and calls)."""
+        self.upload(batch, windows)
+        n = self.run(params)
+        t0 = time.perf_counter()
+        cap = counter_block_bytes(names)
+        if not self._blocks or self._blocks[0].nbytes < cap:
+            for b in self._blocks:
+                b.free()
+            self._blocks = []
+            self._blocks = [PinnedBlock(self, cap) for _ in range(2)]
+        text = counter_text(self, names, self._blocks)
+        self.last_stats.update(n_sites=n, text_s=time.perf_counter() - t0)
+        return text
 
     # ---- K1' -----------------------------------------------------------------------------
     def genotype_count(self, site_tid, site_pos, alt_class, n_cells, min_bq=30, min_mq=255, max_depth=200000,

@@ -350,8 +350,8 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
     index lists for them (bamio.BamStream.set_regions), which hold every record that overlaps a region, in file order;
     plan_chunk drops the others.  Without one it reads the whole file.
     Yields (result, lo, done, stats) in chunk order; stats holds the device, n_reads (reads sent), n_carried (reads
-    the chunk carried in), indexed (the .bai is used), compressed_bytes / inflated_bytes (what the reader read and
-    inflated since the previous yielded chunk) and the engine's last_stats.  After the first error the workers only drain the queue, and
+    the chunk carried in), indexed (the .bai is used), compressed_bytes / inflated_bytes / decode_s (what the reader
+    read and inflated, and the decoder thread's seconds, since the previous yielded chunk) and the engine's last_stats.  After the first error the workers only drain the queue, and
     the error is raised once every thread has stopped.  Closing the generator stops the stream the same way."""
     import queue
     devices = devices or [0]
@@ -371,9 +371,11 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
     def decoder():
         seq, lo, carry, carry_ends, cell_of_raw = 0, 0, None, None, np.zeros(0, np.int32)
         io_sent = (0, 0)  # reader bytes already reported with an earlier chunk
+        decode_s = 0.0    # decoder seconds not yet reported with a chunk
         try:
             while lo < region_end.shape[0] and not errors and not stop.is_set():
                 slot = free_slots.get()
+                t0 = time.perf_counter()
                 got = bs.next_chunk(chunk_bytes, slot, carry, carry_ends)
                 if got is None:
                     free_slots.put(slot)
@@ -397,13 +399,16 @@ def stream_chunks(bam_path, region_start, region_end, devices, cell_map, run, ch
                     cell[tagged] = cell_of_raw[sub.cell[tagged]]
                     sub.cell = cell
                     io = (bs.compressed_bytes, bs.inflated_bytes)
+                    decode_s += time.perf_counter() - t0
                     todo.put((seq, sub, ends[send], n_carried, lo, done, slot,
                               dict(indexed=index_note is None, compressed_bytes=io[0] - io_sent[0],
-                                   inflated_bytes=io[1] - io_sent[1])))
-                    io_sent = io
+                                   inflated_bytes=io[1] - io_sent[1], decode_s=decode_s)))
+                    io_sent, decode_s = io, 0.0
                     seq += 1
-                elif slot is not None:
-                    free_slots.put(slot)
+                else:
+                    decode_s += time.perf_counter() - t0
+                    if slot is not None:
+                        free_slots.put(slot)
                 lo = done
                 if last is None:
                     break
@@ -470,13 +475,16 @@ def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, 
                  stats_out=None):
     """BaseCellCounter over a BAM of any size with bounded host memory (reference: the per-window pool of
     BaseCellCounter.py:344-409).  The windows are the regions of stream_chunks: a chunk runs ls_pileup_count on those
-    of its complete windows that a read reaches, and this thread appends the rows to one file per contig.  The table
+    of its complete windows that a read reaches, and this thread appends the rows to one file per contig.  The rows are
+    formatted on the device (Engine.pileup_count_text), or from the fetched counts by ls_write_counter_rows with
+    LONGSOM_COUNTER_TEXT=host and for an engine without a text writer.  The table
     lists the contigs in NAME order (collect_result sorts the window files by name), the BAM delivers them in header
     order: a contig's file is appended to the table as soon as every contig before it in name order is complete, so at
     the end only the last few are left to copy.  Returns the number of sites written; stats_out, if given, receives
     the stats of every chunk."""
     import contextlib
     import shutil
+    t_start = time.time()
     bs = bamio.BamStream(bam_path)  # the header only: stream_chunks decodes the reads
     names = bs.contig_names
     bs.close()
@@ -484,17 +492,28 @@ def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, 
     win = sorted((tid_of[c], s, e) for c, s, e in named_windows if c in tid_of and e > s)
     order = sorted({t for t, _s, _e in win}, key=lambda t: names[t])
     fasta_lock = threading.Lock()
-    busy = {"device": 0.0, "writer": 0.0, "concat": 0.0}
+    busy = {"decode": 0.0, "device": 0.0, "text": 0.0, "writer": 0.0, "concat": 0.0}
     cells = {}  # cleaned barcode (CB.split('-')[0], BaseCellCounter.py:246) -> dense id in first-appearance order
+    host_text = os.environ.get("LONGSOM_COUNTER_TEXT", "device") == "host"
+    names_b = [n.encode() for n in names]
 
     def run(eng, batch, ends, lo, done):
+        """The chunk's sites as SiteCounts (rows formatted by the writer) or, where the engine writes the rows itself,
+        as (n_sites, {tid: text})."""
         t0 = time.time()
         iv = prune_and_sort_windows([(names[t], s, e) for t, s, e in win[lo:done]], names, batch, ends)
         with fasta_lock:
             contig_seq = {t: fasta.contig(names[t]) for t in sorted({w[0] for w in iv})}
-        sites = eng.pileup_count(batch, Windows.from_intervals(iv, contig_seq), params)
+        w = Windows.from_intervals(iv, contig_seq)
+        if host_text or not hasattr(eng, "pileup_count_text"):  # (a stand-in engine has no text writer)
+            res = eng.pileup_count(batch, w, params)
+        else:
+            text = eng.pileup_count_text(batch, w, params, names_b)
+            res = (eng.last_stats["n_sites"], text)
+            busy["text"] += eng.last_stats["text_s"]
+            t0 += eng.last_stats["text_s"]
         busy["device"] += time.time() - t0
-        return sites
+        return res
 
     parts, out, next_part, n_sites = {}, None, 0, 0
 
@@ -535,14 +554,22 @@ def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, 
     cell_map = lambda b: cells.setdefault(b.split("-")[0], len(cells))
     try:
         with contextlib.closing(stream_chunks(bam_path, wk_start, wk_end, devices, cell_map, run, chunk_bytes)) as chunks:
-            for sites, _lo, done, stats in chunks:
+            for res, _lo, done, stats in chunks:
                 t0 = time.time()
+                busy["decode"] += stats["decode_s"]
                 if stats_out is not None:
                     stats_out.append(stats)
-                n_sites += sites.n_sites
-                for t in np.unique(sites.tid).tolist():
-                    path = parts.setdefault(t, "%s.part.%d.%d" % (out_file, os.getpid(), t))
-                    write_counter_rows(path, names[t], sites, t)
+                if isinstance(res, SiteCounts):
+                    n_sites += res.n_sites
+                    for t in np.unique(res.tid).tolist():
+                        path = parts.setdefault(t, "%s.part.%d.%d" % (out_file, os.getpid(), t))
+                        write_counter_rows(path, names[t], res, t)
+                else:
+                    n_sites += res[0]
+                    for t, text in res[1].items():
+                        path = parts.setdefault(t, "%s.part.%d.%d" % (out_file, os.getpid(), t))
+                        with open(path, "ab") as f:
+                            f.write(text)
                 busy["writer"] += time.time() - t0
                 append_ready(win[done][0] if done < len(win) else len(names))
         if n_sites == 0:
@@ -552,8 +579,9 @@ def stream_count(bam_path, named_windows, fasta, params: CountParams, out_file, 
         out.close()
         out = None
         if os.environ.get("LS_STREAM_TIMING"):
-            print("[stream_count] busy seconds: " + ", ".join("%s %.2f" % kv for kv in sorted(busy.items())) +
-                  "; peak RSS of this process %.2f GB" % _peak_rss_gb(), file=sys.stderr)
+            print("[stream_count] busy seconds: " + ", ".join("%s %.3f" % kv for kv in sorted(busy.items())) +
+                  "; wall %.3f s; peak RSS of this process %.2f GB" % (time.time() - t_start, _peak_rss_gb()),
+                  file=sys.stderr)
         return n_sites
     finally:
         for path in parts.values():
