@@ -344,6 +344,42 @@ int ls_geno_long_times(ls_ctx *ctx, double *ms_text, double *ms_copy, int64_t *b
 /* frees the long table's device buffers (a later text call is LS_E_STATE until the next load) */
 int ls_geno_long_release(ls_ctx *ctx);
 
+/* ---- BaseCellCalling.step1 ----------------------------------------------------------------------
+ * Replaces the per-row work of BaseCellCalling.step1.py:78-467 (the parse of the merged table, the betabinom.sf calls
+ * at :196,201,329-330, the contexts of :97-104, the label cascade and the output lines), on one line-aligned byte range
+ * of the table's body at a time.  The text equals that of the host passes ls_s1_parse + ls_s1_format of
+ * csrc/host/ls_step1.cpp, given the same tails.
+ *   load    copies the range to the device and parses it.  LS_E_ARG, with the row in ls_last_error, for a row
+ *           ls_s1_parse refuses, and for a range with a '\r' (the host passes read universal newlines), a candidate
+ *           allele at a depth or cell count of 0 or a VAF / MCF of 4e5 or more.  The CHROM names this range is the
+ *           first to name (since the last release) are written to new_names, NUL-terminated one after the other, with
+ *           the ids *first_new .. *first_new + *n_new - 1; LS_E_CAPACITY when they do not fit names_cap (len + 1
+ *           always suffices).  *n_queries: the beta-binomial tails the call evaluates.
+ *   contig  makes contig `id` resident (its bases as in the FASTA, any case).  Rows of a contig never made resident
+ *           print '.' contexts.  Contigs stay resident across loads, until the release.
+ *   call    the tails (K2, alpha1/beta1 on read counts, alpha2/beta2 on cell counts, rounded as np.round(p, 4)), the
+ *           labels and the length of every output row.  LS_E_ARG where ls_s1_format refuses (a NaN among a call's
+ *           per-allele tails); LS_E_STATE without a load.
+ *   text    the output rows row_lo .. row_lo + *rows_done - 1, as many whole rows as fit in capacity bytes: each input
+ *           row with the twenty INFO columns inserted after its 4th tab, '##' rows as they are.  A row longer than
+ *           capacity is LS_E_CAPACITY; LS_E_STATE without a call since the last load.
+ *   release frees the range's buffers and the resident contigs.                                                     */
+typedef struct ls_step1_in {
+  const int32_t *ct_cols;      /* [n_ct] the cell-type columns of the table, ascending, each >= 4 */
+  const char *ct_names;        /* their header names, back to back */
+  const int64_t *ct_name_off;  /* [n_ct+1] */
+  int32_t n_ct;                /* at most 64 */
+  int32_t min_cov, min_cells, min_ac_cells, min_ac_reads, min_cell_types, max_cell_types;
+  int32_t reserved;
+  double alpha1, beta1, alpha2, beta2;
+} ls_step1_in;
+int ls_step1_load(ls_ctx *ctx, const char *data, int64_t len, const ls_step1_in *in, int64_t *n_rows,
+                  int64_t *n_queries, char *new_names, int64_t names_cap, int32_t *first_new, int32_t *n_new);
+int ls_step1_contig(ls_ctx *ctx, int32_t id, const uint8_t *seq, int64_t len);
+int ls_step1_call(ls_ctx *ctx, int64_t *bytes, int64_t *longest_row);
+int ls_step1_text(ls_ctx *ctx, int64_t row_lo, char *out, int64_t capacity, int64_t *rows_done, int64_t *bytes);
+int ls_step1_release(ls_ctx *ctx);
+
 /* ---- device-resident handles for benchmarking (inputs already in HBM) ----------------------- */
 int ls_device_synchronize(ls_ctx *ctx);
 /* PCI address ("0000:1b:00.0") of a CUDA device ordinal, for NUMA placement of the host staging buffers; no context */

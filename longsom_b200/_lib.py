@@ -24,7 +24,7 @@ ABI_SYMBOLS = [
     "ls_betabinom_sf", "ls_site_mask", "ls_site_table_load", "ls_site_table_lookup", "ls_device_synchronize", "ls_device_pci_bus_id", "ls_flush_l2",
     "ls_geno_matrix_load", "ls_geno_matrix_text", "ls_geno_long_load", "ls_geno_long_text", "ls_geno_long_times",
     "ls_geno_long_release", "ls_pileup_text_load", "ls_pileup_text",
-    "ls_pileup_sites_upload",
+    "ls_pileup_sites_upload", "ls_step1_load", "ls_step1_contig", "ls_step1_call", "ls_step1_text", "ls_step1_release",
 ]
 LS_GENO_MATRIX_DP, LS_GENO_MATRIX_ALT, LS_GENO_MATRIX_VAF, LS_GENO_MATRIX_BINARY = 0, 1, 2, 3
 LS_GENO_ROW_CHRM, LS_GENO_ROW_FUSION = 1, 2
@@ -91,6 +91,14 @@ class LsGenoLongIn(C.Structure):
                 ("pvalue", C.c_double)]
 
 
+class LsStep1In(C.Structure):
+    _fields_ = [("ct_cols", C.c_void_p), ("ct_names", C.c_void_p), ("ct_name_off", C.c_void_p), ("n_ct", C.c_int32),
+                ("min_cov", C.c_int32), ("min_cells", C.c_int32), ("min_ac_cells", C.c_int32),
+                ("min_ac_reads", C.c_int32), ("min_cell_types", C.c_int32), ("max_cell_types", C.c_int32),
+                ("reserved", C.c_int32), ("alpha1", C.c_double), ("beta1", C.c_double), ("alpha2", C.c_double),
+                ("beta2", C.c_double)]
+
+
 class LongSomError(RuntimeError):
     pass
 
@@ -143,6 +151,12 @@ def load():
     lib.ls_geno_long_text.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, P(C.c_int64), P(C.c_int64)]
     lib.ls_geno_long_times.argtypes = [C.c_void_p, P(C.c_double), P(C.c_double), P(C.c_int64), P(C.c_int64)]
     lib.ls_geno_long_release.argtypes = [C.c_void_p]
+    lib.ls_step1_load.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, P(LsStep1In), P(C.c_int64), P(C.c_int64), C.c_void_p,
+                                  C.c_int64, P(C.c_int32), P(C.c_int32)]
+    lib.ls_step1_contig.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64]
+    lib.ls_step1_call.argtypes = [C.c_void_p, P(C.c_int64), P(C.c_int64)]
+    lib.ls_step1_text.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, P(C.c_int64), P(C.c_int64)]
+    lib.ls_step1_release.argtypes = [C.c_void_p]
     lib.ls_device_synchronize.argtypes = [C.c_void_p]
     lib.ls_flush_l2.argtypes = [C.c_void_p]
     for name in ABI_SYMBOLS:

@@ -5,9 +5,11 @@ betabinom.sf 2-12 times (~100 us each, :196,201,329-330).  Here the table is par
 (k, n) query of the run is gathered into two arrays (read counts with alpha1/beta1, cell counts
 with alpha2/beta2), the tails are computed in two GPU launches (K2, ls_betabinom_sf), and the
 label cascade (SURVEY.md Appendix C) is applied on the rounded p-values exactly as the
-reference does.  Output bytes are identical, including its quirks (Q5-Q8).  The per-row Python of the two passes
-is what this step costs, so tables above 8 MB are cut into byte ranges handled by forked worker processes
-(LONGSOM_PROCS, default min(16, cores)); the GPU calls stay in the parent."""
+reference does.  Output bytes are identical, including its quirks (Q5-Q8).  With the CUDA engine the whole row loop
+runs on the device (ls_step1.cu), one byte range of the table at a time; the host passes of ls_step1.cpp serve
+stand-in engines and the ranges the device refuses.  The Python passes stay as the statement of the reference; when
+they run on a table above 8 MB, it is cut into byte ranges handled by forked worker processes (LONGSOM_PROCS, default
+min(16, cores)); the GPU calls stay in the parent."""
 import argparse
 import os
 import sys
@@ -396,6 +398,88 @@ class _NativeRange:
             self.h = None
 
 
+STEP1_BLOCK_BYTES = 16 << 20   # text block of the device path (two pinned blocks, one filled while the other is written)
+last_times = {}                # busy seconds of the stages of the last device-called table (tools/cli_step1_timing.py)
+
+
+def _device_ranges(eng, out, ranges, read, cell_types_idx, fa, P, alphas, tails):
+    """The byte ranges of the table called on the device, one at a time, their text written to `out` in blocks of whole
+    rows: the parse, the tails, the labels, the contexts (from contigs kept resident on the device) and the rows are
+    computed in HBM.  The next range is read from the file while the device works on the current one.  A range the
+    device refuses is redone by the host passes (_NativeRange, with the same K2 tails), which give the same bytes; a
+    range they refuse raises ValueError.  Returns (rows, beta-binomial tails)."""
+    from concurrent.futures import ThreadPoolExecutor
+    import time
+    from .._lib import LS_E_ARG, LongSomError
+    from ..blocks import PinnedBlock, write_blocks
+    cols = sorted(cell_types_idx)
+    names = [cell_types_idx[c].encode() for c in cols]
+    n_rows = n_queries = n_host = 0
+    bufs, cap = [], 0
+    T = dict(read_s=0.0, call_s=0.0, text_s=0.0, write_s=0.0)  # text_s: the block loop, its file writes overlapped
+
+    def timed_read(rng):
+        t = time.perf_counter()
+        data = read(rng)
+        T["read_s"] += time.perf_counter() - t
+        return data
+
+    def host_range(data):
+        r = _NativeRange(data, cell_types_idx, P)
+        try:
+            r1, r2 = tails(r.q)
+            out.write(r.format(r1, r2, fa, P))
+            return r.n_rows, len(r1) + len(r2)
+        finally:
+            r.close()
+    try:
+        with ThreadPoolExecutor(1) as reader:
+            nxt = reader.submit(timed_read, ranges[0]) if ranges else None
+            for i in range(len(ranges)):
+                data = nxt.result()
+                nxt = reader.submit(timed_read, ranges[i + 1]) if i + 1 < len(ranges) else None
+                t0 = time.perf_counter()
+                try:
+                    rows, nq, new = eng.step1_load(data, cols, names, P.min_reads, P.min_cells, P.min_ac_cells,
+                                                   P.min_ac_reads, P.min_cell_types, P.max_cell_types, *alphas)
+                    for cid, name in new:   # a contig is made resident the first time a range names it
+                        if fa is None:
+                            continue
+                        try:
+                            seq = fa.contig(name)
+                        except Exception:
+                            continue        # not in the FASTA: its rows print '.' contexts
+                        eng.step1_contig(cid, seq)
+                    nbytes, longest = eng.step1_call()
+                except LongSomError as e:
+                    if getattr(e, "code", None) != LS_E_ARG:
+                        raise
+                    r, q = host_range(data)
+                    n_rows, n_queries, n_host = n_rows + r, n_queries + q, n_host + r
+                    T["call_s"] += time.perf_counter() - t0
+                    continue
+                t1 = time.perf_counter()
+                T["call_s"] += t1 - t0
+                if max(STEP1_BLOCK_BYTES, longest) > cap:
+                    for b in bufs:
+                        b.free()
+                    bufs = []
+                    cap = max(STEP1_BLOCK_BYTES, longest)
+                    bufs = [PinnedBlock(eng, cap) for _ in range(2)]
+                T["write_s"] += write_blocks(out, eng.step1_text, rows, bufs, cap)
+                T["text_s"] += time.perf_counter() - t1
+                n_rows += rows
+                n_queries += nq
+    finally:
+        for b in bufs:
+            b.free()
+        eng.step1_release()
+    T.update(rows=n_rows, host_rows=n_host)
+    last_times.clear()
+    last_times.update(T)
+    return n_rows, n_queries
+
+
 def _native_ok(P):
     return P.fisher_cutoff == 1 and os.environ.get("LONGSOM_STEP1_NATIVE", "1") != "0"
 
@@ -484,9 +568,10 @@ def variant_calling_step1(infile, outfile, fasta, alpha1, beta1, alpha2, beta2, 
         return np.round(p1, 4), np.round(p2, 4)
 
     if native:
-        # Native row passes, in waves of byte ranges so that the memory in flight does not grow with the table: every
-        # wave is parsed on threads (the library releases the GIL), its queries go through K2 in one call, it is
-        # formatted on threads and appended to the output.  A wave the strict parser refuses discards what has been
+        # Native row passes, in byte ranges so that the memory in flight does not grow with the table.  With the CUDA
+        # engine every range is called on the device (_device_ranges); otherwise the ranges go in waves through the
+        # host passes: parsed on threads (the library releases the GIL), the wave's queries through K2 in one call,
+        # formatted on threads and appended to the output.  A range the host parser refuses discards what has been
         # written and leaves the whole table to the Python passes below (whose exceptions are the reference's).
         from concurrent.futures import ThreadPoolExecutor
         nthr = 1 if body_bytes < (4 << 20) else min(16, _available_cpus())
@@ -498,38 +583,48 @@ def variant_calling_step1(infile, outfile, fasta, alpha1, beta1, alpha2, beta2, 
         n_rows = n_queries = 0
         ok = False
 
-        def parse(rng):
+        def read(rng):
             with open(infile, 'rb') as f:
                 f.seek(rng[0])
-                return _NativeRange(f.read(rng[1] - rng[0]), cell_types_idx, P)
+                return f.read(rng[1] - rng[0])
+
+        def parse(rng):
+            return _NativeRange(read(rng), cell_types_idx, P)
         try:
-            with open(tmp_out, 'wb') as out, ThreadPoolExecutor(nthr) as ex:
+            with open(tmp_out, 'wb') as out:
                 out.write("".join(out_lines).encode())
-                for w0 in range(0, len(ranges), nthr):
-                    wave = []
-                    try:
-                        for r in ex.map(parse, ranges[w0:w0 + nthr]):   # (a refusal surfaces here as ValueError)
-                            wave.append(r)
-                        qs = [r.q for r in wave]
-                        r1, r2 = tails(tuple(np.concatenate([q[j] for q in qs]) for j in range(4)))
-                        o1 = np.concatenate([[0], np.cumsum([len(q[0]) for q in qs])]).astype(np.int64)
-                        o2 = np.concatenate([[0], np.cumsum([len(q[2]) for q in qs])]).astype(np.int64)
-                        if fa is not None:     # contigs are loaded once, before the threads share the reader
-                            for r in wave:
-                                for ci in range(r.lib.ls_s1_n_chroms(r.h)):
-                                    try:
-                                        fa.contig(r.lib.ls_s1_chrom(r.h, ci).decode())
-                                    except Exception:
-                                        pass
-                        texts = list(ex.map(lambda kr: kr[1].format(r1[o1[kr[0]]:o1[kr[0] + 1]], r2[o2[kr[0]]:o2[kr[0] + 1]], fa, P),
-                                            enumerate(wave)))
-                        for t in texts:
-                            out.write(t)
-                        n_rows += sum(r.n_rows for r in wave)
-                        n_queries += len(r1) + len(r2)
-                    finally:
-                        for r in wave:
-                            r.close()
+                # the device path needs the CUDA engine; stand-in engines (the CPU tests' scipy tails) keep the host passes
+                if hasattr(Engine if callable(engine) else engine, "step1_load"):
+                    n_rows, n_queries = _device_ranges(get_engine(), out, ranges, read, cell_types_idx, fa, P,
+                                                       (alpha1, beta1, alpha2, beta2), tails)
+                else:
+                    with ThreadPoolExecutor(nthr) as ex:
+                        for w0 in range(0, len(ranges), nthr):
+                            wave = []
+                            try:
+                                for r in ex.map(parse, ranges[w0:w0 + nthr]):   # (a refusal surfaces here as ValueError)
+                                    wave.append(r)
+                                qs = [r.q for r in wave]
+                                r1, r2 = tails(tuple(np.concatenate([q[j] for q in qs]) for j in range(4)))
+                                o1 = np.concatenate([[0], np.cumsum([len(q[0]) for q in qs])]).astype(np.int64)
+                                o2 = np.concatenate([[0], np.cumsum([len(q[2]) for q in qs])]).astype(np.int64)
+                                if fa is not None:     # contigs are loaded once, before the threads share the reader
+                                    for r in wave:
+                                        for ci in range(r.lib.ls_s1_n_chroms(r.h)):
+                                            try:
+                                                fa.contig(r.lib.ls_s1_chrom(r.h, ci).decode())
+                                            except Exception:
+                                                pass
+                                texts = list(ex.map(lambda kr: kr[1].format(r1[o1[kr[0]]:o1[kr[0] + 1]],
+                                                                            r2[o2[kr[0]]:o2[kr[0] + 1]], fa, P),
+                                                    enumerate(wave)))
+                                for t in texts:
+                                    out.write(t)
+                                n_rows += sum(r.n_rows for r in wave)
+                                n_queries += len(r1) + len(r2)
+                            finally:
+                                for r in wave:
+                                    r.close()
             os.replace(tmp_out, outfile)
             ok = True
         except ValueError:

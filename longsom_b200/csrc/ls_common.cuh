@@ -176,6 +176,43 @@ struct CounterTextState {
   bool loaded = false;   // cleared by ls_pileup_upload and ls_pileup_run
 };
 
+// BaseCellCalling.step1 on the device: one byte range of the merged table between ls_step1_load and the
+// ls_step1_text calls, and the reference contigs, resident from the first range that names them to ls_step1_release
+struct Step1State {
+  DBuf data;                      // the range's bytes
+  DBuf flag, row_lo;              // [len] line-start flags, scanned; [n_rows+1] line starts, then len
+  DBuf rows, calls;               // [n_rows] S1Row; [n_rows][n_ct] S1Call
+  DBuf qoff, run;                 // 2 x [n_rows+1] query counts, scanned; contig-run flags and their scan
+  DBuf run_lo, run_ctg;           // per contig run: its first row's line start and CHROM length; its contig id
+  DBuf q, p;                      // queries k1 n1 k2 n2 (int32) and tails p1 p2 (double)
+  DBuf cols, names, name_off;     // the cell-type columns and their header names
+  DBuf ctg_ptr, ctg_len;          // per contig id: the resident bases, their number (-1: not resident)
+  DBuf lens, off, out, result;    // row lengths, their 64-bit scan, a text call's block, flags and totals
+  std::vector<DBuf *> contigs;    // [contig id] resident bases (nullptr: the FASTA does not have it)
+  std::vector<int64_t> contig_len;
+  std::vector<std::string> contig_names;
+  std::vector<int64_t> h_off;     // [n_rows+1] host copy of off: plans the blocks
+  int64_t len = 0, n_rows = 0, n_q1 = 0, n_q2 = 0;
+  int32_t n_ct = 0, min_cov = 0, min_cells = 0, min_ac_cells = 0, min_ac_reads = 0, min_cell_types = 0,
+          max_cell_types = 0;
+  double alpha1 = 0.0, beta1 = 0.0, alpha2 = 0.0, beta2 = 0.0;
+  bool loaded = false, called = false;
+  void release() {
+    for (DBuf *b : {&data, &flag, &row_lo, &rows, &calls, &qoff, &run, &run_lo, &run_ctg, &q, &p, &cols, &names,
+                    &name_off, &ctg_ptr, &ctg_len, &lens, &off, &out, &result})
+      b->release();
+    for (DBuf *b : contigs) delete b;
+    contigs.clear();
+    contig_len.clear();
+    contig_names.clear();
+    std::vector<int64_t>().swap(h_off);
+    loaded = called = false;
+  }
+  ~Step1State() {
+    for (DBuf *b : contigs) delete b;
+  }
+};
+
 // What a replay of ls_pileup_run takes from the last run on the batch that it can stand for
 struct ReplaySnapshot {
   bool valid = false;
@@ -234,6 +271,7 @@ struct ls_ctx {
   GenoMatrixState gm;  // genotype matrix writer
   GenoLongState gl;    // genotype long-table writer
   CounterTextState ct;  // counter table writer
+  Step1State s1;        // BaseCellCalling.step1
 };
 
 #define LS_CK(call)                                                                        \

@@ -9,6 +9,7 @@ Mirrors the reference's unit operations:
   Engine.site_mask        <-> step2.build_dict / GetExtraFilters    (BaseCellCalling.step2.py:124-221)
   Engine.geno_matrix_*    <-> the pandas pivots of SingleCellGenotype (SingleCellGenotype.py:351-379)
   Engine.geno_long_*      <-> the long-table row loops of both genotype scripts (SingleCellGenotype.py:128-214)
+  Engine.step1_*          <-> the row loop of BaseCellCalling.step1 (BaseCellCalling.step1.py:78-467), one byte range
 Every method runs on the GPU; there is no CPU path behind any of them.
 """
 import ctypes as C
@@ -278,6 +279,57 @@ class Engine:
     def geno_long_release(self):
         """Frees the device buffers of the loaded long table."""
         self._check(self._lib.ls_geno_long_release(self._ctx), "ls_geno_long_release")
+
+    # ---- BaseCellCalling.step1 -----------------------------------------------------------
+    def step1_load(self, data, cols, names, min_cov, min_cells, min_ac_cells, min_ac_reads, min_cell_types,
+                   max_cell_types, alpha1, beta1, alpha2, beta2):
+        """Copies one line-aligned byte range of the merged table's body (bytes) to the device and parses it.  cols:
+        the cell-type columns, ascending; names: their header names (bytes).  Returns (rows, queries, new), new being
+        [(contig id, CHROM name)] of the contigs no earlier range (since step1_release) has named.  A row the parser
+        refuses raises LongSomError with code LS_E_ARG."""
+        cols = np.ascontiguousarray(cols, np.int32)
+        off = np.zeros(len(names) + 1, np.int64)
+        np.cumsum(np.fromiter((len(x) for x in names), np.int64, len(names)), out=off[1:])
+        blob = b"".join(names)
+        vp = lambda a: a.ctypes.data_as(C.c_void_p) if a.size else None
+        s = L.LsStep1In(vp(cols), C.cast(C.c_char_p(blob), C.c_void_p), off.ctypes.data_as(C.c_void_p), len(cols),
+                        int(min_cov), int(min_cells), int(min_ac_cells), int(min_ac_reads), int(min_cell_types),
+                        int(max_cell_types), 0, float(alpha1), float(beta1), float(alpha2), float(beta2))
+        buf = np.empty(len(data) + 1, np.uint8)   # the new names fit in len + 1 bytes; untouched pages cost nothing
+        rows, nq, first, nn = C.c_int64(0), C.c_int64(0), C.c_int32(0), C.c_int32(0)
+        self._check(self._lib.ls_step1_load(self._ctx, C.cast(C.c_char_p(data), C.c_void_p), len(data), C.byref(s),
+                                            C.byref(rows), C.byref(nq), buf.ctypes.data, buf.shape[0], C.byref(first),
+                                            C.byref(nn)), "ls_step1_load")
+        new, at = [], 0
+        for i in range(nn.value):
+            end = at + int(np.argmax(buf[at:] == 0))
+            new.append((first.value + i, buf[at:end].tobytes().decode()))
+            at = end + 1
+        return int(rows.value), int(nq.value), new
+
+    def step1_contig(self, cid, seq):
+        """Makes contig `cid` (an id from step1_load) resident on the device: seq, its bases as uint8."""
+        seq = np.ascontiguousarray(seq, np.uint8)
+        self._check(self._lib.ls_step1_contig(self._ctx, int(cid), seq.ctypes.data_as(C.c_void_p) if seq.size else None,
+                                              seq.shape[0]), "ls_step1_contig")
+
+    def step1_call(self):
+        """Tails, labels and row lengths of the loaded range: (bytes of its text, longest row)."""
+        nb, longest = C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.ls_step1_call(self._ctx, C.byref(nb), C.byref(longest)), "ls_step1_call")
+        return int(nb.value), int(longest.value)
+
+    def step1_text(self, row_lo, out, capacity):
+        """Text of the whole rows row_lo.. of the called range that fit in `capacity` bytes at address `out`: (rows
+        written, bytes)."""
+        rows, nb = C.c_int64(0), C.c_int64(0)
+        self._check(self._lib.ls_step1_text(self._ctx, int(row_lo), out, int(capacity), C.byref(rows), C.byref(nb)),
+                    "ls_step1_text")
+        return int(rows.value), int(nb.value)
+
+    def step1_release(self):
+        """Frees the range's device buffers and the resident contigs."""
+        self._check(self._lib.ls_step1_release(self._ctx), "ls_step1_release")
 
     # ---- K2 ------------------------------------------------------------------------------
     def betabinom_sf(self, k, n, a, b):
